@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ms+cs dense contrastive loss hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2] [--dump-outputs DIR]
 
 A step = one forward + backward of the loss over one batch of synthetic inputs (SURVEY.md §8d).
 N=1 workload: cfg2 = HRNet-W48 Cityscapes ms+cs (4 scales, 512x1024 crops, bs 12, 256-d).
@@ -18,6 +18,8 @@ Defaults: K=100 timed steps after W=20 warm-up steps (a step is ~1 ms; the short
 versions made the timed region sensitive to the start-up of a fresh process); `--impl reference`: K=5, W=1 (a CPU
 step takes seconds); exactly K steps after W are timed on a bounded SAMPLE of the workload (the first images of the same
 batch), sized from a calibration step so that the run ends within ~4 minutes (`cpu_baseline.sample` says which).
+--steps / --warmup set the timed loop of the headline number; the two side records of the GPU run keep fixed counts,
+stated in their own fields: `pooled` (cfg5, 10 steps after 3) and `cpu_baseline` (2 steps after 1 on 3 images).
 """
 import argparse
 import json
@@ -246,6 +248,37 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, mod, feats):
+    """Writes what one step returned to its caller as ``out_dir/<name>.npy``: ``loss``, the per-scale terms the module
+    exposes for logging (``ms_losses``, ``cs_losses``), and per scale the dense feature gradient at the pixels that
+    carry one (every other entry is exactly zero): ``grad<s>_pixels`` (flat index (image * h + y) * w + x, float64) and
+    ``grad<s>_rows`` (pixels x C, float32).  A scale whose rows exceed its share of DUMP_BYTES keeps a fixed, seeded
+    sample of them (pixel order kept)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": np.array([float(loss.detach())], dtype=np.float64)}
+    for key in ("ms_losses", "cs_losses"):
+        vals = getattr(mod, key, None)
+        if vals:
+            arrays[key] = np.array([float(v) for v in vals], dtype=np.float64)
+    share = (DUMP_BYTES - (1 << 20)) // len(feats)
+    for s, f in enumerate(feats):
+        C = f.shape[1]
+        g = f.grad.detach().permute(0, 2, 3, 1).reshape(-1, C)
+        pix = (g != 0).any(dim=1).nonzero().squeeze(1)
+        keep = share // (C * 4 + 8)
+        if pix.numel() > keep:
+            sel = torch.randperm(pix.numel(), generator=torch.Generator().manual_seed(s))[:keep].sort().values
+            pix = pix[sel.to(pix.device)]
+        arrays[f"grad{s}_pixels"] = pix.cpu().double().numpy()
+        arrays[f"grad{s}_rows"] = g[pix].float().cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def measure_pooled(dev, rank, world, dist, steps=10, warmup=3):
     """The sharded configuration north_star names (cfg5: 64 images pooled over the ranks, anchor rows sharded, keys /
     row statistics / gradient rows exchanged): ms per step at this world size and -- measured in the same run by rank 0
@@ -338,7 +371,9 @@ def main():
     ap.add_argument("--gpus", type=int, default=1)
     # a step is ~1 ms: the defaults keep the timed region (0.1 s) well above start-up effects of a fresh process
     # (cold page cache, allocator growth); the whole default run still takes well under a minute
-    ap.add_argument("--steps", type=int, default=None, help="default: 100 (--impl reference: 5)")
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of the headline loop; default: 100 (--impl reference: 5). The pooled and "
+                         "cpu_baseline side records use fixed counts (see the module docstring)")
     ap.add_argument("--warmup", type=int, default=None, help="default: 20 (--impl reference: 1)")
     ap.add_argument("--impl", default="mscs", choices=["mscs", "reference"])
     ap.add_argument("--workload", default="cfg2")
@@ -347,10 +382,17 @@ def main():
     ap.add_argument("--layout", default="nchw", choices=["nchw", "nhwc"],
                     help="memory order of the feature maps: nchw = what the reference's projector emits (headline); "
                          "nhwc = torch.channels_last (row gather / scatter)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss, its logged per-scale terms and the feature gradients "
+                         "of the last timed step as DIR/<name>.npy (rank 0; at most 64 MB, see dump_outputs)")
     args = ap.parse_args()
     ref = args.impl == "reference"       # a reference step is seconds of CPU work, one of ours a millisecond
+    if ref and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the GPU path; it does not apply to --impl reference")
     args.steps = args.steps if args.steps is not None else (5 if ref else 100)
     args.warmup = args.warmup if args.warmup is not None else (1 if ref else 20)
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
@@ -425,6 +467,8 @@ def main():
     e1.record()
     barrier()
     stage_ms = {k: sum(a.elapsed_time(b) for a, b in v) / len(v) for k, v in _ops.TIMING.items()}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, mod, feats)
     _ops.TIMING, _ops.TIMING_ALL = {}, True
     n_stage = max(3, min(args.steps, 50))
     for i in range(n_stage):

@@ -1,6 +1,6 @@
 """Generate the golden fixtures under tests/golden/ from the EXECUTABLE REFERENCE.
 
-Run in the build container only (needs /root/reference):   python tests/golden/make_golden.py
+Needs a checkout of the original project:   MSCS_REFERENCE=<checkout> python tests/golden/make_golden.py
 The reference's loss modules are imported unmodified; two shims make them run on CPU
 (SURVEY.md §8c): a stub ``utils`` package (the real one needs matplotlib) that serves the real
 ``utils.defaults.DATASETS_INFO``, and ``torch.Tensor.cuda`` replaced by identity for the
@@ -24,7 +24,7 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
+REF = os.environ.get("MSCS_REFERENCE", "")
 
 
 def import_reference():

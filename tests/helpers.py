@@ -42,6 +42,37 @@ def cosine(a, b):
     return float(a @ b / np.sqrt((a @ a) * (b @ b)))
 
 
+class LossWrapperBoundary:
+    """The calling convention of the reference's ``losses/LossWrapper.py`` for the contrastive classes, restated: the
+    class is built by NAME from the ``losses`` namespace (``globals()[loss_class](config)``, :33), called as
+    ``module(labels, deep_features)`` (:68-71), the returned tensor is multiplied IN PLACE by the loss weight (:90) and
+    logged detached (:91), the per-scale ``ms_losses`` / ``cs_losses`` of the _ms class are logged under
+    ``<name>_ms<i>`` / ``<name>_cs<i>`` (:94-101) and the weighted losses are summed into ``total_loss`` (:102)."""
+
+    def __init__(self, config, namespace):
+        self.loss_weightings = dict(config["losses"])
+        self.loss_classes = {k: getattr(namespace, k)(config) for k in self.loss_weightings}
+        self.loss_vals = {k: 0 for k in self.loss_weightings}
+        self.total_loss = None
+
+    def __call__(self, prediction, labels, deep_features=None):
+        total = None
+        for key, w in self.loss_weightings.items():
+            module = self.loss_classes[key]
+            loss = module(labels, deep_features)
+            loss *= w
+            self.loss_vals[key] = loss.detach()
+            if key == "DenseContrastiveLossV2_ms":
+                for i, v in enumerate(module.ms_losses):
+                    self.loss_vals[f"{key}_ms{i}"] = v
+                if module.cross_scale_contrast:
+                    for i, v in enumerate(module.cs_losses):
+                        self.loss_vals[f"{key}_cs{i}"] = v
+            total = loss if total is None else total + loss
+        self.total_loss = total
+        return total
+
+
 def make_module(meta, device=None):
     import mscs_b200
     cls = mscs_b200.DenseContrastiveLossV2 if meta["single_scale"] else mscs_b200.DenseContrastiveLossV2_ms

@@ -1,5 +1,5 @@
-"""GPU: the co-losses on one label read (SURVEY.md 8f item 2, mscs_b200/coloss.py, csrc/ce.cu) against ATen and against
-the reference's own LossWrapper run live on this GPU (oracle/_ref) with CrossEntropyLoss + DenseContrastiveLossV2_ms.
+"""GPU: the co-losses on one label read (SURVEY.md 8f item 2, mscs_b200/coloss.py, csrc/ce.cu) against ATen, and the
+LossWrapper-shaped combination CrossEntropyLoss + DenseContrastiveLossV2_ms against ATen plus the fp64 oracle.
 
 Tolerances: the label pass and K1 on compact labels are bit-exact; the fused cross entropy is fp32 against fp32 ATen
 (loss <= 1e-5 relative, gradient max-abs <= 1e-5 of the gradient's max); the combined total follows north_star
@@ -81,40 +81,72 @@ def test_k1_on_compact_labels_is_bit_exact(dev):
     assert float(l64) == float(l16)
 
 
-def test_fused_colosses_vs_reference_losswrapper_live(dev):
-    """CrossEntropyLoss + DenseContrastiveLossV2_ms through the reference's own LossWrapper and classes on this GPU
-    against FusedCoLosses on the same inputs and generator state."""
+# What the reference's LossWrapper builds for CrossEntropyLoss (LossWrapper.py:22-31), kept here independently of the
+# code under test: (number of label ids incl. the ignore id, ignore_index, class weights).  The Cityscapes weights are
+# the published HRNet Cityscapes cross-entropy weights the reference hard-codes; every other dataset is unweighted.
+CE_SETUP = {
+    "CITYSCAPES": (20, 19, [0.8373, 0.918, 0.866, 1.0345, 1.0166, 0.9969, 0.9754, 1.0489, 0.8786, 1.0023, 0.9539,
+                            0.9843, 1.1116, 0.9037, 1.0865, 1.0955, 1.0865, 1.1529, 1.0507]),
+    "ADE20K": (151, 150, None),
+}
+
+
+def test_fused_colosses_vs_aten_and_fp64_oracle(dev):
+    """CrossEntropyLoss + DenseContrastiveLossV2_ms as the reference's LossWrapper combines them -- its
+    ``nn.CrossEntropyLoss(ignore_index, weight)`` (ATen, this GPU, set up from CE_SETUP: class-weighted for Cityscapes)
+    and the fp64 oracle of the contrastive loss, each weighted, same ``loss_vals`` keys -- against FusedCoLosses on the
+    same inputs and generator state."""
+    _colosses_vs_aten_and_fp64_oracle("CITYSCAPES", dev)
+
+
+def test_fused_colosses_unweighted_dataset_vs_aten_and_fp64_oracle(dev):
+    """The same for a dataset the reference's LossWrapper does not weight (ADE20K: plain cross entropy, ignore 150)."""
+    _colosses_vs_aten_and_fp64_oracle("ADE20K", dev)
+
+
+def _colosses_vs_aten_and_fp64_oracle(dataset, dev):
     import mscs_b200
     from mscs_b200 import synth
-    from oracle import ref_loader
-    if ref_loader.find_root() is None:
-        pytest.fail("oracle/_ref/ is missing: __graft_entry__.build() stages it in the build container")
-    ref = ref_loader.load(cpu=False)
-    cfg = dict(dataset="CITYSCAPES", experiment=1, temperature=0.1, scales=3, weights=[1.0, 0.7, 0.4],
+    from oracle import loss_fp64
+    from oracle.config import oracle_cfg
+    from oracle.mt19937 import MT19937
+    A, ignore, class_weights = CE_SETUP[dataset]
+    cfg = dict(dataset=dataset, experiment=1, temperature=0.1, scales=3, weights=[1.0, 0.7, 0.4],
                cross_scale_contrast=True, w_high_low=0.5, w_high_mid=0.25, min_views_per_class=5,
                max_views_per_class=40, max_features_total=1200,
                losses={"CrossEntropyLoss": 1.0, "DenseContrastiveLossV2_ms": 0.1}, device=dev)
     n, H, W = 3, 128, 256
-    labels = synth.synth_labels(n, H, W, 19, 7, 16, 0.05, 51).to(dev)
+    labels = synth.synth_labels(n, H, W, ignore, 7, 16, 0.05, 51).to(dev)
     g = torch.Generator().manual_seed(52)
-    pred = (2.0 * torch.randn(n, 19, H, W, generator=g)).to(dev)
+    pred = (2.0 * torch.randn(n, A - 1, H, W, generator=g)).to(dev)
     feats = [torch.randn(n, 64, H // s, W // s, generator=g).to(dev) for s in (4, 8, 16)]
     torch.manual_seed(7)
     rng = torch.get_rng_state()
 
-    def run(wrapper):
-        p = pred.clone().requires_grad_(True)
-        f = [x.clone().requires_grad_(True) for x in feats]
-        torch.set_rng_state(rng)
-        total = wrapper(p, labels, deep_features=f)
-        total.backward()
-        torch.cuda.synchronize()
-        return float(total), {k: float(v) for k, v in wrapper.loss_vals.items()}, p.grad, [x.grad for x in f]
+    w_ce, w_dc = cfg["losses"]["CrossEntropyLoss"], cfg["losses"]["DenseContrastiveLossV2_ms"]
+    p = pred.clone().requires_grad_(True)
+    wt = None if class_weights is None else torch.tensor(class_weights, device=dev)
+    ce = torch.nn.CrossEntropyLoss(ignore_index=ignore, weight=wt)(p, labels)
+    (w_ce * ce).backward()
+    gen = MT19937.from_torch_state(rng.numpy().tobytes())
+    dc = loss_fp64.ms_cs_loss(labels.cpu().numpy(), [f.cpu().numpy() for f in feats], oracle_cfg(cfg, A), gen)
+    t_r = w_ce * float(ce) + w_dc * dc["total"]
+    vals_r = {"CrossEntropyLoss": w_ce * float(ce), "DenseContrastiveLossV2_ms": w_dc * dc["total"]}
+    vals_r.update({f"DenseContrastiveLossV2_ms_ms{i}": v for i, v in enumerate(dc["ms"])})
+    vals_r.update({f"DenseContrastiveLossV2_ms_cs{i}": v for i, v in enumerate(dc["cs"])})
+    gp_r = p.grad
+    gf_r = [torch.from_numpy(w_dc * g) for g in dc["grads"]]
 
-    with torch.cuda.device(dev):
-        t_r, vals_r, gp_r, gf_r = run(ref.LossWrapper(cfg))
-    t_o, vals_o, gp_o, gf_o = run(mscs_b200.FusedCoLosses(cfg))
-    print(f"co-losses: total {t_o:.6f} reference LossWrapper {t_r:.6f}")
+    wrapper = mscs_b200.FusedCoLosses(cfg)
+    p = pred.clone().requires_grad_(True)
+    f = [x.clone().requires_grad_(True) for x in feats]
+    torch.set_rng_state(rng)
+    total = wrapper(p, labels, deep_features=f)
+    total.backward()
+    torch.cuda.synchronize()
+    t_o, vals_o = float(total), {k: float(v) for k, v in wrapper.loss_vals.items()}
+    gp_o, gf_o = p.grad, [x.grad.cpu() for x in f]
+    print(f"{dataset} co-losses: total {t_o:.6f} ATen cross entropy + fp64 oracle {t_r:.6f}")
     assert abs(t_o - t_r) < 1e-3 * abs(t_r)
     assert set(vals_o) == set(vals_r)
     for k in vals_r:

@@ -1,7 +1,7 @@
 """GPU: the projector tail evaluated on the sampled rows only (SURVEY.md 8f item 1, mscs_b200/projector.py) against the
 DENSE evaluation it replaces -- ``nn.Conv2d(c_prev, d, 1)`` on every pixel (the last layer of the reference's
-projector, models/Projector.py:69) followed by the reference's OWN ``DenseContrastiveLossV2_ms`` run live on this GPU
-(oracle/_ref, fp32 ATen) and by this repository's drop-in class.  Same labels, same generator state: the sampled
+projector, models/Projector.py:69) followed by the fp64 oracle of ``DenseContrastiveLossV2_ms`` and by this repository's
+drop-in class.  Same labels, same generator state: the sampled
 pixels are identical, so loss and the gradients w.r.t. the pre-projection features, the weights and the biases must
 agree within the north_star tolerances (loss 1e-3 relative, gradient cosine >= 0.999)."""
 import numpy as np
@@ -61,21 +61,30 @@ CFG = dict(dataset="CITYSCAPES", experiment=1, temperature=0.1, scales=3, weight
            max_views_per_class=40, max_features_total=1200)
 
 
-def test_projector_tail_vs_dense_reference_live(dev):
-    from oracle import ref_loader
-    if ref_loader.find_root() is None:
-        pytest.fail("oracle/_ref/ is missing: __graft_entry__.build() stages it in the build container")
-    ref = ref_loader.load(cpu=False)
+def test_projector_tail_vs_dense_fp64_oracle(dev):
+    """The dense evaluation with the fp64 oracle as the loss: ``nn.Conv2d`` on every pixel, oracle loss and gradient
+    w.r.t. the projected maps, autograd back through the convolutions."""
+    from oracle import loss_fp64
+    from oracle.config import oracle_cfg
+    from oracle.mt19937 import MT19937
     labels, zs, mod = _case(dev, 3, 48, 64, 128, 256, [4, 8, 16], CFG, 31)
     torch.manual_seed(9)
     rng = torch.get_rng_state()
     l_s, gz_s, gw_s, gb_s = _run_sparse(mod, labels, zs, rng)
-    rng_after = torch.get_rng_state()
-    with torch.cuda.device(dev):
-        l_r, gz_r, gw_r, gb_r = _run_dense(ref.DenseContrastiveLossV2_ms(dict(CFG)), mod, labels, zs, rng)
-    assert torch.equal(torch.get_rng_state(), rng_after)
-    rel = abs(float(l_s) - float(l_r)) / abs(float(l_r))
-    print(f"projector tail: loss {float(l_s):.6f} dense reference {float(l_r):.6f} rel {rel:.2e}")
+    rng_after = MT19937.from_torch_state(torch.get_rng_state().numpy().tobytes())
+    zg = [z.clone().requires_grad_(True) for z in zs]
+    mod.zero_grad()
+    ys = [t(z) for t, z in zip(mod.tails, zg)]
+    gen = MT19937.from_torch_state(rng.numpy().tobytes())
+    res = loss_fp64.ms_cs_loss(labels.cpu().numpy(), [y.detach().cpu().double().numpy() for y in ys],
+                               oracle_cfg(CFG, 20), gen)
+    assert gen.pos == rng_after.pos and np.array_equal(gen.mt, rng_after.mt)
+    torch.autograd.backward(ys, [torch.from_numpy(g).to(dev, torch.float32) for g in res["grads"]])
+    torch.cuda.synchronize()
+    l_r, gz_r = res["total"], [z.grad for z in zg]
+    gw_r, gb_r = [t.weight.grad.clone() for t in mod.tails], [t.bias.grad.clone() for t in mod.tails]
+    rel = abs(float(l_s) - l_r) / abs(l_r)
+    print(f"projector tail: loss {float(l_s):.6f} dense fp64 oracle {l_r:.6f} rel {rel:.2e}")
     assert rel < 1e-3
     for s in range(len(zs)):
         assert torch.equal((gz_s[s] != 0).any(dim=1), (gz_r[s] != 0).any(dim=1)), "different pixels carry a gradient"

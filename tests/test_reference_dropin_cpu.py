@@ -1,4 +1,5 @@
-"""CPU, build container only (needs /root/reference, skipped elsewhere): the UNMODIFIED reference LossWrapper builds
+"""CPU, needs a checkout of the original project (MSCS_REFERENCE=<checkout>, skipped without one): the UNMODIFIED
+reference LossWrapper builds
 and dispatches this repository's classes once they are registered under the reference's names
 (LossWrapper.py:33 `globals()[loss_class](config)`, :68-71 `module(labels, deep_features)`).
 Runs in a subprocess: the import shims (stub `utils` / `losses` packages) must not leak into other tests."""
@@ -10,7 +11,7 @@ import pytest
 
 from helpers import ROOT
 
-REF = "/root/reference"
+REF = os.environ.get("MSCS_REFERENCE", "")
 
 SCRIPT = r'''
 import importlib, os, sys, types
@@ -62,7 +63,8 @@ print("DROPIN-OK")
 '''
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "losses")), reason="needs the reference checkout")
+@pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "losses")),
+                    reason="needs a checkout of the original project (MSCS_REFERENCE)")
 def test_reference_losswrapper_builds_and_dispatches_our_classes(tmp_path):
     script = tmp_path / "dropin.py"
     script.write_text(SCRIPT)
