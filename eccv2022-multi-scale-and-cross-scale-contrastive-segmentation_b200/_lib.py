@@ -5,6 +5,7 @@ import os
 
 MAX_SCALES, MAX_TERMS = 8, 16
 MAX_RANKS, IPC_HANDLE_BYTES = 8, 64      # MSCS_MAX_RANKS, MSCS_IPC_HANDLE_BYTES
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2   # MSCS_DTYPE_*: element type of feature maps / logits and their gradients
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MSCS_LIB") or os.path.join(_HERE, "libmscs.so")   # MSCS_LIB: profiling build
@@ -25,18 +26,20 @@ class ScalePlan(C.Structure):
 
 class GatherItem(C.Structure):
     _fields_ = [("feat", C.c_void_p), ("n", C.c_int32), ("C", C.c_int32), ("plane", C.c_int32), ("slot", C.c_void_p),
-                ("n_rows_dev", C.c_void_p), ("anc_bf16", C.c_void_p), ("anc_f32", C.c_void_p), ("inv_norm", C.c_void_p)]
+                ("n_rows_dev", C.c_void_p), ("anc_bf16", C.c_void_p), ("anc_f32", C.c_void_p), ("inv_norm", C.c_void_p),
+                ("dtype", C.c_int32)]
 
 
 class ScatterItem(C.Structure):
     _fields_ = [("dF", C.c_void_p), ("ldF", C.c_int32), ("anc_f32", C.c_void_p), ("inv_norm", C.c_void_p),
-                ("slot", C.c_void_p), ("n", C.c_int32), ("C", C.c_int32), ("plane", C.c_int32), ("dfeat", C.c_void_p)]
+                ("slot", C.c_void_p), ("n", C.c_int32), ("C", C.c_int32), ("plane", C.c_int32), ("dfeat", C.c_void_p),
+                ("dtype", C.c_int32)]
 
 
 class RowsItem(C.Structure):
     _fields_ = [("feat", C.c_void_p), ("pix", C.c_void_p), ("n_rows_dev", C.c_void_p), ("rows", C.c_int32),
                 ("C", C.c_int32), ("anc_bf16", C.c_void_p), ("anc_f32", C.c_void_p), ("inv_norm", C.c_void_p),
-                ("dF", C.c_void_p), ("ldF", C.c_int32), ("dfeat", C.c_void_p)]
+                ("dF", C.c_void_p), ("ldF", C.c_int32), ("dfeat", C.c_void_p), ("dtype", C.c_int32)]
 
 
 class Term(C.Structure):
@@ -131,9 +134,9 @@ _SIGNATURES = {
     "mscs_sample_hist_i16": (C.c_int, [C.POINTER(SampleCfg), C.c_void_p, C.c_void_p, C.c_void_p]),
     "mscs_sample_plan_i16": (C.c_int, [C.POINTER(SampleCfg), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mscs_ce_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
-                                  C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+                                  C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "mscs_ce_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
-                                   C.c_void_p, C.c_void_p, C.c_void_p]),
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "mscs_gather_rows_raw": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mscs_scatter_rows_raw": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                         C.c_void_p]),

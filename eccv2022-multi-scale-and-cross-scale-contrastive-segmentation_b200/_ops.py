@@ -30,6 +30,8 @@ _DENSE_ONE_PASS = os.environ.get("MSCS_DENSE", "1") != "0"
 # 0.094 ms, r02: a box of {8 pixels x 256 channels} is 256 rows of 32 bytes, which the TMA unit streams at ~0.2 rows per
 # clock and SM), so the lane-load kernel stays the default
 _GATHER_TMA = os.environ.get("MSCS_GATHER", "lanes") == "tma"
+# element types the kernels read and write natively (MSCS_DTYPE_* codes of the C ABI); see half_io_ok
+_DTYPE_CODE = {torch.float32: _lib.DTYPE_F32, torch.bfloat16: _lib.DTYPE_BF16, torch.float16: _lib.DTYPE_F16}
 
 # optional per-stage device timing (bench.py): {stage: [(start_event, end_event), ...]} or None
 TIMING = None
@@ -557,7 +559,7 @@ def scatter_grad(dF, aset, sample, feat_shape, dtype, prezeroed=None, slot=None)
 class _GradBuffers:
     """Dense feature gradients zero-filled ahead of time on a side stream (the zero fill is the
     largest HBM term of the whole path, SURVEY.md §8d, and does not depend on any result).  One slab for all
-    scales and one fill: the per-scale tensors handed to autograd are views of it."""
+    scales and one fill: the per-scale tensors handed to autograd are views of it, in the dtype of the maps."""
     _side = {}
 
     def __init__(self, feats, needs, nhwc=False, extra=0):
@@ -565,21 +567,23 @@ class _GradBuffers:
         side = self._side.get(dev)
         if side is None:
             side = self._side[dev] = torch.cuda.Stream(device=dev)
-        sizes = [f.numel() if (need and (nhwc or (f.shape[2] * f.shape[3]) % 8 == 0)) else 0
-                 for f, need in zip(feats, needs)]
+        # bytes per buffer, each rounded up to 16 (row stores of the scatter; mixed dtypes stay aligned)
+        sizes = [(f.numel() * f.element_size() + 15) // 16 * 16
+                 if (need and (nhwc or (f.shape[2] * f.shape[3]) % 8 == 0)) else 0 for f, need in zip(feats, needs)]
         # `extra` floats after the dense gradients: the gradient-row slab (dF) of the backward, zeroed by the same fill
-        dense = (sum(sizes) + 63) // 64 * 64          # dF starts 256-byte aligned (vector reductions / loads)
-        self.slab = torch.empty(dense + extra if extra else sum(sizes), dtype=torch.float32, device=dev)
-        self.dF = self.slab[dense:] if extra else None
+        dense = (sum(sizes) + 255) // 256 * 256       # dF starts 256-byte aligned (vector reductions / loads)
+        self.slab = torch.empty(dense + 4 * extra if extra else sum(sizes), dtype=torch.uint8, device=dev)
+        self.dF = self.slab[dense:].view(torch.float32) if extra else None
         self.bufs, off = [], 0
         for f, n_ in zip(feats, sizes):
             if not n_:
                 self.bufs.append(None)
             elif nhwc:      # same (n, C, h, w) shape, channels-last strides like the input
                 n, Cc, h, w = f.shape
-                self.bufs.append(self.slab[off:off + n_].view(n, h, w, Cc).permute(0, 3, 1, 2))
+                buf = self.slab[off:off + f.numel() * f.element_size()].view(f.dtype)
+                self.bufs.append(buf.view(n, h, w, Cc).permute(0, 3, 1, 2))
             else:
-                self.bufs.append(self.slab[off:off + n_].view(f.shape))
+                self.bufs.append(self.slab[off:off + f.numel() * f.element_size()].view(f.dtype).view(f.shape))
             off += n_
         self.side, self.ready = side, None
 
@@ -589,7 +593,7 @@ class _GradBuffers:
         side = self.side
         side.wait_stream(_cur_stream())
         if self.slab.numel() or extra:
-            regions = ([(self.slab.data_ptr(), 4 * self.slab.numel())] if self.slab.numel() else []) + \
+            regions = ([(self.slab.data_ptr(), self.slab.numel())] if self.slab.numel() else []) + \
                 ([extra] if extra else [])
             ptrs = _lib.ptr_array([r[0] for r in regions])
             if TIMING is not None:      # bench.py: the fill's own duration, on the stream it runs on
@@ -867,6 +871,31 @@ def fast_path_ok(spec, world):
     return world == 1 and v_cap * 12 <= 200 * 1024
 
 
+def half_io_ok(sp, world):
+    """Whether bf16 / fp16 feature maps are handed to the kernels as they are (no fp32 copy; the dense gradients are
+    written in the maps' dtype): the single-process fast path with the channels-last row gather, or with the NCHW lane
+    gather and the one-pass dense writer.  Every other route -- pooled mode, planes that are not a multiple of 8 pixels,
+    MSCS_GATHER=tma, MSCS_DENSE=0 -- converts the maps to fp32 first and the gradients back afterwards."""
+    if not fast_path_ok(sp.spec, world):
+        return False
+    return sp.nhwc or (all(sp.slot_sizes) and _DENSE_ONE_PASS and not _GATHER_TMA)
+
+
+def _dense_grad_slab(shapes, dtypes, dev):
+    """ONE allocation for the dense gradients of the one-pass writer and its pixel-mask words behind them: the
+    per-scale gradient views (dtype `dtypes[j]`), their byte offsets, and the byte offset of the mask.  Planes are a
+    multiple of 8 pixels, so every part starts 16-byte aligned (the writer's 16-byte stores)."""
+    nbytes = [shp[0] * shp[1] * shp[2] * shp[3] * dt.itemsize for shp, dt in zip(shapes, dtypes)]
+    mask_words = sum((shp[0] * shp[2] * shp[3] + 31) // 32 for shp in shapes)
+    slab = torch.empty(sum(nbytes) + 4 * mask_words, dtype=torch.uint8, device=dev)    # gradients | pixel mask
+    views, offs, off = [], [], 0
+    for shp, dt, nb in zip(shapes, dtypes, nbytes):
+        views.append(slab[off:off + nb].view(dt).view(shp))
+        offs.append(off)
+        off += nb
+    return slab, views, offs, off
+
+
 _hp_streams = {}
 
 
@@ -1005,6 +1034,7 @@ class _Workspace:
 class _StepState:
     """Buffers of one call (kept alive for the backward)."""
     entry = None
+    io_dtypes = None        # dtypes of the maps the kernels read and of the gradients they write (None: all fp32)
 
     def __del__(self):
         e, self.entry = self.entry, None
@@ -1013,12 +1043,14 @@ class _StepState:
 
 
 def run_forward(sp, labels, feats32, needs, comm=None, philox=None):
-    """philox: None (reference stream: torch CPU generator) or (seed, call index) of the opt-in counter-based stream."""
+    """philox: None (reference stream: torch CPU generator) or (seed, call index) of the opt-in counter-based stream.
+    feats32: fp32 maps, or bf16 / fp16 ones where half_io_ok(sp, world) holds (fast path only)."""
     pooled = comm is not None and comm.world > 1
     # device-driven order (selection, gather and similarity forward enqueued before the host sees the plan): single
     # process, every plane a multiple of 8 pixels (slot maps), selection shared memory within limits
     if fast_path_ok(sp.spec, 1 if not pooled else comm.world) and (sp.nhwc or all(x != 0 for x in sp.slot_sizes)):
         return _run_forward_fast(sp, labels, feats32, needs, philox)
+    assert all(f.dtype == torch.float32 for f in feats32), "half maps are converted by the caller off the fast path"
     assert not sp.nhwc, "channels-last inputs are converted by the caller unless the fast path applies"
     if philox is not None:
         raise NotImplementedError("sampler='philox' is implemented for the single-process path with feature planes "
@@ -1094,7 +1126,7 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     _t = _seg("fwd: grad buffers", _t)
     ch.labels, ch.labels_i16 = labels.data_ptr(), int(labels.dtype == torch.int16)
     for s in range(S):
-        e.gitems[s].feat = feats32[s].data_ptr()
+        e.gitems[s].feat, e.gitems[s].dtype = feats32[s].data_ptr(), _DTYPE_CODE[feats32[s].dtype]
     # gradient-row accumulators of the backward: cleared by the chain on the caller's stream, next to the sampling
     # kernels, when the one-pass dense writer will be used (otherwise they come pre-zeroed with the dense gradients, or
     # no gradient is wanted at all)
@@ -1104,15 +1136,12 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     # plan, with the addresses entered into the backward's prebuilt structures -- not in the window after the wait
     grad_slab = grad_outs = None
     if dF_in_ws and all(needs) and not sp.nhwc:
-        sizes = [f.numel() for f in feats32]
-        mask_words = sum((f.shape[0] * f.shape[2] * f.shape[3] + 31) // 32 for f in feats32)
-        grad_slab = torch.empty(sum(sizes) + mask_words, dtype=torch.float32, device=dev)    # gradients | pixel mask
-        sbase, off, grad_outs = grad_slab.data_ptr(), 0, []
+        grad_slab, grad_outs, offs, mask_off = _dense_grad_slab([f.shape for f in feats32], [f.dtype for f in feats32],
+                                                                dev)
+        sbase = grad_slab.data_ptr()
         for j in range(S):
-            grad_outs.append(grad_slab[off:off + sizes[j]].view(feats32[j].shape))
-            e.bw_items[j].dfeat = sbase + 4 * off
-            off += sizes[j]
-        grad_mask_ptr = sbase + 4 * off
+            e.bw_items[j].dfeat, e.bw_items[j].dtype = sbase + offs[j], _DTYPE_CODE[feats32[j].dtype]
+        grad_mask_ptr = sbase + mask_off
     evs = None
     if TIMING is not None and TIMING_ALL:      # stage accounting (bench.py): five events recorded INSIDE the chain
         evs = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
@@ -1156,6 +1185,7 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     state.dF_ws = e.dF_ptr if dF_in_ws else None
     state.grad_slab, state.grad_outs = grad_slab, grad_outs
     state.grad_mask_ptr = grad_mask_ptr if grad_slab is not None else None
+    state.io_dtypes = [f.dtype for f in feats32]
     for s in range(S):
         e.bw_rows[s] = samples[s].N
     return state
@@ -1483,6 +1513,7 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
         g = grad_out.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
     grads = []
     fbase = state.fslab.data_ptr()
+    io = state.io_dtypes or [torch.float32] * S         # dtypes the kernels write the dense gradients in
     dense = (not sp.nhwc) and state.gradbufs is None and \
         all((not needs[s]) or (state.slots[s] is not None) for s in range(S))
     if dense:
@@ -1495,23 +1526,20 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
             outs, mask_ptr = dict(enumerate(state.grad_outs)), state.grad_mask_ptr
             state.grad_outs = None
         else:
-            sizes = [shapes[s][0] * shapes[s][1] * shapes[s][2] * shapes[s][3] for s in idx]
-            mask_words = sum((shapes[s][0] * shapes[s][2] * shapes[s][3] + 31) // 32 for s in idx)
-            slab = torch.empty(sum(sizes) + mask_words, dtype=torch.float32, device=dev)    # gradients | pixel mask
+            slab, views, offs, mask_off = _dense_grad_slab([shapes[s] for s in idx], [io[s] for s in idx], dev)
             sbase = slab.data_ptr()
-            mask_ptr = sbase + 4 * sum(sizes)
-            outs, off = {}, 0
+            mask_ptr = sbase + mask_off
+            outs = {}
             items = (_lib.ScatterItem * max(1, len(idx)))()
             rows = (C.c_int32 * max(1, len(idx)))()
             for j, s in enumerate(idx):
                 n, Cc, h, w = shapes[s]
-                outs[s] = slab[off:off + sizes[j]].view(shapes[s])
+                outs[s] = views[j]
                 it = items[j]
                 it.dF, it.ldF, it.anc_f32, it.inv_norm = ptrs[s], sp.C_pad, fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
                 it.slot, it.n, it.C, it.plane = state.slots[s].data_ptr(), n, Cc, h * w
-                it.dfeat = sbase + 4 * off
+                it.dfeat, it.dtype = sbase + offs[j], _DTYPE_CODE[io[s]]
                 rows[j] = state.samples[s].N
-                off += sizes[j]
         evs, evp = None, None
         if TIMING is not None:
             evs = [torch.cuda.Event(enable_timing=True) for _ in range(3 if TIMING_ALL else 2)]
@@ -1525,7 +1553,7 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
             TIMING.setdefault("sim_bwd", []).append((evs[0], evs[1]))
             if len(evs) == 3:
                 TIMING.setdefault("scatter", []).append((evs[1], evs[2]))
-        return [None if not needs[s] else (outs[s] if dtypes[s] == torch.float32 else outs[s].to(dtypes[s]))
+        return [None if not needs[s] else (outs[s] if outs[s].dtype == dtypes[s] else outs[s].to(dtypes[s]))
                 for s in range(S)]
     with _timed("sim_bwd"):
         _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st),
@@ -1543,15 +1571,15 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
                 n, Cc, h, w = shapes[s]
                 pre = gb.take(s) if gb is not None else None
                 if pre is None:      # second backward through the same graph
-                    pre = torch.zeros((n, h, w, Cc), dtype=torch.float32, device=dev).permute(0, 3, 1, 2)
+                    pre = torch.zeros((n, h, w, Cc), dtype=io[s], device=dev).permute(0, 3, 1, 2)
                 outs[s] = pre
                 it = items[j]
                 it.pix, it.rows, it.C = state.samples[s].ptr(2), state.samples[s].N, Cc
                 it.anc_f32, it.inv_norm = fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
-                it.dF, it.ldF, it.dfeat = ptrs[s], sp.C_pad, pre.data_ptr()
+                it.dF, it.ldF, it.dfeat, it.dtype = ptrs[s], sp.C_pad, pre.data_ptr(), _DTYPE_CODE[io[s]]
             if idx:
                 _lib.check(lib.mscs_scatter_rows_nhwc_batch(items, len(idx), st), "mscs_scatter_rows_nhwc_batch")
-            return [None if not needs[s] else (outs[s] if dtypes[s] == torch.float32 else outs[s].to(dtypes[s]))
+            return [None if not needs[s] else (outs[s] if outs[s].dtype == dtypes[s] else outs[s].to(dtypes[s]))
                     for s in range(S)]
     with _timed("scatter"):
         gb = state.gradbufs
@@ -1608,24 +1636,27 @@ class MsCsContrastiveFn(torch.autograd.Function):
         world = comm.world if comm is not None else 1
         nhwc = fast_path_ok(spec, world) and all(
             f.dim() == 4 and f.is_contiguous(memory_format=torch.channels_last) and not f.is_contiguous() for f in feats)
-        feats32 = []
         for f in feats:
             _require_device(f)
-            f32 = f.detach()
-            if f32.dtype != torch.float32:
-                f32 = f32.float()
-            feats32.append(f32 if nhwc else f32.contiguous())
-        if labels.device != feats32[0].device:
-            labels = labels.to(feats32[0].device)
+        dev = feats[0].device
+        if labels.device != dev:
+            labels = labels.to(dev)
         needs = [bool(ctx.needs_input_grad[4 + i]) for i in range(len(feats))]
         if labels.dtype not in (torch.int64, torch.int16):     # int16: compact labels of the fused label pass
             labels = labels.long()
         labels = labels.contiguous()
-        with torch.cuda.device(feats32[0].device), _pin_stream():
+        with torch.cuda.device(dev), _pin_stream():
             world, rank = (comm.world, comm.rank) if comm is not None else (1, 0)
-            sp = _step_plan(feats32[0].device, labels.shape, [tuple(f.shape) for f in feats32], spec, single_scale,
-                            world, rank, nhwc)
-            state = run_forward(sp, labels, feats32, needs, comm, holder.get("philox"))
+            sp = _step_plan(dev, labels.shape, [tuple(f.shape) for f in feats], spec, single_scale, world, rank, nhwc)
+            # bf16 / fp16 maps go to the kernels as they are where half_io_ok holds; everything else as an fp32 copy
+            half_ok = half_io_ok(sp, world)
+            maps = []
+            for f in feats:
+                m = f.detach()
+                if m.dtype != torch.float32 and not (half_ok and m.dtype in _DTYPE_CODE):
+                    m = m.float()
+                maps.append(m if nhwc else m.contiguous())
+            state = run_forward(sp, labels, maps, needs, comm, holder.get("philox"))
         holder["samples"], holder["state"] = state.samples, state
         ctx.state, ctx.needs = state, needs
         ctx.shapes = [tuple(f.shape) for f in feats]

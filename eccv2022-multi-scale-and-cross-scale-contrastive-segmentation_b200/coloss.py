@@ -47,10 +47,13 @@ class _FusedCEFn(torch.autograd.Function):
     def forward(ctx, logits, compact, weight, ignore_index):
         lib = _lib.load()
         _ops._require_device(logits)
+        # fp32, bf16 and fp16 logits are read as they are (dlogits come back in the same dtype); others as an fp32 copy
         x = logits.detach()
-        if x.dtype != torch.float32:
+        if x.dtype not in _ops._DTYPE_CODE:
             x = x.float()
         x = x.contiguous()
+        if x.dtype != torch.float32 and x.data_ptr() % 8:      # a view at an odd offset: the kernels load 8 bytes
+            x = x.clone()
         n, K, H, W = x.shape
         if compact.shape != (n, H, W):
             raise ValueError(f"labels {compact.shape} do not match the logits {tuple(x.shape)}")
@@ -61,8 +64,8 @@ class _FusedCEFn(torch.autograd.Function):
         with torch.cuda.device(x.device):
             _lib.check(lib.mscs_ce_forward(x.data_ptr(), compact.lab16.data_ptr(), n, K, H * W,
                                            None if w is None else w.data_ptr(), int(ignore_index), compact.hist.data_ptr(),
-                                           compact.num_classes, scratch.data_ptr(), out.data_ptr(), _ops._stream()),
-                       "mscs_ce_forward")
+                                           compact.num_classes, scratch.data_ptr(), out.data_ptr(), _ops._stream(),
+                                           _ops._DTYPE_CODE[x.dtype]), "mscs_ce_forward")
             loss.copy_(out[0])
         ctx.x, ctx.compact, ctx.w, ctx.ignore, ctx.out, ctx.dtype = x, compact, w, int(ignore_index), out, logits.dtype
         return loss
@@ -77,8 +80,9 @@ class _FusedCEFn(torch.autograd.Function):
         with torch.cuda.device(x.device):
             _lib.check(lib.mscs_ce_backward(x.data_ptr(), ctx.compact.lab16.data_ptr(), n, K, H * W,
                                             None if ctx.w is None else ctx.w.data_ptr(), ctx.ignore, g.data_ptr(),
-                                            ctx.out[1:].data_ptr(), dx.data_ptr(), _ops._stream()), "mscs_ce_backward")
-        return (dx if ctx.dtype == torch.float32 else dx.to(ctx.dtype)), None, None, None
+                                            ctx.out[1:].data_ptr(), dx.data_ptr(), _ops._stream(),
+                                            _ops._DTYPE_CODE[x.dtype]), "mscs_ce_backward")
+        return (dx if dx.dtype == ctx.dtype else dx.to(ctx.dtype)), None, None, None
 
 
 class CrossEntropyLabelPass(nn.Module):

@@ -13,7 +13,8 @@
 // three times the traffic):
 //   k_ce_fwd   loss_sum = sum_valid w[y] (logsumexp(x) - x_y)          reads the logits once
 //   k_ce_bwd   dx_k = (g / denom) w[y] (softmax_k - [k == y]), 0 on ignored pixels   reads once (+L1), writes once
-// thread = 4 consecutive pixels (float4 per class plane), online max / sum over the classes.
+// thread = 4 consecutive pixels (float4 per class plane, 8 bytes for bf16 / fp16 logits), online max / sum over the
+// classes.  Half logits are widened on load and dlogits rounded on store; the arithmetic is the fp32 kernel's.
 #include "common.cuh"
 
 namespace mscs {
@@ -71,17 +72,18 @@ __global__ void k_ce_finalize(const int* __restrict__ hist, const float* __restr
 }
 
 struct CeArgs {
-  const float* logits; const short* lab16; const float* weight;
+  const void* logits; const short* lab16; const float* weight;
   int K, plane, ignore; long long n_quads;      // quads of 4 consecutive pixels (plane % 4 == 0)
 };
 
 // online (max, sum exp) over the class planes of 4 consecutive pixels
-__device__ __forceinline__ void ce_stats(const float* __restrict__ base, int K, size_t plane, float (&mx)[4], float (&se)[4]) {
+template <typename T>
+__device__ __forceinline__ void ce_stats(const T* __restrict__ base, int K, size_t plane, float (&mx)[4], float (&se)[4]) {
 #pragma unroll
   for (int q = 0; q < 4; ++q) { mx[q] = -INFINITY; se[q] = 0.f; }
   for (int k = 0; k < K; ++k) {
-    const float4 x = *reinterpret_cast<const float4*>(base + (size_t)k * plane);
-    const float xv[4] = {x.x, x.y, x.z, x.w};
+    float xv[4];
+    ld4(base + (size_t)k * plane, xv);
 #pragma unroll
     for (int q = 0; q < 4; ++q) {      // one exponential per element (accurate expf: the kernels are HBM-bound)
       const float d = xv[q] - mx[q];
@@ -91,6 +93,7 @@ __device__ __forceinline__ void ce_stats(const float* __restrict__ base, int K, 
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256) k_ce_fwd(const __grid_constant__ CeArgs a, double* __restrict__ loss_sum) {
   __shared__ double red[8];
   double part = 0.0;
@@ -104,13 +107,13 @@ __global__ void __launch_bounds__(256) k_ce_fwd(const __grid_constant__ CeArgs a
 #pragma unroll
     for (int q = 0; q < 4; ++q) any = any || (y[q] >= 0 && y[q] < a.K && y[q] != a.ignore);
     if (any) {
-      const float* base = a.logits + (size_t)b * a.K * a.plane + p;
+      const T* base = static_cast<const T*>(a.logits) + (size_t)b * a.K * a.plane + p;
       float mx[4], se[4];
       ce_stats(base, a.K, (size_t)a.plane, mx, se);
 #pragma unroll
       for (int q = 0; q < 4; ++q)
         if (y[q] >= 0 && y[q] < a.K && y[q] != a.ignore) {
-          const float xy = base[(size_t)y[q] * a.plane + q];
+          const float xy = to_f32(base[(size_t)y[q] * a.plane + q]);
           const float w = a.weight ? a.weight[y[q]] : 1.f;
           part += (double)(w * (mx[q] + logf(se[q]) - xy));
         }
@@ -127,9 +130,10 @@ __global__ void __launch_bounds__(256) k_ce_fwd(const __grid_constant__ CeArgs a
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
 k_ce_bwd(const __grid_constant__ CeArgs a, const float* __restrict__ grad_out, const float* __restrict__ denom,
-         float* __restrict__ dlogits) {
+         T* __restrict__ dlogits) {
   const long long quad = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (quad >= a.n_quads) return;
   const long long pix = quad * 4;
@@ -137,8 +141,8 @@ k_ce_bwd(const __grid_constant__ CeArgs a, const float* __restrict__ grad_out, c
   const short4 y4 = *reinterpret_cast<const short4*>(a.lab16 + pix);
   const int y[4] = {y4.x, y4.y, y4.z, y4.w};
   const size_t off = (size_t)b * a.K * a.plane + p;
-  const float* base = a.logits + off;
-  float* out = dlogits + off;
+  const T* base = static_cast<const T*>(a.logits) + off;
+  T* out = dlogits + off;
   float coef[4];
   bool any = false;
   const float g = *grad_out / *denom;
@@ -149,7 +153,8 @@ k_ce_bwd(const __grid_constant__ CeArgs a, const float* __restrict__ grad_out, c
     any = any || ok;
   }
   if (!any) {      // four ignored pixels: zeros, the logits are not read
-    for (int k = 0; k < a.K; ++k) __stcs(reinterpret_cast<float4*>(out + (size_t)k * a.plane), make_float4(0.f, 0.f, 0.f, 0.f));
+    const float z[4] = {0.f, 0.f, 0.f, 0.f};
+    for (int k = 0; k < a.K; ++k) st4_cs(out + (size_t)k * a.plane, z);
     return;
   }
   float mx[4], se[4];
@@ -158,12 +163,12 @@ k_ce_bwd(const __grid_constant__ CeArgs a, const float* __restrict__ grad_out, c
 #pragma unroll
   for (int q = 0; q < 4; ++q) inv[q] = coef[q] / se[q];
   for (int k = 0; k < a.K; ++k) {
-    const float4 x = *reinterpret_cast<const float4*>(base + (size_t)k * a.plane);      // second read: L1 / L2
-    const float xv[4] = {x.x, x.y, x.z, x.w};
+    float xv[4];
+    ld4(base + (size_t)k * a.plane, xv);      // second read: L1 / L2
     float r[4];
 #pragma unroll
     for (int q = 0; q < 4; ++q) r[q] = expf(xv[q] - mx[q]) * inv[q] - (k == y[q] ? coef[q] : 0.f);
-    __stcs(reinterpret_cast<float4*>(out + (size_t)k * a.plane), make_float4(r[0], r[1], r[2], r[3]));
+    st4_cs(out + (size_t)k * a.plane, r);
   }
 }
 
@@ -186,39 +191,50 @@ extern "C" int mscs_label_pass(const int64_t* labels, int64_t n_pixels, int num_
   return 0;
 }
 
-static int ce_args(CeArgs* a, const float* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
-                   int ignore_index) {
+static int ce_args(CeArgs* a, const void* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
+                   int ignore_index, int dtype) {
   MSCS_CHECK_ARG(logits && lab16, "null pointer argument");
+  MSCS_CHECK_ARG(dtype_bytes(dtype) > 0, "dtype %d unknown (MSCS_DTYPE_F32 / _BF16 / _F16)", dtype);
   MSCS_CHECK_ARG(n >= 1 && K >= 1 && K <= kCeMaxClasses && plane >= 4 && plane % 4 == 0,
                  "unsupported shape (n %d, K %d, plane %d: the plane must be a multiple of 4 pixels)", n, K, plane);
-  MSCS_CHECK_ARG((uintptr_t)logits % 16 == 0 && (uintptr_t)lab16 % 8 == 0, "logits / labels must be 16 / 8 byte aligned");
+  const int al = 4 * dtype_bytes(dtype);      // one load / store of 4 pixels
+  MSCS_CHECK_ARG((uintptr_t)logits % al == 0 && (uintptr_t)lab16 % 8 == 0, "logits / labels must be %d / 8 byte aligned",
+                 al);
   a->logits = logits; a->lab16 = lab16; a->weight = weight; a->K = K; a->plane = plane; a->ignore = ignore_index;
   a->n_quads = (long long)n * plane / 4;
   return 0;
 }
 
-extern "C" int mscs_ce_forward(const float* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
+extern "C" int mscs_ce_forward(const void* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
                                int ignore_index, const int32_t* hist, int num_classes, double* loss_sum_scratch,
-                               float* loss_and_denom, void* stream_) {
+                               float* loss_and_denom, void* stream_, int dtype) {
   CeArgs a;
-  if (int rc = ce_args(&a, logits, lab16, n, K, plane, weight, ignore_index)) return rc;
+  if (int rc = ce_args(&a, logits, lab16, n, K, plane, weight, ignore_index, dtype)) return rc;
   MSCS_CHECK_ARG(hist && loss_sum_scratch && loss_and_denom && num_classes >= 1, "null pointer argument");
   cudaStream_t st = (cudaStream_t)stream_;
   MSCS_CUDA(cudaMemsetAsync(loss_sum_scratch, 0, sizeof(double), st));
-  k_ce_fwd<<<(unsigned)((a.n_quads + 255) / 256), 256, 0, st>>>(a, loss_sum_scratch);
+  const unsigned grid = (unsigned)((a.n_quads + 255) / 256);
+  if (dtype == MSCS_DTYPE_F32) k_ce_fwd<float><<<grid, 256, 0, st>>>(a, loss_sum_scratch);
+  else if (dtype == MSCS_DTYPE_BF16) k_ce_fwd<__nv_bfloat16><<<grid, 256, 0, st>>>(a, loss_sum_scratch);
+  else k_ce_fwd<__half><<<grid, 256, 0, st>>>(a, loss_sum_scratch);
   MSCS_LAUNCH_CHECK();
   k_ce_finalize<<<1, 32, 0, st>>>(hist, weight, K, num_classes, ignore_index, loss_sum_scratch, loss_and_denom);
   MSCS_LAUNCH_CHECK();
   return 0;
 }
 
-extern "C" int mscs_ce_backward(const float* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
-                                int ignore_index, const float* grad_out, const float* denom, float* dlogits,
-                                void* stream_) {
+extern "C" int mscs_ce_backward(const void* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
+                                int ignore_index, const float* grad_out, const float* denom, void* dlogits,
+                                void* stream_, int dtype) {
   CeArgs a;
-  if (int rc = ce_args(&a, logits, lab16, n, K, plane, weight, ignore_index)) return rc;
-  MSCS_CHECK_ARG(grad_out && denom && dlogits && (uintptr_t)dlogits % 16 == 0, "null / misaligned pointer argument");
-  k_ce_bwd<<<(unsigned)((a.n_quads + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(a, grad_out, denom, dlogits);
+  if (int rc = ce_args(&a, logits, lab16, n, K, plane, weight, ignore_index, dtype)) return rc;
+  MSCS_CHECK_ARG(grad_out && denom && dlogits && (uintptr_t)dlogits % (4 * dtype_bytes(dtype)) == 0,
+                 "null / misaligned pointer argument");
+  cudaStream_t st = (cudaStream_t)stream_;
+  const unsigned grid = (unsigned)((a.n_quads + 255) / 256);
+  if (dtype == MSCS_DTYPE_F32) k_ce_bwd<float><<<grid, 256, 0, st>>>(a, grad_out, denom, (float*)dlogits);
+  else if (dtype == MSCS_DTYPE_BF16) k_ce_bwd<__nv_bfloat16><<<grid, 256, 0, st>>>(a, grad_out, denom, (__nv_bfloat16*)dlogits);
+  else k_ce_bwd<__half><<<grid, 256, 0, st>>>(a, grad_out, denom, (__half*)dlogits);
   MSCS_LAUNCH_CHECK();
   return 0;
 }

@@ -88,8 +88,9 @@ k_scatter_grad(const float* __restrict__ dF, int ldF, const float* __restrict__ 
 // Gather in ADDRESS order: one warp per 8-pixel octet of the slot map (18% of them hold a sampled
 // pixel at cfg-2).  Neighbouring warps then touch neighbouring 32-byte sectors of the same channel
 // planes, so the 256 strided sector reads of an anchor hit open DRAM pages instead of random ones.
+template <typename T>
 __device__ __forceinline__ void
-gather_sectors_body(int block, int nblocks, const float* __restrict__ feat, int C, int C_pad, int plane,
+gather_sectors_body(int block, int nblocks, const T* __restrict__ feat, int C, int C_pad, int plane,
                     const int* __restrict__ slot, int n_octets, __nv_bfloat16* __restrict__ anc_bf16,
                     float* __restrict__ anc_f32, float* __restrict__ inv_norm, const int* __restrict__ n_rows_dev) {
   const int lane = threadIdx.x & 31;
@@ -108,18 +109,18 @@ gather_sectors_body(int block, int nblocks, const float* __restrict__ feat, int 
   unsigned act = __ballot_sync(0xffffffffu, s_mine >= 0);
   if (act == 0) return;
   const int b = gp / plane, p = gp - b * plane;
-  const float* src0 = feat + ((size_t)b * C) * plane + p;
+  const T* src0 = feat + ((size_t)b * C) * plane + p;
   while (act) {
     const int j = __ffs(act) - 1;
     act &= act - 1;
     const int row = __shfl_sync(0xffffffffu, s_mine, j);
-    const float* src = src0 + j;
+    const T* src = src0 + j;
     float v[kMaxC / 32];
     float ss = 0.f;
 #pragma unroll
     for (int q = 0; q < kMaxC / 32; ++q) {
       const int c = lane + 32 * q;
-      v[q] = (c < C) ? __ldg(src + (size_t)c * plane) : 0.f;
+      v[q] = (c < C) ? to_f32(__ldg(src + (size_t)c * plane)) : 0.f;
     }
 #pragma unroll
     for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q], v[q], ss);
@@ -150,23 +151,25 @@ k_gather_sectors(const float* __restrict__ feat, int C, int C_pad, int plane, co
                  int n_octets, __nv_bfloat16* __restrict__ anc_bf16, float* __restrict__ anc_f32,
                  float* __restrict__ inv_norm, const int* __restrict__ n_rows_dev) {
   pdl_trigger();
-  gather_sectors_body(blockIdx.x, gridDim.x, feat, C, C_pad, plane, slot, n_octets, anc_bf16, anc_f32, inv_norm,
+  gather_sectors_body<float>(blockIdx.x, gridDim.x, feat, C, C_pad, plane, slot, n_octets, anc_bf16, anc_f32, inv_norm,
                       n_rows_dev);
 }
 
 // all scales of a call in ONE launch (the per-scale launches of the small scales do not fill the GPU and each
-// costs a launch gap): block -> scale through the block prefix
+// costs a launch gap): block -> scale through the block prefix.  One instantiation per element type of the maps; a
+// call that mixes types launches once per type present.
 struct GatherBatch {
-  const float* feat[MSCS_MAX_SCALES]; const int* slot[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
+  const void* feat[MSCS_MAX_SCALES]; const int* slot[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
   __nv_bfloat16* bf16[MSCS_MAX_SCALES]; float* f32[MSCS_MAX_SCALES]; float* inv[MSCS_MAX_SCALES];
   int C[MSCS_MAX_SCALES], plane[MSCS_MAX_SCALES], n_oct[MSCS_MAX_SCALES], block0[MSCS_MAX_SCALES + 1];
   int count;
 };
+template <typename T>
 __global__ void __launch_bounds__(256) k_gather_sectors_batch(const __grid_constant__ GatherBatch g) {
   pdl_trigger();      // the next kernel of the forward (k_row_ranges) is launched programmatically, see common.cuh
   int s = 0;
   while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
-  gather_sectors_body(blockIdx.x - g.block0[s], g.block0[s + 1] - g.block0[s], g.feat[s], g.C[s],
+  gather_sectors_body<T>(blockIdx.x - g.block0[s], g.block0[s + 1] - g.block0[s], static_cast<const T*>(g.feat[s]), g.C[s],
                       (g.C[s] + 63) / 64 * 64, g.plane[s], g.slot[s], g.n_oct[s], g.bf16[s], g.f32[s], g.inv[s],
                       g.n_rows_dev[s]);
 }
@@ -476,13 +479,14 @@ __global__ void __launch_bounds__(256) k_dense_write(const __grid_constant__ Den
 // l + 32 q -- the same lane/channel assignment as the NCHW kernels, so the results are bit-identical.
 // ---------------------------------------------------------------------------------------
 struct RowsBatch {
-  const float* feat[MSCS_MAX_SCALES]; const int* pix[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
+  const void* feat[MSCS_MAX_SCALES]; const int* pix[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
   __nv_bfloat16* bf16[MSCS_MAX_SCALES]; float* f32[MSCS_MAX_SCALES]; float* inv[MSCS_MAX_SCALES];
-  const float* dF[MSCS_MAX_SCALES]; float* dfeat[MSCS_MAX_SCALES];
+  const float* dF[MSCS_MAX_SCALES]; void* dfeat[MSCS_MAX_SCALES];
   int C[MSCS_MAX_SCALES], ldF[MSCS_MAX_SCALES], rows[MSCS_MAX_SCALES], block0[MSCS_MAX_SCALES + 1];
   int count;
 };
 
+template <typename T>
 __global__ void __launch_bounds__(256) k_gather_rows_nhwc(const __grid_constant__ RowsBatch g) {
   pdl_trigger();
   int s = 0;
@@ -498,13 +502,13 @@ __global__ void __launch_bounds__(256) k_gather_rows_nhwc(const __grid_constant_
     for (int c = lane; c < C_pad; c += 32) orow[c] = __float2bfloat16(0.f);
     return;
   }
-  const float* src = g.feat[s] + (size_t)gp * C;
+  const T* src = static_cast<const T*>(g.feat[s]) + (size_t)gp * C;
   float v[kMaxC / 32];
   float ss = 0.f;
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
-    v[q] = (c < C) ? __ldg(src + c) : 0.f;
+    v[q] = (c < C) ? to_f32(__ldg(src + c)) : 0.f;
   }
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q], v[q], ss);
@@ -521,6 +525,7 @@ __global__ void __launch_bounds__(256) k_gather_rows_nhwc(const __grid_constant_
 }
 
 // normalisation backward + row store into the (pre-zeroed) channels-last dense gradient
+template <typename T>
 __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant__ RowsBatch g) {
   int s = 0;
   while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
@@ -543,11 +548,11 @@ __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant
   dot = warp_sum(dot);
   const float inv = g.inv[s][row];
   const bool clamped = inv >= 1e12f;        // ||x|| <= eps: F.normalize divides by the constant eps
-  float* dst = g.dfeat[s] + (size_t)gp * C;
+  T* dst = static_cast<T*>(g.dfeat[s]) + (size_t)gp * C;
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
-    if (c < C) dst[c] = (clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv;
+    if (c < C) dst[c] = from_f32<T>((clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv);
   }
 }
 
@@ -556,34 +561,40 @@ __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant
 // invariant: 97 % of the threads run a pure store loop, the others add up to four independent (predicated) loads of
 // dx[row][c] per channel.  A block writes 2 KB contiguous per channel plane (512 pixels), i.e. whole DRAM pages in
 // linear order per plane -- the order of the memset it replaces, without its second pass over the sampled sectors.
+// Half gradients: a thread owns 8 pixels (two int4 of slot entries, up to eight loads per channel) so that every store
+// is still 16 bytes; a block then covers 1024 pixels.  (The fast path guarantees planes that are a multiple of 8.)
 struct DenseStream {
-  const float* dx[MSCS_MAX_SCALES]; const int* slot[MSCS_MAX_SCALES]; float* dfeat[MSCS_MAX_SCALES];
+  const float* dx[MSCS_MAX_SCALES]; const int* slot[MSCS_MAX_SCALES]; void* dfeat[MSCS_MAX_SCALES];
   int ld[MSCS_MAX_SCALES], C[MSCS_MAX_SCALES], plane[MSCS_MAX_SCALES], npix[MSCS_MAX_SCALES], blk0[MSCS_MAX_SCALES + 1];
   int count;
 };
+template <typename T>
 __global__ void __launch_bounds__(128) k_dense_stream(const __grid_constant__ DenseStream g) {
+  constexpr int P = 16 / sizeof(T);      // pixels per thread: one 16-byte store per channel plane
   int s = 0;
   while (s + 1 < g.count && (int)blockIdx.x >= g.blk0[s + 1]) ++s;
-  const int lin = (((int)blockIdx.x - g.blk0[s]) * 128 + (int)threadIdx.x) * 4;
+  const int lin = (((int)blockIdx.x - g.blk0[s]) * 128 + (int)threadIdx.x) * P;
   if (lin >= g.npix[s]) return;
   const int plane = g.plane[s], C = g.C[s], ld = g.ld[s];
-  const int4 sl = *reinterpret_cast<const int4*>(g.slot[s] + lin);
+  int sl[P];
+#pragma unroll
+  for (int i = 0; i < P; i += 4) {
+    const int4 q = *reinterpret_cast<const int4*>(g.slot[s] + lin + i);
+    sl[i] = q.x; sl[i + 1] = q.y; sl[i + 2] = q.z; sl[i + 3] = q.w;
+  }
   const int b = lin / plane, p = lin - b * plane;
-  float* __restrict__ out = g.dfeat[s] + ((size_t)b * C) * plane + p;
+  T* __restrict__ out = static_cast<T*>(g.dfeat[s]) + ((size_t)b * C) * plane + p;
   const float* __restrict__ dx = g.dx[s];
-  const float* r0 = dx + (size_t)max(sl.x, 0) * ld;
-  const float* r1 = dx + (size_t)max(sl.y, 0) * ld;
-  const float* r2 = dx + (size_t)max(sl.z, 0) * ld;
-  const float* r3 = dx + (size_t)max(sl.w, 0) * ld;
-  const bool h0 = sl.x >= 0, h1 = sl.y >= 0, h2 = sl.z >= 0, h3 = sl.w >= 0;
+  const float* r[P];
+  bool h[P];
+#pragma unroll
+  for (int i = 0; i < P; ++i) { r[i] = dx + (size_t)max(sl[i], 0) * ld; h[i] = sl[i] >= 0; }
 #pragma unroll 8
   for (int c = 0; c < C; ++c) {
-    float4 v;
-    v.x = h0 ? __ldg(r0 + c) : 0.f;
-    v.y = h1 ? __ldg(r1 + c) : 0.f;
-    v.z = h2 ? __ldg(r2 + c) : 0.f;
-    v.w = h3 ? __ldg(r3 + c) : 0.f;
-    __stcs(reinterpret_cast<float4*>(out + (size_t)c * plane), v);
+    float v[P];
+#pragma unroll
+    for (int i = 0; i < P; ++i) v[i] = h[i] ? __ldg(r[i] + c) : 0.f;
+    st16_cs(out + (size_t)c * plane, v);
   }
 }
 
@@ -693,30 +704,54 @@ extern "C" int mscs_scatter_sectors_pull(void* const* slabs, int world, size_t d
   return 0;
 }
 
+// element-type checks shared by the batched entry points: a known MSCS_DTYPE_* code and an address aligned to `align`
+// bytes (at least the element size)
+static int check_dtype(int s, int dtype, const void* p, int align, const char* what) {
+  MSCS_CHECK_ARG(dtype_bytes(dtype) > 0, "item %d: dtype %d unknown (MSCS_DTYPE_F32 / _BF16 / _F16)", s, dtype);
+  const int a = align > dtype_bytes(dtype) ? align : dtype_bytes(dtype);
+  MSCS_CHECK_ARG((uintptr_t)p % a == 0, "item %d: %s must be %d-byte aligned", s, what, a);
+  return 0;
+}
+
+// the items of one element type, one launch
+template <typename T>
+static int gather_sectors_launch(const mscs_gather_item* items, int count, int dtype, cudaStream_t st) {
+  GatherBatch g{};
+  int blocks = 0;
+  for (int s = 0; s < count; ++s) {
+    const mscs_gather_item& it = items[s];
+    if (it.dtype != dtype) continue;
+    const int j = g.count++;
+    g.feat[j] = it.feat; g.slot[j] = it.slot; g.n_rows_dev[j] = it.n_rows_dev;
+    g.bf16[j] = (__nv_bfloat16*)it.anc_bf16; g.f32[j] = it.anc_f32; g.inv[j] = it.inv_norm;
+    g.C[j] = it.C; g.plane[j] = it.plane; g.n_oct[j] = it.n * (it.plane / 8);
+  }
+  if (g.count == 0) return 0;
+  for (int j = 0; j < g.count; ++j) {
+    g.block0[j] = blocks;
+    blocks += ceil_div(g.n_oct[j], 8) + 1;      // + the block that zeroes the padding rows
+  }
+  g.block0[g.count] = blocks;
+  k_gather_sectors_batch<T><<<blocks, 256, 0, st>>>(g);
+  MSCS_LAUNCH_CHECK();
+  return 0;
+}
+
 // One launch for every scale of a call (see mscs.h)
 extern "C" int mscs_gather_normalize_sectors_batch(const mscs_gather_item* items, int count, void* stream_) {
   MSCS_CHECK_ARG(items && count >= 1 && count <= MSCS_MAX_SCALES, "bad item count %d", count);
-  GatherBatch g{};
-  g.count = count;
-  int blocks = 0;
   for (int s = 0; s < count; ++s) {
     const mscs_gather_item& it = items[s];
     MSCS_CHECK_ARG(it.feat && it.slot && it.n_rows_dev && it.anc_bf16 && it.anc_f32 && it.inv_norm,
                    "item %d: null pointer argument", s);
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC, "item %d: C=%d unsupported (1..%d)", s, it.C, kMaxC);
     MSCS_CHECK_ARG(it.n >= 1 && it.plane >= 8 && it.plane % 8 == 0, "item %d: plane must be a multiple of 8", s);
-    g.feat[s] = it.feat; g.slot[s] = it.slot; g.n_rows_dev[s] = it.n_rows_dev;
-    g.bf16[s] = (__nv_bfloat16*)it.anc_bf16; g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm;
-    g.C[s] = it.C; g.plane[s] = it.plane; g.n_oct[s] = it.n * (it.plane / 8);
+    if (int rc = check_dtype(s, it.dtype, it.feat, 1, "feat")) return rc;
   }
-  for (int s = 0; s < count; ++s) {
-    g.block0[s] = blocks;
-    blocks += ceil_div(g.n_oct[s], 8) + 1;      // + the block that zeroes the padding rows
-  }
-  g.block0[count] = blocks;
-  k_gather_sectors_batch<<<blocks, 256, 0, (cudaStream_t)stream_>>>(g);
-  MSCS_LAUNCH_CHECK();
-  return 0;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (int rc = gather_sectors_launch<float>(items, count, MSCS_DTYPE_F32, st)) return rc;
+  if (int rc = gather_sectors_launch<__nv_bfloat16>(items, count, MSCS_DTYPE_BF16, st)) return rc;
+  return gather_sectors_launch<__half>(items, count, MSCS_DTYPE_F16, st);
 }
 
 // the same gather through bulk-tensor copies (k_gather_tma_batch)
@@ -732,6 +767,8 @@ extern "C" int mscs_gather_normalize_tma_batch(const mscs_gather_item* items, in
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC, "item %d: C=%d unsupported (1..%d)", s, it.C, kMaxC);
     MSCS_CHECK_ARG(it.n >= 1 && it.plane >= 8 && it.plane % 8 == 0, "item %d: plane must be a multiple of 8", s);
     MSCS_CHECK_ARG((uintptr_t)it.feat % 16 == 0, "item %d: feature map must be 16-byte aligned", s);
+    if (int rc = check_dtype(s, it.dtype, it.feat, 16, "feat")) return rc;
+    MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32, "item %d: the TMA gather reads fp32 feature maps only", s);
     if (make_tensor_map_2d(&g.map[s], (int)CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, it.feat, (unsigned long long)it.plane,
                            (unsigned long long)it.n * it.C, (unsigned long long)it.plane * 4, 8, (unsigned)it.C))
       return -1;
@@ -776,7 +813,9 @@ extern "C" int mscs_scatter_sectors_batch(const mscs_scatter_item* items, int co
     MSCS_CHECK_ARG(it.dF && it.anc_f32 && it.inv_norm && it.slot && it.dfeat, "item %d: null pointer argument", s);
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC && it.ldF >= it.C, "item %d: C=%d / ldF=%d unsupported", s, it.C, it.ldF);
     MSCS_CHECK_ARG(it.plane % 8 == 0, "item %d: plane %d is not a multiple of 8 pixels", s, it.plane);
-    g.dF[s] = it.dF; g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot; g.dfeat[s] = it.dfeat;
+    if (int rc = check_dtype(s, it.dtype, it.dfeat, 16, "dfeat")) return rc;
+    MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32, "item %d: the sector scatter writes fp32 gradients only", s);
+    g.dF[s] = it.dF; g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot; g.dfeat[s] = (float*)it.dfeat;
     g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n_oct[s] = it.n * (it.plane / 8);
     g.block0[s] = blocks;
     blocks += ceil_div(g.n_oct[s], 8);
@@ -812,6 +851,25 @@ extern "C" int mscs_scatter_grad(const float* dF, int ldF, const float* anc_f32,
   return 0;
 }
 
+// the dense writer over the items of one element type (128 threads x 16 / sizeof(T) pixels per block)
+template <typename T>
+static int dense_stream_launch(const DenseBatch& g, const mscs_scatter_item* items, int dtype, cudaStream_t st) {
+  DenseStream d{};
+  int blk = 0;
+  for (int s = 0; s < g.count; ++s) {
+    if (items[s].dtype != dtype) continue;
+    const int j = d.count++;
+    d.dx[j] = g.dF[s]; d.slot[j] = g.slot[s]; d.dfeat[j] = items[s].dfeat; d.ld[j] = g.ldF[s]; d.C[j] = g.C[s];
+    d.plane[j] = g.plane[s]; d.npix[j] = g.n[s] * g.plane[s]; d.blk0[j] = blk;
+    blk += ceil_div(d.npix[j], 128 * (16 / (int)sizeof(T)));
+  }
+  if (d.count == 0) return 0;
+  d.blk0[d.count] = blk;
+  k_dense_stream<T><<<blk, 128, 0, st>>>(d);
+  MSCS_LAUNCH_CHECK();
+  return 0;
+}
+
 extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count,
                                         uint32_t* mask_scratch, void* stream_) {
   MSCS_CHECK_ARG(items && rows && mask_scratch && count >= 1 && count <= MSCS_MAX_SCALES, "bad arguments");
@@ -825,8 +883,11 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
     MSCS_CHECK_ARG(it.dF && it.anc_f32 && it.inv_norm && it.slot && it.dfeat, "item %d: null pointer argument", s);
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC && it.ldF >= it.C, "item %d: C=%d / ldF=%d unsupported", s, it.C, it.ldF);
     MSCS_CHECK_ARG(it.plane % 4 == 0 && rows[s] >= 0, "item %d: plane %d is not a multiple of 4 pixels", s, it.plane);
+    if (int rc = check_dtype(s, it.dtype, it.dfeat, 16, "dfeat")) return rc;
+    MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32 || it.plane % 8 == 0,
+                   "item %d: half gradients need a plane that is a multiple of 8 pixels (plane %d)", s, it.plane);
     g.dF[s] = const_cast<float*>(it.dF); g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot;
-    g.dfeat[s] = it.dfeat; g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = rows[s];
+    g.dfeat[s] = (float*)it.dfeat; g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = rows[s];
     MSCS_CHECK_ARG((long long)it.n * it.C * it.plane < (1ll << 32), "item %d: more than 2^32 gradient elements", s);
     g.v4_0[s] = v4;      // block prefix: 2048 floats per block
     v4 += ((long long)it.n * it.C * it.plane + 2047) / 2048;
@@ -840,6 +901,8 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
   cudaStream_t st = (cudaStream_t)stream_;
   static const int writer = [] { const char* e = getenv("MSCS_DENSE_WRITER"); return e ? atoi(e) : 1; }();
   if (writer == 0) {      // first form (round 1): linear float4 walk with a pixel mask
+    for (int s = 0; s < count; ++s)
+      MSCS_CHECK_ARG(items[s].dtype == MSCS_DTYPE_F32, "item %d: MSCS_DENSE_WRITER=0 writes fp32 gradients only", s);
     k_dx_rows<<<rb + mblk, 256, 0, st>>>(g);
     MSCS_LAUNCH_CHECK();
     k_dense_write<<<(unsigned)v4, 256, 0, st>>>(g);
@@ -849,58 +912,59 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
   g.maskblk0[count] = 0;      // no mask blocks: k_dx_rows only turns the gradient rows into dx rows
   k_dx_rows<<<rb > 0 ? rb : 1, 256, 0, st>>>(g);
   MSCS_LAUNCH_CHECK();
-  DenseStream d{};
-  d.count = count;
-  int blk = 0;
-  for (int s = 0; s < count; ++s) {
-    d.dx[s] = g.dF[s]; d.slot[s] = g.slot[s]; d.dfeat[s] = g.dfeat[s]; d.ld[s] = g.ldF[s]; d.C[s] = g.C[s];
-    d.plane[s] = g.plane[s]; d.npix[s] = g.n[s] * g.plane[s]; d.blk0[s] = blk;
-    blk += ceil_div(d.npix[s], 512);
-  }
-  d.blk0[count] = blk;
-  k_dense_stream<<<blk, 128, 0, st>>>(d);
-  MSCS_LAUNCH_CHECK();
-  return 0;
+  if (int rc = dense_stream_launch<float>(g, items, MSCS_DTYPE_F32, st)) return rc;
+  if (int rc = dense_stream_launch<__nv_bfloat16>(g, items, MSCS_DTYPE_BF16, st)) return rc;
+  return dense_stream_launch<__half>(g, items, MSCS_DTYPE_F16, st);
 }
 
-// ---- channels-last (NHWC) row gather / scatter, every scale in one launch (see mscs.h) ----
-static int rows_batch(const mscs_rows_item* items, int count, bool gather, RowsBatch* g, int* blocks_out) {
+// ---- channels-last (NHWC) row gather / scatter, every scale of one element type in one launch (see mscs.h) ----
+static int rows_check(const mscs_rows_item* items, int count, bool gather) {
   MSCS_CHECK_ARG(items && count >= 1 && count <= MSCS_MAX_SCALES, "bad item count %d", count);
-  g->count = count;
-  int blocks = 0;
   for (int s = 0; s < count; ++s) {
     const mscs_rows_item& it = items[s];
     MSCS_CHECK_ARG(it.pix && it.anc_f32 && it.inv_norm, "item %d: null pointer argument", s);
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC && it.rows >= 0, "item %d: C=%d unsupported (1..%d)", s, it.C, kMaxC);
     if (gather) MSCS_CHECK_ARG(it.feat && it.anc_bf16, "item %d: null pointer argument", s);
     else MSCS_CHECK_ARG(it.dF && it.dfeat && it.ldF >= it.C, "item %d: bad gradient arguments", s);
-    g->feat[s] = it.feat; g->pix[s] = it.pix; g->n_rows_dev[s] = it.n_rows_dev;
-    g->bf16[s] = (__nv_bfloat16*)it.anc_bf16; g->f32[s] = it.anc_f32; g->inv[s] = it.inv_norm;
-    g->dF[s] = it.dF; g->dfeat[s] = it.dfeat; g->C[s] = it.C; g->ldF[s] = it.ldF; g->rows[s] = it.rows;
-    g->block0[s] = blocks;
+    if (int rc = check_dtype(s, it.dtype, gather ? it.feat : it.dfeat, 1, gather ? "feat" : "dfeat")) return rc;
+  }
+  return 0;
+}
+
+template <typename T>
+static int rows_launch(const mscs_rows_item* items, int count, bool gather, int dtype, cudaStream_t st) {
+  RowsBatch g{};
+  int blocks = 0;
+  for (int s = 0; s < count; ++s) {
+    const mscs_rows_item& it = items[s];
+    if (it.dtype != dtype) continue;
+    const int j = g.count++;
+    g.feat[j] = it.feat; g.pix[j] = it.pix; g.n_rows_dev[j] = it.n_rows_dev;
+    g.bf16[j] = (__nv_bfloat16*)it.anc_bf16; g.f32[j] = it.anc_f32; g.inv[j] = it.inv_norm;
+    g.dF[j] = it.dF; g.dfeat[j] = it.dfeat; g.C[j] = it.C; g.ldF[j] = it.ldF; g.rows[j] = it.rows;
+    g.block0[j] = blocks;
     blocks += ceil_div(gather ? (it.rows + 255) / 256 * 256 : it.rows, 8);
   }
-  g->block0[count] = blocks;
-  *blocks_out = blocks;
+  g.block0[g.count] = blocks;
+  if (blocks == 0) return 0;
+  if (gather) k_gather_rows_nhwc<T><<<blocks, 256, 0, st>>>(g);
+  else k_scatter_rows_nhwc<T><<<blocks, 256, 0, st>>>(g);
+  MSCS_LAUNCH_CHECK();
   return 0;
+}
+
+static int rows_batch(const mscs_rows_item* items, int count, bool gather, void* stream_) {
+  if (int rc = rows_check(items, count, gather)) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (int rc = rows_launch<float>(items, count, gather, MSCS_DTYPE_F32, st)) return rc;
+  if (int rc = rows_launch<__nv_bfloat16>(items, count, gather, MSCS_DTYPE_BF16, st)) return rc;
+  return rows_launch<__half>(items, count, gather, MSCS_DTYPE_F16, st);
 }
 
 extern "C" int mscs_gather_rows_nhwc_batch(const mscs_rows_item* items, int count, void* stream_) {
-  RowsBatch g{};
-  int blocks = 0;
-  if (int rc = rows_batch(items, count, true, &g, &blocks)) return rc;
-  if (blocks == 0) return 0;
-  k_gather_rows_nhwc<<<blocks, 256, 0, (cudaStream_t)stream_>>>(g);
-  MSCS_LAUNCH_CHECK();
-  return 0;
+  return rows_batch(items, count, true, stream_);
 }
 
 extern "C" int mscs_scatter_rows_nhwc_batch(const mscs_rows_item* items, int count, void* stream_) {
-  RowsBatch g{};
-  int blocks = 0;
-  if (int rc = rows_batch(items, count, false, &g, &blocks)) return rc;
-  if (blocks == 0) return 0;
-  k_scatter_rows_nhwc<<<blocks, 256, 0, (cudaStream_t)stream_>>>(g);
-  MSCS_LAUNCH_CHECK();
-  return 0;
+  return rows_batch(items, count, false, stream_);
 }

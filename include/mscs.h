@@ -32,6 +32,13 @@ extern "C" {
 #define MSCS_MAX_RANKS 8    /* pooled mode: GPUs of one box */
 #define MSCS_IPC_HANDLE_BYTES 64
 
+/* element type of a feature map / its dense gradient (the `dtype` member of the gather / rows / scatter items) and of
+ * the CE logits / dlogits.  Half inputs are widened exactly to fp32 on load; all arithmetic is fp32; half outputs are
+ * rounded to nearest even on store (the rounding of torch's Tensor.to). */
+#define MSCS_DTYPE_F32 0
+#define MSCS_DTYPE_BF16 1
+#define MSCS_DTYPE_F16 2
+
 /* library info ------------------------------------------------------------------------- */
 const char* mscs_version(void);
 const char* mscs_last_error(void);
@@ -160,7 +167,7 @@ int mscs_mt19937_advance_host(uint32_t* mt_state_host, int* mt_pos, uint64_t k);
 /* ---------------------------------------------------------------------------------------
  * K2 -- gather + L2 normalise.  Replaces the strided gather features[b,:,idx] (V2.py:123)
  * and F.normalize(p=2, dim=1) (V2.py:138, _ms.py:95,104).
- *   feat : fp32 NCHW (n,C,fh,fw) contiguous;  pix/N from K1
+ *   feat : NCHW (n,C,fh,fw) contiguous, fp32 (the batched form also bf16 / fp16, see `dtype`);  pix/N from K1
  *   anc_bf16 : (N_pad, C_pad) bf16 row-major, C_pad = C rounded up to 64, N_pad = N rounded
  *              up to 256; padding is written as zeros   (operand of the similarity kernels)
  *   anc_f32  : (N, C) fp32 unit rows (used by the normalisation backward)
@@ -176,15 +183,18 @@ int mscs_gather_normalize_sectors(const float* feat, int n, int C, int plane, co
 int mscs_gather_normalize_sectors_async(const float* feat, int n, int C, int plane, const int32_t* slot,
                                         const int32_t* n_rows_dev, void* anc_bf16, float* anc_f32, float* inv_norm,
                                         void* stream);
-/* every scale of a call in ONE launch (device-driven form, see above) */
+/* every scale of a call in ONE launch (device-driven form, see above).  `dtype` (MSCS_DTYPE_*, last member: a
+ * zero-initialised item is fp32) is the element type of `feat`; scales of different dtypes may be mixed (one launch
+ * per dtype present).  The outputs are the same for a half map and for its exact fp32 widening. */
 typedef struct {
-  const float* feat; int32_t n, C, plane; const int32_t* slot; const int32_t* n_rows_dev;
+  const void* feat; int32_t n, C, plane; const int32_t* slot; const int32_t* n_rows_dev;
   void* anc_bf16; float* anc_f32; float* inv_norm;
+  int32_t dtype;
 } mscs_gather_item;
 int mscs_gather_normalize_sectors_batch(const mscs_gather_item* items, int count, void* stream);
 /* The same gather with the strided walk over the channel planes done by the TMA unit: one bulk-tensor copy of
  * {8 pixels x C channels} per octet of the slot map that holds a sampled pixel, staged in shared memory
- * (feature maps 16-byte aligned). */
+ * (feature maps 16-byte aligned; fp32 items only). */
 int mscs_gather_normalize_tma_batch(const mscs_gather_item* items, int count, void* stream);
 
 /* ---------------------------------------------------------------------------------------
@@ -273,27 +283,32 @@ int mscs_scatter_grad(const float* dF, int ldF, const float* anc_f32, const floa
 int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream);
 int mscs_scatter_sectors(const float* dF, int ldF, const float* anc_f32, const float* inv_norm,
                          const int32_t* slot, int n, int C, int plane, float* dfeat, void* stream);
-/* every scale of a call in ONE launch */
+/* every scale of a call in ONE launch.  `dtype` (last member, MSCS_DTYPE_*): element type of `dfeat`; the gradient rows
+ * dF stay fp32.  mscs_scatter_sectors_batch takes fp32 items only. */
 typedef struct {
   const float* dF; int32_t ldF; const float* anc_f32; const float* inv_norm; const int32_t* slot;
-  int32_t n, C, plane; float* dfeat;
+  int32_t n, C, plane; void* dfeat;
+  int32_t dtype;
 } mscs_scatter_item;
 int mscs_scatter_sectors_batch(const mscs_scatter_item* items, int count, void* stream);
-/* Channels-last feature maps (memory order [n][h][w][C]): an anchor is one contiguous row of C floats, so the gather
+/* Channels-last feature maps (memory order [n][h][w][C]): an anchor is one contiguous row of C elements, so the gather
  * (+ L2 normalisation) and the scatter (normalisation backward into the pre-zeroed channels-last dense gradient) are
  * row copies driven by `pix` (global pixel id = image * plane + pixel of every sorted anchor row, -1 = not local).
- * `rows`: number of anchor rows, or their upper bound when `n_rows_dev` (device-resident count, gather only) is set. */
+ * `rows`: number of anchor rows, or their upper bound when `n_rows_dev` (device-resident count, gather only) is set.
+ * `dtype` (last member, MSCS_DTYPE_*): element type of `feat` and `dfeat`. */
 typedef struct {
-  const float* feat; const int32_t* pix; const int32_t* n_rows_dev; int32_t rows, C;
+  const void* feat; const int32_t* pix; const int32_t* n_rows_dev; int32_t rows, C;
   void* anc_bf16; float* anc_f32; float* inv_norm;          /* gather outputs / scatter inputs */
-  const float* dF; int32_t ldF; float* dfeat;               /* scatter only */
+  const float* dF; int32_t ldF; void* dfeat;                /* scatter only */
+  int32_t dtype;
 } mscs_rows_item;
 int mscs_gather_rows_nhwc_batch(const mscs_rows_item* items, int count, void* stream);
 int mscs_scatter_rows_nhwc_batch(const mscs_rows_item* items, int count, void* stream);
 /* Dense gradients of every scale written in ONE streaming pass, zeros included (no pre-zeroed buffer needed):
- * dF rows are first turned into dx rows IN PLACE (rows[s] rows of item s), then every float4 of every dfeat is
- * written once.  plane must be a multiple of 4.  mask_scratch: sum over items of ceil(n*plane/32) uint32 words
- * (one bit per pixel: sampled or not, built inside the call). */
+ * dF rows are first turned into dx rows IN PLACE (rows[s] rows of item s), then every 16 bytes of every dfeat are
+ * written once (4 fp32 or 8 half pixels of a channel plane per store).  plane must be a multiple of 4 (fp32) or 8
+ * (bf16 / fp16), dfeat 16-byte aligned.  mask_scratch: sum over items of ceil(n*plane/32) uint32 words (one bit per
+ * pixel: sampled or not, built inside the call). */
 int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count, uint32_t* mask_scratch,
                              void* stream);
 
@@ -347,21 +362,24 @@ int mscs_backward_chain(const mscs_sim_job* job, const float* grad_out, float* c
  *                      (mscs_sample_hist_i16 / mscs_sample_plan_i16: same results as the int64 entry points) and the
  *                      CE kernels; the histogram gives the CE normaliser sum_valid w[y] before the logits are read.
  *   mscs_ce_forward    loss_and_denom[0] = sum_valid w[y] (logsumexp(x) - x_y) / denom,  [1] = denom = sum_c w[c] hist[c]
- *                      (c < K, c != ignore_index); logits fp32 NCHW (n, K, plane), plane % 4 == 0; weight NULL = ones;
+ *                      (c < K, c != ignore_index); logits NCHW (n, K, plane), plane % 4 == 0; weight NULL = ones;
  *                      labels >= K or == ignore_index are ignored; loss_sum_scratch: one double of device scratch.
  *   mscs_ce_backward   dlogits = (*grad_out / *denom) w[y] (softmax(x) - onehot(y)), zeros on ignored pixels: one fused
  *                      pass (ATen: log_softmax backward + nll_loss backward).
+ *   `dtype` (MSCS_DTYPE_*): element type of logits and dlogits (fp32: 16-byte aligned, half: 8-byte aligned); the
+ *   arithmetic is fp32 either way, dlogits are rounded to nearest even on store.
  * ------------------------------------------------------------------------------------- */
 int mscs_label_pass(const int64_t* labels, int64_t n_pixels, int num_classes, int16_t* lab16, int32_t* hist,
                     void* stream);
 int mscs_sample_hist_i16(const mscs_sample_cfg* cfg, const int16_t* lab16, void* workspace, void* stream);
 int mscs_sample_plan_i16(const mscs_sample_cfg* cfg, const int16_t* lab16, void* workspace, mscs_scale_plan* plan_dev,
                          void* stream);
-int mscs_ce_forward(const float* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
+int mscs_ce_forward(const void* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
                     int ignore_index, const int32_t* hist, int num_classes, double* loss_sum_scratch,
-                    float* loss_and_denom, void* stream);
-int mscs_ce_backward(const float* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
-                     int ignore_index, const float* grad_out, const float* denom, float* dlogits, void* stream);
+                    float* loss_and_denom, void* stream, int dtype);
+int mscs_ce_backward(const void* logits, const int16_t* lab16, int n, int K, int plane, const float* weight,
+                     int ignore_index, const float* grad_out, const float* denom, void* dlogits, void* stream,
+                     int dtype);
 
 /* ---------------------------------------------------------------------------------------
  * Projector tail on the sampled rows only (SURVEY.md 8f item 1; models/Projector.py:49-72: the projector ends in
