@@ -33,7 +33,7 @@ class GatherItem(C.Structure):
 class ScatterItem(C.Structure):
     _fields_ = [("dF", C.c_void_p), ("ldF", C.c_int32), ("anc_f32", C.c_void_p), ("inv_norm", C.c_void_p),
                 ("slot", C.c_void_p), ("n", C.c_int32), ("C", C.c_int32), ("plane", C.c_int32), ("dfeat", C.c_void_p),
-                ("dtype", C.c_int32)]
+                ("dtype", C.c_int32), ("n_rows_dev", C.c_void_p)]
 
 
 class RowsItem(C.Structure):
@@ -105,6 +105,7 @@ _SIGNATURES = {
     "mscs_scatter_dense_batch": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p, C.c_void_p]),
     "mscs_mt19937_stream": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mscs_philox_stream": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p]),
+    "mscs_philox_stream_dev": (C.c_int, [C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mscs_sample_select": (C.c_int, [C.POINTER(SampleCfg), C.POINTER(ScalePlan), C.c_void_p, C.c_void_p,
                                      _PTRS, _PTRS, _PTRS, _PTRS, _PTRS, _PTRS, C.c_void_p]),
     "mscs_gather_normalize_sectors": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,

@@ -855,12 +855,13 @@ class _StepPlan:
 _step_plans = {}
 
 
-def _step_plan(dev, label_shape, feat_shapes, spec, single_scale, world=1, rank=0, nhwc=False):
+def _step_plan(dev, label_shape, feat_shapes, spec, single_scale, world=1, rank=0, nhwc=False, create=True):
+    """The cached plan of these shapes and this configuration (create=False: None when no call has made it yet)."""
     key = (dev, tuple(label_shape), tuple(feat_shapes), spec.num_classes, spec.temperature, spec.cs_temperature,
            spec.min_views, spec.max_views, spec.max_total, tuple(spec.weights), spec.cross_scale,
            spec.detach_deepest, spec.w_high_low, spec.w_high_mid, single_scale, world, rank, nhwc)
     p = _step_plans.get(key)
-    if p is None:
+    if p is None and create:
         p = _step_plans[key] = _StepPlan(dev, label_shape, feat_shapes, spec, single_scale, world, rank, nhwc)
     return p
 
@@ -879,6 +880,52 @@ def half_io_ok(sp, world):
     if not fast_path_ok(sp.spec, world):
         return False
     return sp.nhwc or (all(sp.slot_sizes) and _DENSE_ONE_PASS and not _GATHER_TMA)
+
+
+def channels_last_ok(spec, world, feats):
+    """Channels-last feature maps (memory order [n][h][w][C]) are consumed as they are by the single-process fast path:
+    an anchor is then one contiguous row (gather / scatter become row copies)."""
+    return fast_path_ok(spec, world) and all(
+        f.dim() == 4 and f.is_contiguous(memory_format=torch.channels_last) and not f.is_contiguous() for f in feats)
+
+
+# first call index of graph replays: eager calls count up from 0 and never get here
+GRAPH_CALL_BASE = 2 ** 62
+
+
+def graph_mode(spec, world, single_scale, labels, feats, counter):
+    """Whether this call is being captured into a CUDA graph (``torch.cuda.graph``), which the single-process fast path
+    with sampler='philox' supports: the call then enqueues work without ever waiting for the host (the row counts stay
+    on the device, the Philox call index is read from ``counter``).  Everything that cannot be captured raises a
+    RuntimeError here, before anything is enqueued, so that the capture still ends cleanly.  Outside a capture: False
+    (the eager path, unchanged)."""
+    if not (feats[0].is_cuda and torch.cuda.is_current_stream_capturing()):      # (a CUDA tensor: a runtime exists)
+        return False
+
+    def refuse(why):
+        raise RuntimeError(f"the contrastive loss cannot be captured in a CUDA graph: {why}")
+
+    if world > 1:
+        refuse("the pooled mode (comm) exchanges control data through the host")
+    if spec.sampler != "philox":
+        refuse("sampler='reference' advances the torch CPU generator by a label-dependent number of draws; "
+               "use sampler='philox'")
+    if single_scale and spec.cross_scale:
+        refuse("DenseContrastiveLossV2 with cross_scale_contrast=True returns sampled features of a data-dependent shape")
+    if not _DENSE_ONE_PASS or _GATHER_TMA:
+        refuse("MSCS_DENSE=0 and MSCS_GATHER=tma take host-driven routes")
+    if not fast_path_ok(spec, world):
+        refuse("the selection table of this configuration exceeds the device-driven path's shared memory")
+    if any(f.device != feats[0].device for f in feats) or labels.device != feats[0].device:
+        refuse("labels and feature maps must already be on the GPU")
+    nhwc = channels_last_ok(spec, world, feats)
+    if not nhwc and any((f.shape[2] * f.shape[3]) % 8 for f in feats):
+        refuse("feature planes that are not a multiple of 8 pixels take the host-driven path")
+    sp = _step_plan(feats[0].device, labels.shape, [tuple(f.shape) for f in feats], spec, single_scale, world, 0, nhwc,
+                    create=False)
+    if sp is None or counter is None or counter.device != feats[0].device:
+        refuse("run one eager call with the same shapes and configuration before capturing (warm-up)")
+    return True
 
 
 def _dense_grad_slab(shapes, dtypes, dev):
@@ -932,6 +979,26 @@ def _raise_plan_errors(plan, S, spec):
             raise ValueError(f"scale {s}: {plan[s].V} views per class exceed the supported 16384")
 
 
+def fetch_graph_plan(state):
+    """Logged scalars [term losses..., total, inf/NaN flag] and plan records of the latest replay of a captured call, in
+    ONE device->host copy (the only synchronisation).  Valid until the next replay of the graph."""
+    sp, e = state.sp, state.entry
+    nb = C.sizeof(_lib.ScalePlan) * sp.S
+    off = sp.slab_off["plan"]
+    raw = torch.cat([state.scalars.view(torch.uint8), e.slab[off:off + nb]]).cpu().numpy()
+    ns = 4 * state.scalars.numel()
+    plan = (_lib.ScalePlan * sp.S).from_buffer_copy(raw[ns:].tobytes())
+    return raw[:ns].view(np.float32).tolist(), plan
+
+
+def graph_samples(state, plan):
+    """The ScaleSample list of a captured call's latest replay (views of the graph's workspace: the next replay
+    overwrites them)."""
+    sp, e = state.sp, state.entry
+    return [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w, e.islab,
+                        sp.ioff[s], sp.A) for s in range(sp.S)]
+
+
 def _fill_job(job, sp, A, bbase, ibase, sbase, cbase, work_ptr):
     """Everything of the similarity job that follows from the slab layouts (sized by upper bounds)."""
     job.num_terms, job.C_pad, job.num_classes = len(sp.terms), sp.C_pad, A
@@ -959,8 +1026,10 @@ class _Workspace:
     replaces ``last_state``), so steady-state training ping-pongs between two of them and does no per-call slab
     allocation or structure filling.  The scalars handed to the caller live in a fresh tensor per call."""
 
-    def __init__(self, sp):
+    def __init__(self, sp, graph=False):
         dev, S, A = sp.dev, sp.S, sp.A
+        # graph: allocated inside a CUDA graph capture and used by its replays only -- never returned to the pool
+        self.graph = graph
         self.slab = slab = torch.empty(sp.slab_bytes, dtype=torch.uint8, device=dev)
         sb, so = slab.data_ptr(), sp.slab_off
         self.islab = slab[so["islab"]:so["islab"] + 4 * sp.islab_n].view(torch.int32)
@@ -1016,6 +1085,15 @@ class _Workspace:
                 it.dF, it.ldF = self.dF_ptr + 4 * sp.dF_off[s], sp.C_pad
                 it.anc_f32, it.inv_norm = self.fbase + 4 * sp.foff[s][0], self.fbase + 4 * sp.foff[s][1]
                 it.slot, it.n, it.C, it.plane = self.slots[s].data_ptr(), n, Cc, h * w
+        self.rows_dev = [self.plan_dev + s * plan_sz + 8 for s in range(S)]      # &plan_dev[s].N
+        if graph:       # the backward of a captured call never sees the plan: upper bounds + device-resident counts
+            for i, (a, k, *_rest) in enumerate(sp.terms):
+                t = self.job_bwd.terms[i]
+                t.N1, t.N2 = sp.Ncap[a], sp.Ncap[k]
+                t.n1_dev, t.n2_dev = self.rows_dev[a], self.rows_dev[k]
+            for s in range(S):
+                self.bw_rows[s] = sp.Ncap[s]
+                self.bw_items[s].n_rows_dev = self.rows_dev[s]
         self.plan = (_lib.ScalePlan * S)()
         self.last_stream = None
         self.philox = None          # stream buffer of the opt-in counter-based sampler (allocated on first use)
@@ -1038,18 +1116,19 @@ class _StepState:
 
     def __del__(self):
         e, self.entry = self.entry, None
-        if e is not None:
+        if e is not None and not e.graph:
             self.sp.ws_pool.append(e)
 
 
-def run_forward(sp, labels, feats32, needs, comm=None, philox=None):
+def run_forward(sp, labels, feats32, needs, comm=None, philox=None, graph=False):
     """philox: None (reference stream: torch CPU generator) or (seed, call index) of the opt-in counter-based stream.
-    feats32: fp32 maps, or bf16 / fp16 ones where half_io_ok(sp, world) holds (fast path only)."""
+    feats32: fp32 maps, or bf16 / fp16 ones where half_io_ok(sp, world) holds (fast path only).
+    graph: the call is captured into a CUDA graph (see graph_mode); philox is then (seed, int64 device call index)."""
     pooled = comm is not None and comm.world > 1
     # device-driven order (selection, gather and similarity forward enqueued before the host sees the plan): single
     # process, every plane a multiple of 8 pixels (slot maps), selection shared memory within limits
     if fast_path_ok(sp.spec, 1 if not pooled else comm.world) and (sp.nhwc or all(x != 0 for x in sp.slot_sizes)):
-        return _run_forward_fast(sp, labels, feats32, needs, philox)
+        return _run_forward_fast(sp, labels, feats32, needs, philox, graph)
     assert all(f.dtype == torch.float32 for f in feats32), "half maps are converted by the caller off the fast path"
     assert not sp.nhwc, "channels-last inputs are converted by the caller unless the fast path applies"
     if philox is not None:
@@ -1073,16 +1152,23 @@ def _finish_rng(sp, dev, mt, pos, total, defer=False):
     _stream_cache(dev).release_and_prefetch(mt2, pos2, sp.max_draws + _MT_N, defer)
 
 
-def _run_forward_fast(sp, labels, feats32, needs, philox=None):
+def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
     """Single process.  Selection, gather AND the similarity forward are driven by the DEVICE plan records and enqueued
     before the host looks at the plan: the one host wait of the forward pass (needed to raise the reference's errors
-    and to size the backward) overlaps ~0.5 ms of queued GPU work instead of draining the stream."""
+    and to size the backward) overlaps ~0.5 ms of queued GPU work instead of draining the stream.
+
+    graph (CUDA graph capture): no host wait at all.  A fresh workspace of the graph's own; the backward structures
+    carry the upper bounds and the device-resident row counts; errors, sampling results and the logging flag stay in
+    the device plan records (read by the caller after a replay: fetch_graph_plan)."""
     lib = _lib.load()
     dev, S, A, spec = sp.dev, sp.S, sp.A, sp.spec
     st, cur = _stream(), _cur_stream()
     import time
     _t = time.perf_counter() if HOST_SEG is not None else 0.0
-    e = sp.ws_pool.pop() if sp.ws_pool else _Workspace(sp)
+    if graph:
+        e = _Workspace(sp, graph=True)
+    else:
+        e = sp.ws_pool.pop() if sp.ws_pool else _Workspace(sp)
     if e.last_stream is not None and e.last_stream != cur:
         cur.wait_stream(e.last_stream)          # reuse on another stream: order after its previous user
     e.last_stream = cur
@@ -1111,8 +1197,12 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
         if hp is not None:
             hp.wait_stream(cur)
         ch.draws, ch.wait_event = e.philox.data_ptr(), None
-        _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws, ch.draws,
-                                          st_s), "mscs_philox_stream")
+        if graph:       # call index in device memory, incremented behind the generator: every replay draws anew
+            _lib.check(lib.mscs_philox_stream_dev(int(philox[0]) & (2 ** 64 - 1), philox[1].data_ptr(), sp.max_draws,
+                                                  ch.draws, st_s), "mscs_philox_stream_dev")
+        else:
+            _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws, ch.draws,
+                                              st_s), "mscs_philox_stream")
     _t = _seg("fwd: rng state + stream acquire", _t)
     # dense gradients + gradient rows: pre-zeroed on a side stream, sampled sectors rewritten by the backward
     # (default: the backward writes them in one streaming pass instead, see _DENSE_ONE_PASS and gather.cu).
@@ -1122,6 +1212,8 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     gradbufs = _GradBuffers(feats32, needs, sp.nhwc, sp.dF_n) \
         if (any(needs) and (sp.nhwc or not _DENSE_ONE_PASS)) else None
     if gradbufs is not None:
+        if graph:       # filled on the caller's stream: a forward captured without its backward leaves no open fork
+            gradbufs.side = cur
         gradbufs.start_fill()
     _t = _seg("fwd: grad buffers", _t)
     ch.labels, ch.labels_i16 = labels.data_ptr(), int(labels.dtype == torch.int16)
@@ -1143,7 +1235,7 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
             e.bw_items[j].dfeat, e.bw_items[j].dtype = sbase + offs[j], _DTYPE_CODE[feats32[j].dtype]
         grad_mask_ptr = sbase + mask_off
     evs = None
-    if TIMING is not None and TIMING_ALL:      # stage accounting (bench.py): five events recorded INSIDE the chain
+    if TIMING is not None and TIMING_ALL and not graph:      # stage accounting (bench.py): five events INSIDE the chain
         evs = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
         for i, ev in enumerate(evs):
             ev.record()         # creates the CUDA event; the chain records it again at its stage boundary
@@ -1157,7 +1249,7 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     # ONE call: fills, hist -> tile scan -> plan -> select on the sampling stream (programmatic dependent launches; the
     # plan records travel to the host on a private stream), gather + similarity forward on the caller's stream, all
     # driven by the DEVICE plan records, then the one host wait of the forward pass (plan records only)
-    _lib.check(lib.mscs_forward_chain(C.byref(ch), st_s, st, plan), "mscs_forward_chain")
+    _lib.check(lib.mscs_forward_chain(C.byref(ch), st_s, st, None if graph else plan), "mscs_forward_chain")
     if HOST_WAIT is not None:
         HOST_WAIT.append(time.perf_counter() - _t0)
     if evs is not None:
@@ -1167,13 +1259,17 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     _t = time.perf_counter() if HOST_SEG is not None else 0.0
     state = _StepState()
     state.sp, state.entry = sp, e          # (from here on an exception returns the workspace to the pool)
-    _raise_plan_errors(plan, S, spec)
-    total = sum(int(plan[s].draws) for s in range(S))
-    samples = [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w,
-                           e.islab, sp.ioff[s], A) for s in range(S)]
-    for i, (a, k, *_rest) in enumerate(sp.terms):      # the backward is launched with the actual counts
-        t = e.job_bwd.terms[i]
-        t.N1, t.N2 = samples[a].N, samples[k].N
+    state.graph = graph
+    if graph:           # nothing is known on the host: the backward structures hold the device-count form already
+        samples = None
+    else:
+        _raise_plan_errors(plan, S, spec)
+        total = sum(int(plan[s].draws) for s in range(S))
+        samples = [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w,
+                               e.islab, sp.ioff[s], A) for s in range(S)]
+        for i, (a, k, *_rest) in enumerate(sp.terms):      # the backward is launched with the actual counts
+            t = e.job_bwd.terms[i]
+            t.N1, t.N2 = samples[a].N, samples[k].N
     _t = _seg("fwd: after wait", _t)
     if philox is None:
         _finish_rng(sp, dev, mt, pos, total, defer=any(needs))
@@ -1186,8 +1282,9 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None):
     state.grad_slab, state.grad_outs = grad_slab, grad_outs
     state.grad_mask_ptr = grad_mask_ptr if grad_slab is not None else None
     state.io_dtypes = [f.dtype for f in feats32]
-    for s in range(S):
-        e.bw_rows[s] = samples[s].N
+    if not graph:
+        for s in range(S):
+            e.bw_rows[s] = samples[s].N
     return state
 
 
@@ -1514,6 +1611,10 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
     grads = []
     fbase = state.fslab.data_ptr()
     io = state.io_dtypes or [torch.float32] * S         # dtypes the kernels write the dense gradients in
+    # a captured call: row counts only on the device (upper bounds on the host), no generator prefetch to launch
+    graph = getattr(state, "graph", False)
+    rows_dev = e.rows_dev if graph else [None] * S
+    n_rows = (lambda s: sp.Ncap[s]) if graph else (lambda s: state.samples[s].N)
     dense = (not sp.nhwc) and state.gradbufs is None and \
         all((not needs[s]) or (state.slots[s] is not None) for s in range(S))
     if dense:
@@ -1538,8 +1639,8 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
                 it = items[j]
                 it.dF, it.ldF, it.anc_f32, it.inv_norm = ptrs[s], sp.C_pad, fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
                 it.slot, it.n, it.C, it.plane = state.slots[s].data_ptr(), n, Cc, h * w
-                it.dfeat, it.dtype = sbase + offs[j], _DTYPE_CODE[io[s]]
-                rows[j] = state.samples[s].N
+                it.dfeat, it.dtype, it.n_rows_dev = sbase + offs[j], _DTYPE_CODE[io[s]], rows_dev[s]
+                rows[j] = n_rows(s)
         evs, evp = None, None
         if TIMING is not None:
             evs = [torch.cuda.Event(enable_timing=True) for _ in range(3 if TIMING_ALL else 2)]
@@ -1548,7 +1649,8 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
             evp = _lib.ptr_array([ev.cuda_event for ev in evs] + [None] * (3 - len(evs)))
         _lib.check(lib.mscs_backward_chain(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, items, rows,
                                            len(idx), mask_ptr, evp, st), "mscs_backward_chain")
-        _stream_cache(dev).flush()        # the deferred generator launch of the next call's stream
+        if not graph:
+            _stream_cache(dev).flush()    # the deferred generator launch of the next call's stream
         if evs is not None:
             TIMING.setdefault("sim_bwd", []).append((evs[0], evs[1]))
             if len(evs) == 3:
@@ -1558,7 +1660,8 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
     with _timed("sim_bwd"):
         _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st),
                    "mscs_sim_backward")
-    _stream_cache(dev).flush()            # the deferred generator launch of the next call's stream
+    if not graph:
+        _stream_cache(dev).flush()        # the deferred generator launch of the next call's stream
     if sp.nhwc:
         with _timed("scatter"):
             gb = state.gradbufs
@@ -1574,7 +1677,8 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
                     pre = torch.zeros((n, h, w, Cc), dtype=io[s], device=dev).permute(0, 3, 1, 2)
                 outs[s] = pre
                 it = items[j]
-                it.pix, it.rows, it.C = state.samples[s].ptr(2), state.samples[s].N, Cc
+                it.pix = e.islab.data_ptr() + 4 * sp.ioff[s][2] if graph else state.samples[s].ptr(2)
+                it.rows, it.C, it.n_rows_dev = n_rows(s), Cc, rows_dev[s]
                 it.anc_f32, it.inv_norm = fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
                 it.dF, it.ldF, it.dfeat, it.dtype = ptrs[s], sp.C_pad, pre.data_ptr(), _DTYPE_CODE[io[s]]
             if idx:
@@ -1627,15 +1731,17 @@ class MsCsContrastiveFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, labels, spec, single_scale, holder, *feats):
         comm = holder.get("comm")
+        world = comm.world if comm is not None else 1
+        philox = holder.get("philox")
+        # decided (and refused) before anything is enqueued
+        graph = graph_mode(spec, world, single_scale, labels, feats, philox[1] if philox is not None else None)
         if not _device_checked[0]:
             if not _lib.load().mscs_device_ok():
                 raise RuntimeError("mscs_b200 needs a compute-capability 10.x (B200) device; no fallback exists")
             _device_checked[0] = True
         # channels-last feature maps (memory order [n][h][w][C]) are consumed as they are by the single-process fast
         # path: an anchor is then one contiguous row (gather / scatter become row copies)
-        world = comm.world if comm is not None else 1
-        nhwc = fast_path_ok(spec, world) and all(
-            f.dim() == 4 and f.is_contiguous(memory_format=torch.channels_last) and not f.is_contiguous() for f in feats)
+        nhwc = channels_last_ok(spec, world, feats)
         for f in feats:
             _require_device(f)
         dev = feats[0].device
@@ -1656,7 +1762,7 @@ class MsCsContrastiveFn(torch.autograd.Function):
                 if m.dtype != torch.float32 and not (half_ok and m.dtype in _DTYPE_CODE):
                     m = m.float()
                 maps.append(m if nhwc else m.contiguous())
-            state = run_forward(sp, labels, maps, needs, comm, holder.get("philox"))
+            state = run_forward(sp, labels, maps, needs, comm, philox, graph)
         holder["samples"], holder["state"] = state.samples, state
         ctx.state, ctx.needs = state, needs
         ctx.shapes = [tuple(f.shape) for f in feats]

@@ -414,7 +414,8 @@ __global__ void __launch_bounds__(256) k_dx_rows(const __grid_constant__ DenseBa
   while (s + 1 < g.count && (int)blockIdx.x >= g.rowblk0[s + 1]) ++s;
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.rowblk0[s]) * 8 + (threadIdx.x >> 5);
-  if (row >= g.rows[s]) return;
+  // rows[s] sizes the grid; with a device-resident count it is an upper bound and the rows beyond the count are stale
+  if (row >= g.rows[s] || (g.n_rows_dev[s] && row >= *g.n_rows_dev[s])) return;
   const int C = g.C[s];
   float* gr = g.dF[s] + (size_t)row * g.ldF[s];
   const float* f = g.f32[s] + (size_t)row * C;
@@ -531,7 +532,7 @@ __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant
   while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.block0[s]) * 8 + (threadIdx.x >> 5);
-  if (row >= g.rows[s]) return;
+  if (row >= g.rows[s] || (g.n_rows_dev[s] && row >= *g.n_rows_dev[s])) return;      // (as k_dx_rows)
   const int gp = g.pix[s][row];
   if (gp < 0) return;
   const int C = g.C[s];
@@ -888,6 +889,7 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
                    "item %d: half gradients need a plane that is a multiple of 8 pixels (plane %d)", s, it.plane);
     g.dF[s] = const_cast<float*>(it.dF); g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot;
     g.dfeat[s] = (float*)it.dfeat; g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = rows[s];
+    g.n_rows_dev[s] = it.n_rows_dev;
     MSCS_CHECK_ARG((long long)it.n * it.C * it.plane < (1ll << 32), "item %d: more than 2^32 gradient elements", s);
     g.v4_0[s] = v4;      // block prefix: 2048 floats per block
     v4 += ((long long)it.n * it.C * it.plane + 2047) / 2048;

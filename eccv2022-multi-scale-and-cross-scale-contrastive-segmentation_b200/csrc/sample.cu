@@ -597,10 +597,7 @@ __device__ __forceinline__ uint32_t mt_untemper(uint32_t y) {
   return t;
 }
 
-__global__ void __launch_bounds__(256)
-k_philox_stream(unsigned long long seed, unsigned long long call, unsigned long long n_quads, uint4* __restrict__ out) {
-  const unsigned long long q = (unsigned long long)blockIdx.x * 256ull + threadIdx.x;
-  if (q >= n_quads) return;
+__device__ __forceinline__ uint4 philox_quad(unsigned long long seed, unsigned long long call, unsigned long long q) {
   uint4 c = make_uint4((uint32_t)q, (uint32_t)(q >> 32), (uint32_t)call, (uint32_t)(call >> 32));
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
 #pragma unroll
@@ -610,15 +607,55 @@ k_philox_stream(unsigned long long seed, unsigned long long call, unsigned long 
     c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
     k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
   }
-  out[q] = make_uint4(mt_untemper(c.x), mt_untemper(c.y), mt_untemper(c.z), mt_untemper(c.w));
+  return make_uint4(mt_untemper(c.x), mt_untemper(c.y), mt_untemper(c.z), mt_untemper(c.w));
+}
+
+__global__ void __launch_bounds__(256)
+k_philox_stream(unsigned long long seed, unsigned long long call, unsigned long long n_quads, uint4* __restrict__ out) {
+  const unsigned long long q = (unsigned long long)blockIdx.x * 256ull + threadIdx.x;
+  if (q >= n_quads) return;
+  out[q] = philox_quad(seed, call, q);
+}
+
+// the call index read from device memory (CUDA graphs: a replay runs the captured launch with its arguments frozen)
+__global__ void __launch_bounds__(256) k_philox_stream_dev(unsigned long long seed,
+                                                           const unsigned long long* __restrict__ call_dev,
+                                                           unsigned long long n_quads, uint4* __restrict__ out) {
+  const unsigned long long q = (unsigned long long)blockIdx.x * 256ull + threadIdx.x;
+  if (q >= n_quads) return;
+  out[q] = philox_quad(seed, *call_dev, q);
+}
+
+// next call index: a launch of its own behind the generator on the same stream, i.e. after every reader of the old one
+__global__ void k_philox_call_next(unsigned long long* call_dev) { *call_dev += 1ull; }
+
+static int philox_args(const uint32_t* draws_dev, uint64_t n_words) {
+  MSCS_CHECK_ARG(draws_dev && ((uintptr_t)draws_dev & 15) == 0, "draws_dev must be a 16-byte aligned device pointer");
+  MSCS_CHECK_ARG((n_words + 3) / 4 <= 0x7fffffffull * 256ull, "stream too long");
+  return 0;
 }
 
 extern "C" int mscs_philox_stream(uint64_t seed, uint64_t call, uint64_t n_words, uint32_t* draws_dev, void* stream_) {
-  MSCS_CHECK_ARG(draws_dev && ((uintptr_t)draws_dev & 15) == 0, "draws_dev must be a 16-byte aligned device pointer");
+  if (int rc = philox_args(draws_dev, n_words)) return rc;
   if (n_words == 0) return 0;
   const unsigned long long quads = (n_words + 3) / 4;       // the buffer holds n_words rounded up to 4 words
-  MSCS_CHECK_ARG(quads <= 0x7fffffffull * 256ull, "stream too long");
   k_philox_stream<<<(unsigned)((quads + 255) / 256), 256, 0, (cudaStream_t)stream_>>>(seed, call, quads, (uint4*)draws_dev);
+  MSCS_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int mscs_philox_stream_dev(uint64_t seed, uint64_t* call_dev, uint64_t n_words, uint32_t* draws_dev,
+                                      void* stream_) {
+  MSCS_CHECK_ARG(call_dev && ((uintptr_t)call_dev & 7) == 0, "call_dev must be an 8-byte aligned device pointer");
+  if (int rc = philox_args(draws_dev, n_words)) return rc;
+  cudaStream_t st = (cudaStream_t)stream_;
+  const unsigned long long quads = (n_words + 3) / 4;
+  if (quads > 0) {
+    k_philox_stream_dev<<<(unsigned)((quads + 255) / 256), 256, 0, st>>>(seed, (const unsigned long long*)call_dev,
+                                                                         quads, (uint4*)draws_dev);
+    MSCS_LAUNCH_CHECK();
+  }
+  k_philox_call_next<<<1, 1, 0, st>>>((unsigned long long*)call_dev);
   MSCS_LAUNCH_CHECK();
   return 0;
 }

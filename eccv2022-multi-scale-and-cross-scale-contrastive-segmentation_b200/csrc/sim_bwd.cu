@@ -52,6 +52,9 @@ struct BwdArgs {
   WorkTable work;
   const float* grad_out;
   int flags;
+  // DEV instance only: device-resident row / column counts of every pass (n_rows / n_cols are then upper bounds).
+  // Kept behind every field the eager instance reads, so that instance compiles as it did without them.
+  const int* rows_dev[MSCS_MAX_PASSES]; const int* cols_dev[MSCS_MAX_PASSES];
 };
 
 __host__ __device__ constexpr size_t bwd_smem_bytes(int KB) {
@@ -67,7 +70,10 @@ __device__ __forceinline__ void red_add_v4(float* addr, float a, float b, float 
                : "memory");
 }
 
-template <int KB>
+// DEV: the row and column counts of a pass are read from device memory (args.rows_dev / cols_dev, written by the
+// sampling plan of the same step) once per run, after the PDL wait; rows and columns beyond them -- stale data of
+// earlier calls inside the upper bounds -- are treated exactly like the padding beyond n_rows / n_cols
+template <int KB, bool DEV>
 __global__ void __launch_bounds__(kBwdThreads, 1) k_sim_bwd(const __grid_constant__ BwdArgs args) {
   constexpr int CP = KB * 64;                       // padded channel count = N of the second MMA
   extern __shared__ uint8_t smem_raw[];
@@ -232,6 +238,8 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_sim_bwd(const __grid_constan
       const bool have_n = wk.next(nx);      // next run's work item: its dependent global loads overlap this run
       const BwdDev& p = args.p[sg.owner];
       const int row = sg.rb * 128 + r_loc;
+      int dev_rows = 0, dev_cols = 0;
+      if constexpr (DEV) { dev_rows = *args.rows_dev[sg.owner]; dev_cols = *args.cols_dev[sg.owner]; }
       if (warp == 4) MSCS_TRACE_EV(3, 3, 64u + seg);
       // ---- X rows of this run -> TMEM (A operand layout: lane = row, two bf16 per column).  Every S MMA of the
       // previous run has completed: this warp has passed the s_full wait of its last tile.
@@ -250,7 +258,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_sim_bwd(const __grid_constan
       ptx::tc_fence_before();
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(x_full);
-      const bool valid = row < p.n_rows;
+      const bool valid = row < (DEV ? dev_rows : p.n_rows);
       int p0 = 0, p1 = 0;
       if (valid) { const int y = p.row_cls[row]; p0 = p.col_seg[y]; p1 = p.col_seg[y + 1]; }
       const unsigned plen = (unsigned)(p1 - p0);
@@ -273,7 +281,7 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_sim_bwd(const __grid_constan
         pf_s = 0.f; pf_pn = 0.f; pf_neg = 1.f;
         if (ct_ < sg.c_end) {
           const int c = ct_ * kTileN + (lane >> 4) * kBwdSub + cq * 16 + (lane & 15);
-          if (c < p.n_cols) {
+          if (c < (DEV ? dev_cols : p.n_cols)) {
             if (p.col_cs) pf_s = p.col_cs[c];
             if (p.col_cpn) pf_pn = p.col_cpn[c];
             if (p.col_neg) pf_neg = p.col_neg[c];
@@ -410,12 +418,12 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_sim_bwd(const __grid_constan
 
 using namespace mscs;
 
-template <int KB>
+template <int KB, bool DEV>
 static int launch_bwd(const BwdArgs& args, cudaStream_t st) {
   const size_t smem = bwd_smem_bytes(KB);
   if (int rc = ensure_trap_buffer()) return rc;
-  MSCS_CUDA(cudaFuncSetAttribute(k_sim_bwd<KB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  MSCS_CUDA(launch_k(k_sim_bwd<KB>, persistent_ctas(), kBwdThreads, smem, st, args));
+  MSCS_CUDA(cudaFuncSetAttribute(k_sim_bwd<KB, DEV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  MSCS_CUDA(launch_k(k_sim_bwd<KB, DEV>, persistent_ctas(), kBwdThreads, smem, st, args));
   MSCS_LAUNCH_CHECK();
   return 0;
 }
@@ -432,9 +440,12 @@ extern "C" int mscs_sim_backward_sets(const mscs_sim_job* job, const float* grad
   int rc = validate_job(job);
   if (rc) return rc;
   MSCS_CHECK_ARG(job->work && grad_out && dF_sets && dF_ld, "null pointer argument");
+  // device-resident row counts (n1_dev / n2_dev): for every term or for none; N1 / N2 are then upper bounds that size
+  // the work table and the tensor maps, and the kernels read the actual counts
+  const bool dev_counts = job->terms[0].n1_dev != nullptr;
   for (int t = 0; t < job->num_terms; ++t)
-    MSCS_CHECK_ARG(!job->terms[t].n1_dev && !job->terms[t].n2_dev,
-                   "term %d: the backward needs the actual row counts in N1 / N2 (n1_dev / n2_dev must be NULL)", t);
+    MSCS_CHECK_ARG((job->terms[t].n1_dev != nullptr) == dev_counts && (job->terms[t].n2_dev != nullptr) == dev_counts,
+                   "term %d: n1_dev / n2_dev must be set for every term or for none", t);
   cudaStream_t st = (cudaStream_t)stream_;
   BwdPass passes[MSCS_MAX_PASSES];
   int np = build_passes(job, passes);
@@ -478,7 +489,8 @@ extern "C" int mscs_sim_backward_sets(const mscs_sim_job* job, const float* grad
     args.p[i] = BwdDev{p.row_cls, p.col_seg, p.row_cs, p.row_cpn, p.row_neg, p.col_cs, p.col_cpn, p.col_neg,
                        (const __nv_bfloat16*)p.x_bf16, dF_sets[p.row_set], dF_ld[p.row_set], p.n_rows, p.n_cols,
                        p.self_mask, ym, p.scale_log2, p.out_scale};
-    b.t[i] = BuildTerm{p.row_cls, p.col_seg, p.n_rows, p.n_cols, nitems, p.rb_lo, 0, 1 << 30, nullptr, nullptr};
+    b.t[i] = BuildTerm{p.row_cls, p.col_seg, p.n_rows, p.n_cols, nitems, p.rb_lo, 0, 1 << 30, p.n_rows_dev, p.n_cols_dev};
+    args.rows_dev[i] = p.n_rows_dev; args.cols_dev[i] = p.n_cols_dev;
     nitems += p.rb_hi - p.rb_lo;
   }
   b.num_terms = np; b.nitems = nitems; b.rows_per_item = 128; b.mode = 0;
@@ -490,11 +502,19 @@ extern "C" int mscs_sim_backward_sets(const mscs_sim_job* job, const float* grad
   rc = launch_build_work(b, st);
   if (rc) return rc;
   args.work = WorkTable{b.items, b.prefix, nitems, b.pad};
+  if (dev_counts) {
+    switch (job->C_pad / 64) {
+      case 1: return launch_bwd<1, true>(args, st);
+      case 2: return launch_bwd<2, true>(args, st);
+      case 3: return launch_bwd<3, true>(args, st);
+      default: return launch_bwd<4, true>(args, st);
+    }
+  }
   switch (job->C_pad / 64) {
-    case 1: return launch_bwd<1>(args, st);
-    case 2: return launch_bwd<2>(args, st);
-    case 3: return launch_bwd<3>(args, st);
-    default: return launch_bwd<4>(args, st);
+    case 1: return launch_bwd<1, false>(args, st);
+    case 2: return launch_bwd<2, false>(args, st);
+    case 3: return launch_bwd<3, false>(args, st);
+    default: return launch_bwd<4, false>(args, st);
   }
 }
 

@@ -27,6 +27,7 @@ struct BwdPass {
   const float* row_cs; const float* row_cpn; const float* row_neg;   // row-side coefficients or null
   const float* col_cs; const float* col_cpn; const float* col_neg;   // col-side coefficients or null
   int n_rows, n_cols;
+  const int* n_rows_dev; const int* n_cols_dev;   // device-resident counts (n_rows / n_cols: upper bounds) or null
   int rb_lo, rb_hi;       // row tiles (128 rows) this rank handles
   int self_mask;
   int row_set, col_set;
@@ -42,6 +43,7 @@ static inline int build_passes(const mscs_sim_job* job, BwdPass* out) {
     p.x_bf16 = m.a_bf16; p.y_bf16 = m.k_bf16; p.row_cls = m.a_cls; p.col_seg = m.k_seg; p.col_cls = m.k_cls;
     p.row_cs = m.coef_s; p.row_cpn = m.coef_pn; p.row_neg = m.neg_sum;
     p.n_rows = m.N1; p.n_cols = m.N2; p.self_mask = m.self_mask; p.row_set = m.a_set; p.col_set = m.k_set;
+    p.n_rows_dev = m.n1_dev; p.n_cols_dev = m.n2_dev;
     p.scale_log2 = kLog2e / m.temperature; p.out_scale = m.weight / m.temperature;
     { const bool all = m.row_begin == 0 && m.row_end == 0;      // 0,0 = every row; begin == end = none
       p.rb_lo = (all ? 0 : m.row_begin) / 128; p.rb_hi = ((all ? m.N1 : m.row_end) + 127) / 128;
@@ -53,6 +55,7 @@ static inline int build_passes(const mscs_sim_job* job, BwdPass* out) {
       q.x_bf16 = m.k_bf16; q.y_bf16 = m.a_bf16; q.row_cls = m.k_cls; q.col_seg = m.a_seg; q.col_cls = m.a_cls;
       q.col_cs = m.coef_s; q.col_cpn = m.coef_pn; q.col_neg = m.neg_sum;
       q.n_rows = m.N2; q.n_cols = m.N1; q.self_mask = 0; q.row_set = m.k_set; q.col_set = m.a_set;
+      q.n_rows_dev = m.n2_dev; q.n_cols_dev = m.n1_dev;
       q.scale_log2 = p.scale_log2; q.out_scale = p.out_scale;
       { const bool all = m.krow_begin == 0 && m.krow_end == 0;
         q.rb_lo = (all ? 0 : m.krow_begin) / 128; q.rb_hi = ((all ? m.N2 : m.krow_end) + 127) / 128;

@@ -303,6 +303,9 @@ extern "C" int mscs_debug_sim_backward_simt(const mscs_sim_job* job, const float
   int rc = validate_job(job);
   if (rc) return rc;
   MSCS_CHECK_ARG(f32_sets && grad_out && dF_sets && dF_ld, "null pointer argument");
+  for (int t = 0; t < job->num_terms; ++t)
+    MSCS_CHECK_ARG(!job->terms[t].n1_dev && !job->terms[t].n2_dev,
+                   "term %d: the validation backward needs the actual row counts (n1_dev / n2_dev must be NULL)", t);
   cudaStream_t st = (cudaStream_t)stream_;
   BwdPass passes[MSCS_MAX_PASSES];
   const int np = build_passes(job, passes);

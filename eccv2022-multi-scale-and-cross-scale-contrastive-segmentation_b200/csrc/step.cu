@@ -8,7 +8,8 @@
 //   sample stream: [wait main] [wait draws] workspace fills -> histograms / plan -> plan records copied to the host on a
 //                  private stream -> selection (T, V, N read from the DEVICE plan records)
 //   main stream:   optional clear of the backward's accumulators, [wait sample] gather + normalise -> similarity forward (sweeps + finalise)
-//   host:          waits for the plan records only (errors, row counts for the backward)
+//   host:          waits for the plan records only (errors, row counts for the backward); with plan_host == NULL
+//                  nothing is fetched and nothing waits (CUDA graph capture: the consumers read the device records)
 // backward chain (autograd backward of the same): similarity backward -> normalisation backward + dense writer.
 #include "common.cuh"
 #include "../../include/mscs.h"
@@ -45,7 +46,7 @@ inline int mark(void* ev, cudaStream_t st) {
 
 extern "C" int mscs_forward_chain(const mscs_forward_chain_args* a, void* sample_stream_, void* main_stream_,
                                   mscs_scale_plan* plan_host) {
-  MSCS_CHECK_ARG(a && a->cfg && a->labels && a->workspace && a->plan_dev && a->job && a->gather_items && plan_host,
+  MSCS_CHECK_ARG(a && a->cfg && a->labels && a->workspace && a->plan_dev && a->job && a->gather_items,
                  "null pointer argument");
   MSCS_CHECK_ARG(a->gather_kind >= 0 && a->gather_kind <= 2, "gather_kind %d out of range", a->gather_kind);
   cudaStream_t ss = (cudaStream_t)sample_stream_, ms = (cudaStream_t)main_stream_;
@@ -66,7 +67,7 @@ extern "C" int mscs_forward_chain(const mscs_forward_chain_args* a, void* sample
     CHAIN(mscs_sample_plan_i16(a->cfg, (const int16_t*)a->labels, a->workspace, a->plan_dev, ss));
   else
     CHAIN(mscs_sample_plan(a->cfg, (const int64_t*)a->labels, a->workspace, a->plan_dev, ss));
-  CHAIN(mscs_plan_fetch_begin(a->plan_dev, S, ss));
+  if (plan_host) CHAIN(mscs_plan_fetch_begin(a->plan_dev, S, ss));
   CHAIN(mscs_sample_select_async(a->cfg, a->plan_dev, a->v_cap, a->workspace, a->draws, a->idx_ref, a->pair_ref, a->pix,
                                  a->cls, a->seg, a->slot, ss));
   CHAIN(mark(a->stage_events[1], ss));
@@ -83,6 +84,7 @@ extern "C" int mscs_forward_chain(const mscs_forward_chain_args* a, void* sample
   CHAIN(mark(a->stage_events[3], ms));
   CHAIN(mscs_sim_forward(a->job, ms));
   CHAIN(mark(a->stage_events[4], ms));
+  if (!plan_host) return 0;
   return mscs_plan_fetch_end(plan_host, S);      // the one host wait of the forward pass
 }
 

@@ -14,7 +14,8 @@ import sys
 import torch
 import torch.nn as nn
 
-from ._ops import CompactLabels, LossSpec, MsCsContrastiveFn
+from . import _ops
+from ._ops import GRAPH_CALL_BASE, CompactLabels, LossSpec, MsCsContrastiveFn
 from .datasets import class_facts
 
 
@@ -51,13 +52,52 @@ def _sampler_key(config):
     return s
 
 
-def _philox_key(module, holder):
-    if module._spec.sampler == "philox":
-        holder["philox"] = (module._spec.seed, module._sampler_calls)
-        module._sampler_calls += 1
+def _philox_key(module, holder, dev):
+    """Call index of the counter-based stream.  Eager calls use the host counter ``_sampler_calls`` (0, 1, ...).  A call
+    captured into a CUDA graph uses the module's int64 device counter instead (``graph_call_index``, created at the
+    first call on a device with the value 2**62): every replay reads it and increments it on the device, so replays
+    draw from the call indices 2**62, 2**62 + 1, ..., which eager calls never reach, and leave the host counter alone."""
+    if module._spec.sampler != "philox":
+        return
+    if dev.type == "cuda" and torch.cuda.is_current_stream_capturing():
+        holder["philox"] = (module._spec.seed, module._graph_counter)       # (None: refused by _ops.graph_mode)
+        return
+    if dev.type == "cuda" and (module._graph_counter is None or module._graph_counter.device != dev):
+        module._graph_counter = torch.full((), GRAPH_CALL_BASE, dtype=torch.int64, device=dev)
+    holder["philox"] = (module._spec.seed, module._sampler_calls)
+    module._sampler_calls += 1
 
 
-class DenseContrastiveLossV2(nn.Module):
+class _GraphReadout:
+    """What the loss classes share for CUDA graphs (INTEGRATION.md, "CUDA graphs"): the device call counter and the
+    readout of a captured call's results after a replay."""
+    _graph_counter = None
+
+    @property
+    def graph_call_index(self):
+        """0-d int64 CUDA tensor: the Philox call index the next replay of a captured call draws from (None before the
+        first call).  Assigning copies the value in place, so graphs already captured see it (checkpoint restore)."""
+        return self._graph_counter
+
+    @graph_call_index.setter
+    def graph_call_index(self, value):
+        if self._graph_counter is None:
+            raise RuntimeError("graph_call_index exists after the module's first call on a GPU")
+        self._graph_counter.copy_(torch.as_tensor(value, dtype=torch.int64))
+
+    def fetch_samples(self, state=None):
+        """ScaleSample list of the last call (``state``: of that call's state instead, e.g. a captured one).  For a
+        captured call, read from the device plan records of its latest replay (one synchronisation); it raises the
+        reference's exception when that replay's sampling failed."""
+        st = self.last_state if state is None else state
+        if not getattr(st, "graph", False):
+            return st.samples
+        _scalars, plan = _ops.fetch_graph_plan(st)
+        _ops._raise_plan_errors(plan, st.sp.S, st.sp.spec)
+        return _ops.graph_samples(st, plan)
+
+
+class DenseContrastiveLossV2(_GraphReadout, nn.Module):
     """Single-scale dense supervised contrastive loss.  ``forward(label, features)`` (argument
     order as in the reference, V2.py:44); returns the loss, or -- when ``cross_scale_contrast`` --
     the reference's 4-tuple ``(loss, sampled_features (T,C,V), sampled_labels (T,), False)``."""
@@ -84,12 +124,15 @@ class DenseContrastiveLossV2(nn.Module):
         if isinstance(label, CompactLabels):           # labels of the fused label pass (coloss.py): same results
             label = label.lab16
         holder = {}
-        _philox_key(self, holder)
+        _philox_key(self, holder, features.device)
         self._spec.num_classes = self.num_all_classes          # the reference lets callers override it (V2.py:238)
         total, _terms = MsCsContrastiveFn.apply(label, self._spec, True, holder, features)
-        smp = holder["samples"][0]
         self.last_samples, self.last_state = holder["samples"], holder["state"]
         self._scale = int(label.shape[-1] // features.shape[-1])                         # V2.py:46,203
+        if holder["samples"] is None:          # captured into a CUDA graph: see fetch_logged / fetch_samples
+            self.nan_flag = holder["state"].scalars[-1]
+            return total
+        smp = holder["samples"][0]
         if smp.log_flag:
             self.log_this_step = True                                                    # V2.py:75,83
         self.nan_flag = holder["state"].scalars[-1]      # 0-d device tensor: 1.0 if the loss is inf/NaN (no sync)
@@ -101,12 +144,13 @@ class DenseContrastiveLossV2(nn.Module):
             return total, sampled, smp.pair_ref[:, 1].float(), False
         return total
 
-    def fetch_logged(self):
-        """Scalars of the last call for the logger with a single device->host copy (see the _ms class)."""
-        return _fetch_logged(self, self.last_state, 1, [])
+    def fetch_logged(self, state=None):
+        """Scalars of the last call (or of `state`) for the logger with a single device->host copy (see the _ms
+        class)."""
+        return _fetch_logged(self, self.last_state if state is None else state, 1, [])
 
 
-class DenseContrastiveLossV2_ms(nn.Module):
+class DenseContrastiveLossV2_ms(_GraphReadout, nn.Module):
     """Multi-scale + cross-scale loss.  ``forward(label, features: list)`` (_ms.py:44).
 
     ``comm`` (not a reference argument) switches on the POOLED cross-batch mode: the loss is then the
@@ -145,28 +189,37 @@ class DenseContrastiveLossV2_ms(nn.Module):
         if self.cross_scale_contrast:
             assert len(feats) > 1                            # _ms.py:63
         holder = {"comm": self.comm}
-        _philox_key(self, holder)
+        _philox_key(self, holder, feats[0].device)
         total, terms = MsCsContrastiveFn.apply(label, self._spec, False, holder, *feats)
         state = holder["state"]
         self.last_samples, self.last_state = holder["samples"], state
         self.ms_losses = [terms[s] for s in range(state.num_ms)]
         self.cs_losses = [terms[i] for i in state.cs_logged]
         self.nan_flag = state.scalars[-1]                # 0-d device tensor: 1.0 if the loss is inf/NaN (no sync)
-        if any(s.log_flag for s in holder["samples"]):
+        if holder["samples"] is not None and any(s.log_flag for s in holder["samples"]):
             self.log_this_step = True
         return total
 
-    def fetch_logged(self):
+    def fetch_logged(self, state=None):
         """Scalars of the last call for the logger -- total, ms_losses, cs_losses (unweighted, as the reference logs
-        them) and the inf/NaN flag -- with a single device->host copy (SURVEY.md §8f item 3)."""
-        st = self.last_state
+        them) and the inf/NaN flag -- with a single device->host copy (SURVEY.md §8f item 3).  ``state``: the state of
+        another call, e.g. the ``last_state`` a CUDA graph capture left (its latest replay's values)."""
+        st = self.last_state if state is None else state
         return _fetch_logged(self, st, st.num_ms, st.cs_logged)
 
 
 def _fetch_logged(module, state, num_ms, cs_logged):
     """Everything the reference's logger reads per step, in ONE device->host copy (the reference does one
-    ``.item()`` per scalar plus ``has_inf_or_nan`` = 4+ syncs per step, LoggingManager.py:179-196)."""
-    v = state.scalars.detach().cpu().tolist()
+    ``.item()`` per scalar plus ``has_inf_or_nan`` = 4+ syncs per step, LoggingManager.py:179-196).  A captured call
+    reads its latest replay's plan records in the same copy: the logging flag, and the sampling errors, which raise
+    here as the eager forward would have raised them."""
+    if getattr(state, "graph", False):
+        v, plan = _ops.fetch_graph_plan(state)
+        _ops._raise_plan_errors(plan, state.sp.S, state.sp.spec)
+        if any(plan[s].log_flag for s in range(state.sp.S)):
+            module.log_this_step = True                                                  # V2.py:75,83
+    else:
+        v = state.scalars.detach().cpu().tolist()
     nt = len(v) - 2
     return {"total": v[nt], "ms_losses": v[:num_ms], "cs_losses": [v[i] for i in cs_logged],
             "has_inf_or_nan": v[nt + 1] != 0.0, "log_this_step": bool(module.log_this_step)}

@@ -140,6 +140,10 @@ int mscs_mt19937_stream(const uint32_t* mt_state_host, int mt_pos, uint64_t n_wo
  * buffer convention as mscs_mt19937_stream (the selection kernel tempers what it reads, so the words are stored through
  * the inverse tempering).  draws_dev: 16-byte aligned, n_words rounded up to a multiple of 4 words. */
 int mscs_philox_stream(uint64_t seed, uint64_t call, uint64_t n_words, uint32_t* draws_dev, void* stream);
+/* The same with the call index in DEVICE memory (a CUDA graph replays it unchanged): the words of
+ * mscs_philox_stream(seed, *call_dev, ...), then *call_dev += 1 in a one-thread launch behind the generator on `stream`.
+ * call_dev: 8-byte aligned. */
+int mscs_philox_stream_dev(uint64_t seed, uint64_t* call_dev, uint64_t n_words, uint32_t* draws_dev, void* stream);
 /* Phase 2 (async): per-pair Fisher-Yates prefix + rank->pixel selection from a precomputed stream.
  *   draws_dev : MT19937 stream starting at the generator position of this call;
  * outputs per scale s (arrays of N_s entries, N_s from the fetched plan):
@@ -224,9 +228,11 @@ typedef struct {
   float* s_sum;     /* sum_j pos 1/(e^l_ij + neg_i)     (backward, SURVEY.md App. A) */
   float* coef_s;    /* out: S_i/(div_i N1)  */
   float* coef_pn;   /* out: neg_i/(div_i N1) */
-  /* Optional (forward calls only): the row counts live in DEVICE memory (e.g. &plan_dev[s].N).  N1 / N2 above are
-   * then UPPER BOUNDS (they size grids, work tables and tensor maps) and the kernels read the actual counts, so the
-   * forward can be enqueued before the host has seen the sampling plan.  NULL = N1 / N2 are the actual counts. */
+  /* Optional: the row counts live in DEVICE memory (e.g. &plan_dev[s].N).  N1 / N2 above are then UPPER BOUNDS (they
+   * size grids, work tables and tensor maps) and the kernels read the actual counts, so the forward and the backward
+   * can be enqueued before the host has seen the sampling plan (or without it ever doing so: CUDA graphs).  NULL = N1 /
+   * N2 are the actual counts.  The backward takes them for every term or for none; rows beyond the counts contribute
+   * nothing, and a count of 0 gives an empty pass. */
   const int32_t* n1_dev; const int32_t* n2_dev;
 } mscs_term;
 
@@ -252,7 +258,8 @@ int mscs_sim_forward(const mscs_sim_job* job, void* stream);
 int mscs_sim_forward_sweeps(const mscs_sim_job* job, void* stream);
 int mscs_sim_finalize(const mscs_sim_job* job, void* stream);
 /* backward: dF[set] (N_set, C) fp32 += d total_loss / d unit rows * (*grad_out), for every
- * set; the caller zero-initialises dF.  grad_out is a device scalar (upstream gradient). */
+ * set; the caller zero-initialises dF.  grad_out is a device scalar (upstream gradient).  With device-resident row
+ * counts (mscs_term.n1_dev / n2_dev) only the rows below the counts are written. */
 int mscs_sim_backward(const mscs_sim_job* job, const float* grad_out, float* const* dF_sets,
                       const int32_t* dF_ld, void* stream);
 /* the same restricted to the passes whose row set s has bit s of `set_mask` set (pooled mode: one launch per
@@ -283,18 +290,21 @@ int mscs_scatter_grad(const float* dF, int ldF, const float* anc_f32, const floa
 int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream);
 int mscs_scatter_sectors(const float* dF, int ldF, const float* anc_f32, const float* inv_norm,
                          const int32_t* slot, int n, int C, int plane, float* dfeat, void* stream);
-/* every scale of a call in ONE launch.  `dtype` (last member, MSCS_DTYPE_*): element type of `dfeat`; the gradient rows
- * dF stay fp32.  mscs_scatter_sectors_batch takes fp32 items only. */
+/* every scale of a call in ONE launch.  `dtype` (MSCS_DTYPE_*): element type of `dfeat`; the gradient rows dF stay
+ * fp32.  mscs_scatter_sectors_batch takes fp32 items only.  `n_rows_dev` (last member, mscs_scatter_dense_batch only):
+ * NULL = `rows[s]` is the row count; else the count is read from device memory (e.g. &plan_dev[s].N) and `rows[s]` is
+ * its upper bound.  A zero-initialised tail is an fp32 item with a host count. */
 typedef struct {
   const float* dF; int32_t ldF; const float* anc_f32; const float* inv_norm; const int32_t* slot;
   int32_t n, C, plane; void* dfeat;
   int32_t dtype;
+  const int32_t* n_rows_dev;
 } mscs_scatter_item;
 int mscs_scatter_sectors_batch(const mscs_scatter_item* items, int count, void* stream);
 /* Channels-last feature maps (memory order [n][h][w][C]): an anchor is one contiguous row of C elements, so the gather
  * (+ L2 normalisation) and the scatter (normalisation backward into the pre-zeroed channels-last dense gradient) are
  * row copies driven by `pix` (global pixel id = image * plane + pixel of every sorted anchor row, -1 = not local).
- * `rows`: number of anchor rows, or their upper bound when `n_rows_dev` (device-resident count, gather only) is set.
+ * `rows`: number of anchor rows, or their upper bound when `n_rows_dev` (device-resident count) is set.
  * `dtype` (last member, MSCS_DTYPE_*): element type of `feat` and `dfeat`. */
 typedef struct {
   const void* feat; const int32_t* pix; const int32_t* n_rows_dev; int32_t rows, C;
@@ -321,7 +331,8 @@ int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows
  *           mscs_plan_fetch_begin, mscs_sample_select_async;  on `main_stream` (ordered after the selection): the
  *           batched gather + normalisation, mscs_sim_forward;  then mscs_plan_fetch_end -- the one host wait.
  *           Returns like the parts (0 = ok; plan_host[s].error holds the reference's error conditions).
- *           sample_stream == main_stream runs everything on one stream.
+ *           sample_stream == main_stream runs everything on one stream.  plan_host == NULL: no plan fetch and no host
+ *           wait -- the chain only enqueues work, and the sample stream joins back into main_stream (stream capture).
  * ------------------------------------------------------------------------------------- */
 typedef struct {
   const mscs_sample_cfg* cfg;
