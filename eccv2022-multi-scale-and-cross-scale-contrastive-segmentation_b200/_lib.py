@@ -95,14 +95,11 @@ _SIGNATURES = {
     "mscs_plan_fetch_end": (C.c_int, [C.POINTER(ScalePlan), C.c_int]),
     "mscs_sample_select_async": (C.c_int, [C.POINTER(SampleCfg), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                            _PTRS, _PTRS, _PTRS, _PTRS, _PTRS, _PTRS, C.c_void_p]),
-    "mscs_gather_normalize_sectors_async": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
-                                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mscs_gather_normalize_sectors_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
-    "mscs_gather_normalize_tma_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "mscs_scatter_sectors_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "mscs_gather_rows_nhwc_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "mscs_scatter_rows_nhwc_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
-    "mscs_scatter_dense_batch": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p, C.c_void_p]),
+    "mscs_scatter_dense_batch": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p]),
     "mscs_mt19937_stream": (C.c_int, [C.c_void_p, C.c_int, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mscs_philox_stream": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mscs_philox_stream_dev": (C.c_int, [C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
@@ -117,7 +114,7 @@ _SIGNATURES = {
     "mscs_sim_forward": (C.c_int, [C.POINTER(SimJob), C.c_void_p]),
     "mscs_forward_chain": (C.c_int, [C.POINTER(ForwardChainArgs), C.c_void_p, C.c_void_p, C.c_void_p]),
     "mscs_backward_chain": (C.c_int, [C.POINTER(SimJob), C.c_void_p, _PTRS, C.POINTER(C.c_int32), C.c_void_p,
-                                      C.POINTER(C.c_int32), C.c_int, C.c_void_p, _PTRS, C.c_void_p]),
+                                      C.POINTER(C.c_int32), C.c_int, _PTRS, C.c_void_p]),
     "mscs_sim_forward_sweeps": (C.c_int, [C.POINTER(SimJob), C.c_void_p]),
     "mscs_sim_finalize": (C.c_int, [C.POINTER(SimJob), C.c_void_p]),
     "mscs_sim_backward": (C.c_int, [C.POINTER(SimJob), C.c_void_p, _PTRS, C.POINTER(C.c_int32), C.c_void_p]),
@@ -127,8 +124,6 @@ _SIGNATURES = {
     "mscs_debug_sim_backward_simt": (C.c_int, [C.POINTER(SimJob), _PTRS, C.c_void_p, _PTRS, C.POINTER(C.c_int32),
                                                C.c_void_p]),
     "mscs_slot_map": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
-    "mscs_scatter_sectors": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
-                                       C.c_int, C.c_void_p, C.c_void_p]),
     "mscs_scatter_grad": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                     C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "mscs_label_pass": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

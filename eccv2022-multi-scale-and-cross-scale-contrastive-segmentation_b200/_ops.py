@@ -18,18 +18,10 @@ import torch
 from . import _lib
 
 _MT_N = 624
-# experiment switches, read once at import (nothing on the per-step path calls getenv)
-_NO_PREFETCH = bool(os.environ.get("MSCS_NO_PREFETCH"))      # regenerate the MT19937 stream inline at every call
+# tuning switch, read once at import (nothing on the per-step path calls getenv)
 _USE_HP_STREAM = os.environ.get("MSCS_HP", "1") != "0"       # sampling kernels on a high-priority stream
-# dense gradients: 1 (default) = ONE streaming pass in the backward (k_dense_stream: zeros and values alike, every byte
-# written once); 0 = zero-fill ahead of time on a side stream (memset) + rewrite of the sampled sectors.  Measured
-# (r02, cfg-2): 1.033-1.041 against 1.050-1.054 ms per step -- the memset costs the sampling and gather stages it
-# overlaps 14 + 45 us, the one-pass writer costs 37 us more than the sector rewrite.
-_DENSE_ONE_PASS = os.environ.get("MSCS_DENSE", "1") != "0"
-# K2 through bulk-tensor copies (MSCS_GATHER=tma) instead of strided lane loads: measured SLOWER at cfg-2 (0.137 against
-# 0.094 ms, r02: a box of {8 pixels x 256 channels} is 256 rows of 32 bytes, which the TMA unit streams at ~0.2 rows per
-# clock and SM), so the lane-load kernel stays the default
-_GATHER_TMA = os.environ.get("MSCS_GATHER", "lanes") == "tma"
+# NCHW dense gradients are written in ONE streaming pass by the backward (k_dense_stream); bench.py reads this flag
+_DENSE_ONE_PASS = True
 # element types the kernels read and write natively (MSCS_DTYPE_* codes of the C ABI); see half_io_ok
 _DTYPE_CODE = {torch.float32: _lib.DTYPE_F32, torch.bfloat16: _lib.DTYPE_BF16, torch.float16: _lib.DTYPE_F16}
 
@@ -327,8 +319,6 @@ class _StreamCache:
         """defer: only note the request; `flush` launches it.  The forward of a training step defers: between the plan
         fetch and the launch of the backward the host races ~0.35 ms of queued GPU work (cfg-2), and the generator
         launch (state upload, kernel, events: ~40 us) can as well follow the backward's launches."""
-        if _NO_PREFETCH:      # experiment switch: regenerate inline at the next call
-            return
         with self.lock:
             ev = torch.cuda.Event()
             ev.record(_cur_stream())
@@ -536,24 +526,6 @@ def sim_backward(state, sets, grad_out):
         _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), _lib.ptr_array(ptrs), lds, _stream()),
                    "mscs_sim_backward")
     return dFs
-
-
-def scatter_grad(dF, aset, sample, feat_shape, dtype, prezeroed=None, slot=None):
-    """Normalisation backward + dense gradient.  With a pre-zeroed buffer and a slot map only the
-    32-byte sectors that hold a sampled pixel are rewritten; otherwise zero-fill + scatter."""
-    lib = _lib.load()
-    n, Cc, h, w = feat_shape
-    if prezeroed is not None:
-        out = prezeroed
-        _lib.check(lib.mscs_scatter_sectors(dF.data_ptr(), dF.shape[1], aset.f32.data_ptr(),
-                                            aset.inv_norm.data_ptr(), slot.data_ptr(), n, Cc, h * w,
-                                            out.data_ptr(), _stream()), "mscs_scatter_sectors")
-    else:
-        out = torch.empty(feat_shape, dtype=torch.float32, device=dF.device)
-        _lib.check(lib.mscs_scatter_grad(dF.data_ptr(), dF.shape[1], aset.f32.data_ptr(), aset.inv_norm.data_ptr(),
-                                         sample.pix.data_ptr(), aset.N, n, Cc, h * w, out.data_ptr(), 1, _stream()),
-                   "mscs_scatter_grad")
-    return out if dtype == torch.float32 else out.to(dtype)
 
 
 class _GradBuffers:
@@ -874,12 +846,12 @@ def fast_path_ok(spec, world):
 
 def half_io_ok(sp, world):
     """Whether bf16 / fp16 feature maps are handed to the kernels as they are (no fp32 copy; the dense gradients are
-    written in the maps' dtype): the single-process fast path with the channels-last row gather, or with the NCHW lane
-    gather and the one-pass dense writer.  Every other route -- pooled mode, planes that are not a multiple of 8 pixels,
-    MSCS_GATHER=tma, MSCS_DENSE=0 -- converts the maps to fp32 first and the gradients back afterwards."""
+    written in the maps' dtype): the single-process fast path with the channels-last row gather, or with the NCHW octet
+    gather and the one-pass dense writer.  Every other route -- pooled mode, planes that are not a multiple of 8
+    pixels -- converts the maps to fp32 first and the gradients back afterwards."""
     if not fast_path_ok(sp.spec, world):
         return False
-    return sp.nhwc or (all(sp.slot_sizes) and _DENSE_ONE_PASS and not _GATHER_TMA)
+    return sp.nhwc or all(sp.slot_sizes)
 
 
 def channels_last_ok(spec, world, feats):
@@ -912,8 +884,6 @@ def graph_mode(spec, world, single_scale, labels, feats, counter):
                "use sampler='philox'")
     if single_scale and spec.cross_scale:
         refuse("DenseContrastiveLossV2 with cross_scale_contrast=True returns sampled features of a data-dependent shape")
-    if not _DENSE_ONE_PASS or _GATHER_TMA:
-        refuse("MSCS_DENSE=0 and MSCS_GATHER=tma take host-driven routes")
     if not fast_path_ok(spec, world):
         refuse("the selection table of this configuration exceeds the device-driven path's shared memory")
     if any(f.device != feats[0].device for f in feats) or labels.device != feats[0].device:
@@ -929,18 +899,17 @@ def graph_mode(spec, world, single_scale, labels, feats, counter):
 
 
 def _dense_grad_slab(shapes, dtypes, dev):
-    """ONE allocation for the dense gradients of the one-pass writer and its pixel-mask words behind them: the
-    per-scale gradient views (dtype `dtypes[j]`), their byte offsets, and the byte offset of the mask.  Planes are a
-    multiple of 8 pixels, so every part starts 16-byte aligned (the writer's 16-byte stores)."""
+    """ONE allocation for the dense gradients of the one-pass writer: the slab, the per-scale gradient views (dtype
+    `dtypes[j]`) and their byte offsets.  Planes are a multiple of 8 pixels, so every view starts 16-byte aligned (the
+    writer's 16-byte stores)."""
     nbytes = [shp[0] * shp[1] * shp[2] * shp[3] * dt.itemsize for shp, dt in zip(shapes, dtypes)]
-    mask_words = sum((shp[0] * shp[2] * shp[3] + 31) // 32 for shp in shapes)
-    slab = torch.empty(sum(nbytes) + 4 * mask_words, dtype=torch.uint8, device=dev)    # gradients | pixel mask
+    slab = torch.empty(sum(nbytes), dtype=torch.uint8, device=dev)
     views, offs, off = [], [], 0
     for shp, dt, nb in zip(shapes, dtypes, nbytes):
         views.append(slab[off:off + nb].view(dt).view(shp))
         offs.append(off)
         off += nb
-    return slab, views, offs, off
+    return slab, views, offs
 
 
 _hp_streams = {}
@@ -1105,7 +1074,7 @@ class _Workspace:
         ch.fill_ptrs, ch.fill_values = C.addressof(self.fill_ptrs), C.addressof(self.fill_vals)
         ch.fill_bytes, ch.n_fill = C.addressof(self.fill_bytes), 2
         ch.main_zero_ptr = self.dF_ptr
-        ch.gather_kind = 1 if sp.nhwc else (2 if _GATHER_TMA else 0)
+        ch.gather_kind = 1 if sp.nhwc else 0
         ch.gather_items, ch.job = C.addressof(self.gitems), C.addressof(self.job_fwd)
 
 
@@ -1204,13 +1173,12 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
             _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws, ch.draws,
                                               st_s), "mscs_philox_stream")
     _t = _seg("fwd: rng state + stream acquire", _t)
-    # dense gradients + gradient rows: pre-zeroed on a side stream, sampled sectors rewritten by the backward
-    # (default: the backward writes them in one streaming pass instead, see _DENSE_ONE_PASS and gather.cu).
+    # channels-last dense gradients + gradient rows: pre-zeroed on a side stream, sampled rows written by the backward
+    # (NCHW maps need no fill: the backward writes their dense gradients in one streaming pass, see gather.cu).
     # Started here, next to the small sampling kernels: the fill (535 MB at cfg-2) costs ~70 us of step time
     # WHEREVER it runs (measured next to the sampling kernels, under the forward, under the backward, and as a
     # device-to-device copy from a persistent zero buffer) -- memset and D2D copies run on the SMs.
-    gradbufs = _GradBuffers(feats32, needs, sp.nhwc, sp.dF_n) \
-        if (any(needs) and (sp.nhwc or not _DENSE_ONE_PASS)) else None
+    gradbufs = _GradBuffers(feats32, needs, sp.nhwc, sp.dF_n) if (any(needs) and sp.nhwc) else None
     if gradbufs is not None:
         if graph:       # filled on the caller's stream: a forward captured without its backward leaves no open fork
             gradbufs.side = cur
@@ -1228,12 +1196,10 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
     # plan, with the addresses entered into the backward's prebuilt structures -- not in the window after the wait
     grad_slab = grad_outs = None
     if dF_in_ws and all(needs) and not sp.nhwc:
-        grad_slab, grad_outs, offs, mask_off = _dense_grad_slab([f.shape for f in feats32], [f.dtype for f in feats32],
-                                                                dev)
+        grad_slab, grad_outs, offs = _dense_grad_slab([f.shape for f in feats32], [f.dtype for f in feats32], dev)
         sbase = grad_slab.data_ptr()
         for j in range(S):
             e.bw_items[j].dfeat, e.bw_items[j].dtype = sbase + offs[j], _DTYPE_CODE[feats32[j].dtype]
-        grad_mask_ptr = sbase + mask_off
     evs = None
     if TIMING is not None and TIMING_ALL and not graph:      # stage accounting (bench.py): five events INSIDE the chain
         evs = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
@@ -1280,7 +1246,6 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
     state.num_ms, state.cs_logged, state.comm = S, sp.cs_logged, None
     state.dF_ws = e.dF_ptr if dF_in_ws else None
     state.grad_slab, state.grad_outs = grad_slab, grad_outs
-    state.grad_mask_ptr = grad_mask_ptr if grad_slab is not None else None
     state.io_dtypes = [f.dtype for f in feats32]
     if not graph:
         for s in range(S):
@@ -1624,12 +1589,11 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
         if pre is not None:                 # allocated and entered into the prebuilt structures by the forward
             state.grad_slab = None
             slab, items, rows = pre, e.bw_items, e.bw_rows
-            outs, mask_ptr = dict(enumerate(state.grad_outs)), state.grad_mask_ptr
+            outs = dict(enumerate(state.grad_outs))
             state.grad_outs = None
         else:
-            slab, views, offs, mask_off = _dense_grad_slab([shapes[s] for s in idx], [io[s] for s in idx], dev)
+            slab, views, offs = _dense_grad_slab([shapes[s] for s in idx], [io[s] for s in idx], dev)
             sbase = slab.data_ptr()
-            mask_ptr = sbase + mask_off
             outs = {}
             items = (_lib.ScatterItem * max(1, len(idx)))()
             rows = (C.c_int32 * max(1, len(idx)))()
@@ -1648,7 +1612,7 @@ def run_backward(state, grad_out, needs, shapes, dtypes):
                 ev.record()         # creates the CUDA event; the chain records it again at its stage boundary
             evp = _lib.ptr_array([ev.cuda_event for ev in evs] + [None] * (3 - len(evs)))
         _lib.check(lib.mscs_backward_chain(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, items, rows,
-                                           len(idx), mask_ptr, evp, st), "mscs_backward_chain")
+                                           len(idx), evp, st), "mscs_backward_chain")
         if not graph:
             _stream_cache(dev).flush()    # the deferred generator launch of the next call's stream
         if evs is not None:

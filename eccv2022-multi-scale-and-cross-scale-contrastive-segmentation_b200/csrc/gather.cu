@@ -5,8 +5,7 @@
 //             a dense zero (n,C,h,w) gradient at the sampled pixels.
 // HBM-bound byte movers: NCHW means one anchor is C scalars `plane` floats apart (one 32 B
 // sector per useful 4 B), so one warp owns one anchor and keeps 8 independent loads in flight.
-#include "sim_tc.cuh"
-#include <stdlib.h>
+#include "common.cuh"
 
 namespace mscs {
 
@@ -174,117 +173,6 @@ __global__ void __launch_bounds__(256) k_gather_sectors_batch(const __grid_const
                       g.n_rows_dev[s]);
 }
 
-// ---------------------------------------------------------------------------------------
-// Gather through TMA (round 2; opt-in, MSCS_GATHER=tma -- measured slower than the octet kernel: 0.137 against 0.094 ms
-// at cfg-2, the TMA unit handles the 256 32-byte rows of a box at ~0.2 rows per clock and SM).  The octet kernel above issues, per sampled pixel, 8 load instructions whose 32 lanes
-// hit 32 different channel planes: 256 L1 wavefronts per pixel -- the LSU, not DRAM, bounds it (93 us at cfg-2 with the
-// stream to itself, 2.9 TB/s of sector traffic).  Here the strided walk over the channel planes is ONE bulk-tensor
-// copy per 8-pixel octet: the feature map is described as a 2D tensor [n*C rows][plane columns] and a box of
-// {8 pixels, C rows} (C x 32 bytes, exactly the sectors the octet kernel touches) lands in shared memory as
-// tile[c][8 px]; the lanes then read 32-byte rows of it (two 128-bit loads per channel) and hold all eight pixels of
-// their channels in registers.  Block = 4 warps; a block first compacts the octets of its 1024-pixel chunk of the slot
-// map that hold a sampled pixel, then every warp streams its share through two tile slots (the copy of the next octet
-// is in flight while the current one is normalised and stored).
-// ---------------------------------------------------------------------------------------
-constexpr int kTmaOctets = 128;      // octets per block chunk (1024 pixels)
-struct GatherTma {
-  alignas(64) CUtensorMap map[MSCS_MAX_SCALES];
-  const int* slot[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
-  __nv_bfloat16* bf16[MSCS_MAX_SCALES]; float* f32[MSCS_MAX_SCALES]; float* inv[MSCS_MAX_SCALES];
-  int C[MSCS_MAX_SCALES], plane[MSCS_MAX_SCALES], n_oct[MSCS_MAX_SCALES], block0[MSCS_MAX_SCALES + 1];
-  int count;
-};
-__global__ void __launch_bounds__(128) k_gather_tma_batch(const __grid_constant__ GatherTma g) {
-  extern __shared__ uint8_t smem_raw[];
-  pdl_trigger();
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 127) & ~uintptr_t(127));
-  float* tiles = reinterpret_cast<float*>(smem);                       // [4 warps][2 slots][kMaxC][8]
-  int* l_oct = reinterpret_cast<int*>(smem + 4 * 2 * kMaxC * 32);     // compacted octets of the chunk
-  uint64_t* bars = reinterpret_cast<uint64_t*>(l_oct + kTmaOctets);   // [4 warps][2 slots]
-  int* cnt = reinterpret_cast<int*>(bars + 8);
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
-  const int lb = (int)blockIdx.x - g.block0[s], nb = g.block0[s + 1] - g.block0[s];
-  const int C = g.C[s], C_pad = (C + 63) / 64 * 64, plane = g.plane[s];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (lb == nb - 1) {      // padding rows [N, N_pad) of the operand matrix (the TMA tiles of K3 read them)
-    const int N = *g.n_rows_dev[s], N_pad = (N + 255) / 256 * 256;
-    uint32_t* z = reinterpret_cast<uint32_t*>(g.bf16[s] + (size_t)N * C_pad);
-    for (int i = threadIdx.x; i < (N_pad - N) * (C_pad / 2); i += blockDim.x) z[i] = 0u;
-    return;
-  }
-  if (threadIdx.x == 0) {
-    *cnt = 0;
-    for (int i = 0; i < 8; ++i) ptx::mbar_init(&bars[i], 1);
-    ptx::fence_barrier_init();
-  }
-  __syncthreads();
-  {      // one octet per thread: keep those with a sampled pixel
-    const int oct = lb * kTmaOctets + (int)threadIdx.x;
-    if (oct < g.n_oct[s]) {
-      const int4 a = *reinterpret_cast<const int4*>(g.slot[s] + (size_t)oct * 8);
-      const int4 b = *reinterpret_cast<const int4*>(g.slot[s] + (size_t)oct * 8 + 4);
-      if ((a.x & a.y & a.z & a.w & b.x & b.y & b.z & b.w) >= 0) l_oct[atomicAdd(cnt, 1)] = oct;      // any entry >= 0
-    }
-  }
-  __syncthreads();
-  const int total = *cnt;
-  float* my_tiles = tiles + (size_t)warp * 2 * kMaxC * 8;
-  uint64_t* my_bars = bars + warp * 2;
-  const uint32_t tx = (uint32_t)C * 32u;
-  auto issue = [&](int k, int slot_i) {      // lane 0: bulk copy of octet l_oct[k] into tile slot slot_i
-    const int oct = l_oct[k];
-    const int gp = oct * 8, b = gp / plane, p = gp - b * plane;
-    ptx::mbar_expect_tx(&my_bars[slot_i], tx);
-    ptx::tma_load_2d(my_tiles + (size_t)slot_i * kMaxC * 8, &g.map[s], &my_bars[slot_i], p, b * C);
-  };
-  int k = warp;
-  if (k < total && lane == 0) issue(k, 0);
-  uint32_t n_done = 0;
-  for (; k < total; k += 4, ++n_done) {
-    const int cur = n_done & 1;
-    if (k + 4 < total && lane == 0) issue(k + 4, cur ^ 1);      // the other slot was consumed two iterations ago
-    ptx::mbar_wait(&my_bars[cur], (n_done >> 1) & 1, 301);
-    const int oct = l_oct[k];
-    const int row_mine = lane < 8 ? g.slot[s][(size_t)oct * 8 + lane] : -1;
-    const float* tile = my_tiles + (size_t)cur * kMaxC * 8;
-    float v[kMaxC / 32][8];
-#pragma unroll
-    for (int q = 0; q < kMaxC / 32; ++q) {
-      const int c = lane + 32 * q;
-      if (c < C) {
-        const float4 lo = *reinterpret_cast<const float4*>(tile + c * 8);
-        const float4 hi = *reinterpret_cast<const float4*>(tile + c * 8 + 4);
-        v[q][0] = lo.x; v[q][1] = lo.y; v[q][2] = lo.z; v[q][3] = lo.w;
-        v[q][4] = hi.x; v[q][5] = hi.y; v[q][6] = hi.z; v[q][7] = hi.w;
-      } else {
-#pragma unroll
-        for (int j = 0; j < 8; ++j) v[q][j] = 0.f;
-      }
-    }
-    __syncwarp();      // every lane has read its rows: the slot may be refilled by the issue of the next iteration
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int row = __shfl_sync(0xffffffffu, row_mine, j);
-      if (row < 0) continue;      // warp-uniform
-      float ss = 0.f;
-#pragma unroll
-      for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q][j], v[q][j], ss);
-      ss = warp_sum(ss);
-      const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
-      if (lane == 0) g.inv[s][row] = inv;
-      __nv_bfloat16* orow = g.bf16[s] + (size_t)row * C_pad;
-#pragma unroll
-      for (int q = 0; q < kMaxC / 32; ++q) {
-        const int c = lane + 32 * q;
-        const float f = v[q][j] * inv;
-        if (c < C) g.f32[s][(size_t)row * C + c] = f;
-        if (c < C_pad) orow[c] = __float2bfloat16(c < C ? f : 0.f);
-      }
-    }
-  }
-}
-
 // slot map: slot[image*plane + pixel] = sorted anchor row sampled there, or -1
 __global__ void k_slot_map(const int* __restrict__ pix, int N, int* __restrict__ slot) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -368,49 +256,22 @@ k_scatter_sectors_pull(const __grid_constant__ PullRows pull, int ldF, const flo
 
 
 // ---------------------------------------------------------------------------------------
-// Dense gradient in ONE streaming pass -- OPT-IN alternative (MSCS_DENSE=1) to "zero-fill ahead of time + rewrite
-// the sampled sectors".  The 535 MB zero fill is not really hidden (memset / copy kernels take the SMs away from
-// whatever they overlap: ~70 us of step time wherever it was scheduled), so here every byte of the dense gradient
-// is written exactly once, zeros and values alike.  Measured: the writer reaches only 3.3 TB/s (a plain fill: 7),
-// 0.170 ms against 0.107 + ~0.065 for the default path -- a wash, so it is not the default.  (Variants tried: 8
-// channel planes per thread, 4 float4 per thread with the loads hoisted, a shared-memory mask tile: all slower.)
+// Dense gradient in ONE streaming pass: every byte of the dense gradient is written exactly once, zeros and values
+// alike, so no zero fill has to run ahead of the backward (a 535 MB fill at cfg-2 is not hidden by overlapping it:
+// memset / copy kernels take the SMs away from whatever they run next to, ~70 us of step time wherever it was put).
 //   k_dx_rows:      dF row -> dx row in place   (normalisation backward, N x C, tiny)
-//   k_dense_write:  out[b][c][p..p+3] = slot[b][p+i] >= 0 ? dx[slot][c] : 0   (one float4 per thread)
+//   k_dense_stream: out[b][c][p..p+P) = slot[b][p+i] >= 0 ? dx[slot][c] : 0   (below, after the channels-last kernels)
 // ---------------------------------------------------------------------------------------
 struct DenseBatch {
   float* dF[MSCS_MAX_SCALES]; const float* f32[MSCS_MAX_SCALES]; const float* inv[MSCS_MAX_SCALES];
-  const int* slot[MSCS_MAX_SCALES]; float* dfeat[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
+  const int* slot[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES];
   int ldF[MSCS_MAX_SCALES], C[MSCS_MAX_SCALES], plane[MSCS_MAX_SCALES], n[MSCS_MAX_SCALES], rows[MSCS_MAX_SCALES];
-  long long v4_0[MSCS_MAX_SCALES + 1];      // block prefix of the dense writer
   int rowblk0[MSCS_MAX_SCALES + 1];         // block prefix of the row kernel (8 rows per block)
-  uint32_t* mask[MSCS_MAX_SCALES];          // 1 bit per pixel: sampled or not (built by the row kernel's extra blocks)
-  int maskblk0[MSCS_MAX_SCALES + 1];        // block prefix of the mask blocks (8192 pixels per block), after the row blocks
   int count;
 };
 
 __global__ void __launch_bounds__(256) k_dx_rows(const __grid_constant__ DenseBatch g) {
   int s = 0;
-  if ((int)blockIdx.x >= g.rowblk0[g.count]) {
-    // ---- mask blocks: one 32-bit word per 32 pixels of the slot map (the dense writer then reads 1 bit per pixel
-    // instead of a 4-byte slot entry per pixel and channel) ----
-    const int mb = (int)blockIdx.x - g.rowblk0[g.count];
-    while (s + 1 < g.count && mb >= g.maskblk0[s + 1]) ++s;
-    const unsigned npix = (unsigned)g.n[s] * (unsigned)g.plane[s];
-    const unsigned w = (unsigned)(mb - g.maskblk0[s]) * 256u + threadIdx.x;      // word index
-    if (w * 32u >= npix) return;
-    uint32_t bits = 0;
-    const int* sl = g.slot[s] + (size_t)w * 32;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-      if (w * 32u + i * 4u < npix) {          // npix is a multiple of 4
-        const int4 q = __ldg(reinterpret_cast<const int4*>(sl) + i);
-        bits |= (uint32_t)(q.x >= 0) << (4 * i) | (uint32_t)(q.y >= 0) << (4 * i + 1) |
-                (uint32_t)(q.z >= 0) << (4 * i + 2) | (uint32_t)(q.w >= 0) << (4 * i + 3);
-      }
-    }
-    g.mask[s][w] = bits;
-    return;
-  }
   while (s + 1 < g.count && (int)blockIdx.x >= g.rowblk0[s + 1]) ++s;
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.rowblk0[s]) * 8 + (threadIdx.x >> 5);
@@ -434,41 +295,6 @@ __global__ void __launch_bounds__(256) k_dx_rows(const __grid_constant__ DenseBa
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
     if (c < C) gr[c] = (clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv;
-  }
-}
-
-// Purely sequential writer (the order a memset would use: interleaving several channel planes per block measured
-// slower): block = 2048 consecutive floats of the flattened [b][c][pixel] gradient of ONE scale, thread = two float4.
-// One mask bit per pixel says whether anything was sampled there (97.5 % of the float4 at cfg-2 are plain zero
-// stores); only then the slot entries and the dx values are fetched.  32-bit index arithmetic; v4_0 holds BLOCK
-// prefixes per scale.
-__global__ void __launch_bounds__(256) k_dense_write(const __grid_constant__ DenseBatch g) {
-  int s = 0;
-  while (s + 1 < g.count && (long long)blockIdx.x >= g.v4_0[s + 1]) ++s;
-  const unsigned blk = blockIdx.x - (unsigned)g.v4_0[s];
-  const unsigned plane = (unsigned)g.plane[s], C = (unsigned)g.C[s];
-  const unsigned total = (unsigned)g.n[s] * C * plane;                          // floats of this scale (< 2^32)
-  const uint32_t* __restrict__ mask = g.mask[s];
-  float* __restrict__ out = g.dfeat[s];
-#pragma unroll
-  for (int u = 0; u < 2; ++u) {
-    const unsigned f = blk * 2048u + (u * 256u + threadIdx.x) * 4u;
-    if (f >= total) return;
-    const unsigned bc = f / plane, p = f - bc * plane;
-    const unsigned b = bc / C, c = bc - b * C;
-    const unsigned lin = b * plane + p;
-    const uint32_t m = (__ldg(mask + (lin >> 5)) >> (lin & 31u)) & 0xFu;
-    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (m) {
-      const int4 sl = *reinterpret_cast<const int4*>(g.slot[s] + lin);
-      const float* __restrict__ dx = g.dF[s];
-      const int ld = g.ldF[s];
-      if (sl.x >= 0) v.x = dx[(size_t)sl.x * ld + c];
-      if (sl.y >= 0) v.y = dx[(size_t)sl.y * ld + c];
-      if (sl.z >= 0) v.z = dx[(size_t)sl.z * ld + c];
-      if (sl.w >= 0) v.w = dx[(size_t)sl.w * ld + c];
-    }
-    __stcs(reinterpret_cast<float4*>(out + f), v);
   }
 }
 
@@ -557,7 +383,7 @@ __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant
   }
 }
 
-// One-pass dense writer, second form (round 2): a thread OWNS 4 consecutive pixels and walks the channel planes.
+// One-pass dense writer: a thread OWNS 4 consecutive pixels and walks the channel planes.
 // Its four slot entries are fetched once (one coalesced int4), so the sampled / not-sampled decision is loop
 // invariant: 97 % of the threads run a pure store loop, the others add up to four independent (predicated) loads of
 // dx[row][c] per channel.  A block writes 2 KB contiguous per channel plane (512 pixels), i.e. whole DRAM pages in
@@ -645,40 +471,11 @@ extern "C" int mscs_scatter_rows_raw(const float* drows, int ld, const int32_t* 
   return 0;
 }
 
-// Same, with the number of sampled rows read from device memory (`n_rows_dev`, e.g. &plan_dev[s].N): no host
-// knowledge of the sampling result is needed to enqueue it.
-extern "C" int mscs_gather_normalize_sectors_async(const float* feat, int n, int C, int plane, const int32_t* slot,
-                                                   const int32_t* n_rows_dev, void* anc_bf16, float* anc_f32,
-                                                   float* inv_norm, void* stream_) {
-  MSCS_CHECK_ARG(feat && slot && n_rows_dev && anc_bf16 && anc_f32 && inv_norm, "null pointer argument");
-  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC, "C=%d unsupported (1..%d)", C, kMaxC);
-  MSCS_CHECK_ARG(n >= 1 && plane >= 8 && plane % 8 == 0, "bad sizes (plane must be a multiple of 8)");
-  cudaStream_t st = (cudaStream_t)stream_;
-  const int C_pad = (C + 63) / 64 * 64;
-  const int n_oct = n * (plane / 8);
-  k_gather_sectors<<<ceil_div(n_oct, 8) + 1, 256, 0, st>>>(feat, C, C_pad, plane, slot, n_oct, (__nv_bfloat16*)anc_bf16,
-                                                           anc_f32, inv_norm, n_rows_dev);
-  MSCS_LAUNCH_CHECK();
-  return 0;
-}
-
 extern "C" int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream_) {
   MSCS_CHECK_ARG(pix && slot && N >= 1 && n_pixels >= 1, "bad arguments");
   cudaStream_t st = (cudaStream_t)stream_;
   MSCS_CUDA(cudaMemsetAsync(slot, 0xff, sizeof(int) * (size_t)n_pixels, st));
   k_slot_map<<<ceil_div(N, 256), 256, 0, st>>>(pix, N, slot);
-  MSCS_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int mscs_scatter_sectors(const float* dF, int ldF, const float* anc_f32, const float* inv_norm,
-                                    const int32_t* slot, int n, int C, int plane, float* dfeat, void* stream_) {
-  MSCS_CHECK_ARG(dF && anc_f32 && inv_norm && slot && dfeat, "null pointer argument");
-  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC && ldF >= C, "C=%d / ldF=%d unsupported", C, ldF);
-  MSCS_CHECK_ARG(plane % 8 == 0, "plane %d is not a multiple of 8 pixels: use mscs_scatter_grad", plane);
-  const int n_oct = n * (plane / 8);
-  k_scatter_sectors<<<ceil_div(n_oct, 8), 256, 0, (cudaStream_t)stream_>>>(dF, ldF, anc_f32, inv_norm, slot, n_oct,
-                                                                           C, plane, dfeat, 0);
   MSCS_LAUNCH_CHECK();
   return 0;
 }
@@ -753,42 +550,6 @@ extern "C" int mscs_gather_normalize_sectors_batch(const mscs_gather_item* items
   if (int rc = gather_sectors_launch<float>(items, count, MSCS_DTYPE_F32, st)) return rc;
   if (int rc = gather_sectors_launch<__nv_bfloat16>(items, count, MSCS_DTYPE_BF16, st)) return rc;
   return gather_sectors_launch<__half>(items, count, MSCS_DTYPE_F16, st);
-}
-
-// the same gather through bulk-tensor copies (k_gather_tma_batch)
-extern "C" int mscs_gather_normalize_tma_batch(const mscs_gather_item* items, int count, void* stream_) {
-  MSCS_CHECK_ARG(items && count >= 1 && count <= MSCS_MAX_SCALES, "bad item count %d", count);
-  GatherTma g{};
-  g.count = count;
-  int blocks = 0;
-  for (int s = 0; s < count; ++s) {
-    const mscs_gather_item& it = items[s];
-    MSCS_CHECK_ARG(it.feat && it.slot && it.n_rows_dev && it.anc_bf16 && it.anc_f32 && it.inv_norm,
-                   "item %d: null pointer argument", s);
-    MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC, "item %d: C=%d unsupported (1..%d)", s, it.C, kMaxC);
-    MSCS_CHECK_ARG(it.n >= 1 && it.plane >= 8 && it.plane % 8 == 0, "item %d: plane must be a multiple of 8", s);
-    MSCS_CHECK_ARG((uintptr_t)it.feat % 16 == 0, "item %d: feature map must be 16-byte aligned", s);
-    if (int rc = check_dtype(s, it.dtype, it.feat, 16, "feat")) return rc;
-    MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32, "item %d: the TMA gather reads fp32 feature maps only", s);
-    if (make_tensor_map_2d(&g.map[s], (int)CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, it.feat, (unsigned long long)it.plane,
-                           (unsigned long long)it.n * it.C, (unsigned long long)it.plane * 4, 8, (unsigned)it.C))
-      return -1;
-    g.slot[s] = it.slot; g.n_rows_dev[s] = it.n_rows_dev;
-    g.bf16[s] = (__nv_bfloat16*)it.anc_bf16; g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm;
-    g.C[s] = it.C; g.plane[s] = it.plane; g.n_oct[s] = it.n * (it.plane / 8);
-    g.block0[s] = blocks;
-    blocks += ceil_div(g.n_oct[s], kTmaOctets) + 1;      // + the block that zeroes the padding rows
-  }
-  g.block0[count] = blocks;
-  const size_t smem = 128 + (size_t)4 * 2 * kMaxC * 32 + sizeof(int) * kTmaOctets + 8 * sizeof(uint64_t) + 16;
-  static bool attr_done = false;
-  if (!attr_done) {
-    MSCS_CUDA(cudaFuncSetAttribute(k_gather_tma_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    attr_done = true;
-  }
-  k_gather_tma_batch<<<blocks, 128, smem, (cudaStream_t)stream_>>>(g);
-  MSCS_LAUNCH_CHECK();
-  return 0;
 }
 
 struct ScatterBatch {
@@ -871,14 +632,11 @@ static int dense_stream_launch(const DenseBatch& g, const mscs_scatter_item* ite
   return 0;
 }
 
-extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count,
-                                        uint32_t* mask_scratch, void* stream_) {
-  MSCS_CHECK_ARG(items && rows && mask_scratch && count >= 1 && count <= MSCS_MAX_SCALES, "bad arguments");
+extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count, void* stream_) {
+  MSCS_CHECK_ARG(items && rows && count >= 1 && count <= MSCS_MAX_SCALES, "bad arguments");
   DenseBatch g{};
   g.count = count;
-  long long v4 = 0;
-  int rb = 0, mblk = 0;
-  size_t mask_words = 0;
+  int rb = 0;
   for (int s = 0; s < count; ++s) {
     const mscs_scatter_item& it = items[s];
     MSCS_CHECK_ARG(it.dF && it.anc_f32 && it.inv_norm && it.slot && it.dfeat, "item %d: null pointer argument", s);
@@ -888,30 +646,13 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
     MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32 || it.plane % 8 == 0,
                    "item %d: half gradients need a plane that is a multiple of 8 pixels (plane %d)", s, it.plane);
     g.dF[s] = const_cast<float*>(it.dF); g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot;
-    g.dfeat[s] = (float*)it.dfeat; g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = rows[s];
+    g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = rows[s];
     g.n_rows_dev[s] = it.n_rows_dev;
     MSCS_CHECK_ARG((long long)it.n * it.C * it.plane < (1ll << 32), "item %d: more than 2^32 gradient elements", s);
-    g.v4_0[s] = v4;      // block prefix: 2048 floats per block
-    v4 += ((long long)it.n * it.C * it.plane + 2047) / 2048;
-    g.mask[s] = mask_scratch + mask_words;
-    g.maskblk0[s] = mblk;
-    { const long long words = ((long long)it.n * it.plane + 31) / 32;
-      mask_words += (size_t)words; mblk += (int)((words + 255) / 256); }
     g.rowblk0[s] = rb; rb += ceil_div(rows[s], 8);
   }
-  g.v4_0[count] = v4; g.rowblk0[count] = rb; g.maskblk0[count] = mblk;
+  g.rowblk0[count] = rb;
   cudaStream_t st = (cudaStream_t)stream_;
-  static const int writer = [] { const char* e = getenv("MSCS_DENSE_WRITER"); return e ? atoi(e) : 1; }();
-  if (writer == 0) {      // first form (round 1): linear float4 walk with a pixel mask
-    for (int s = 0; s < count; ++s)
-      MSCS_CHECK_ARG(items[s].dtype == MSCS_DTYPE_F32, "item %d: MSCS_DENSE_WRITER=0 writes fp32 gradients only", s);
-    k_dx_rows<<<rb + mblk, 256, 0, st>>>(g);
-    MSCS_LAUNCH_CHECK();
-    k_dense_write<<<(unsigned)v4, 256, 0, st>>>(g);
-    MSCS_LAUNCH_CHECK();
-    return 0;
-  }
-  g.maskblk0[count] = 0;      // no mask blocks: k_dx_rows only turns the gradient rows into dx rows
   k_dx_rows<<<rb > 0 ? rb : 1, 256, 0, st>>>(g);
   MSCS_LAUNCH_CHECK();
   if (int rc = dense_stream_launch<float>(g, items, MSCS_DTYPE_F32, st)) return rc;

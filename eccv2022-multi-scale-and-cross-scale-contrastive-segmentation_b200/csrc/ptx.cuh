@@ -360,18 +360,6 @@ __device__ __forceinline__ uint64_t ex2_poly2(uint64_t v, uint64_t scale2) {
   const uint32_t plo = (uint32_t)p, phi = (uint32_t)(p >> 32), tlo = (uint32_t)t, thi = (uint32_t)(t >> 32);
   return pack2u(plo + (tlo << 23), phi + (thi << 23));
 }
-// degree-3 variant (max relative error 7.5e-5): for results that are rounded to bf16 anyway (backward W)
-__device__ __forceinline__ uint64_t ex2_poly2_d3(uint64_t v, uint64_t scale2) {
-  const uint64_t magic = pack2(12582912.f, 12582912.f), nmagic = pack2(-12582912.f, -12582912.f);
-  const uint64_t t = fma2(v, scale2, magic);
-  const uint64_t n = add2(t, nmagic);
-  const uint64_t f = fma2(v, scale2, n ^ 0x8000000080000000ull);
-  uint64_t p = fma2(pack2(0.055171653628349304f, 0.055171653628349304f), f, pack2(0.2426111251115799f, 0.2426111251115799f));
-  p = fma2(p, f, pack2(0.6932609677314758f, 0.6932609677314758f));
-  p = fma2(p, f, pack2(0.9999280571937561f, 0.9999280571937561f));
-  const uint32_t plo = (uint32_t)p, phi = (uint32_t)(p >> 32), tlo = (uint32_t)t, thi = (uint32_t)(t >> 32);
-  return pack2u(plo + (tlo << 23), phi + (thi << 23));
-}
 __device__ __forceinline__ float lg2(float x) {
   float y;
   asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));

@@ -51,7 +51,6 @@ struct BwdArgs {
   BwdDev p[MSCS_MAX_PASSES];
   WorkTable work;
   const float* grad_out;
-  int flags;
   // DEV instance only: device-resident row / column counts of every pass (n_rows / n_cols are then upper bounds).
   // Kept behind every field the eager instance reads, so that instance compiles as it did without them.
   const int* rows_dev[MSCS_MAX_PASSES]; const int* cols_dev[MSCS_MAX_PASSES];
@@ -321,17 +320,11 @@ __global__ void __launch_bounds__(kBwdThreads, 1) k_sim_bwd(const __grid_constan
               const float4 cc = *reinterpret_cast<const float4*>(cs_s + c);
 #pragma unroll
               for (int q = 0; q < 2; ++q) {
-                // every second pair takes its exponentials from the FMA pipe (degree-3 polynomial, 7.5e-5 relative --
-                // W is rounded to bf16 right after): the MUFU unit (16/clk/SM) otherwise keeps this conversion, which
-                // sits on the S -> dX critical path of every tile, at ~750 cycles
-                uint64_t e2;
-                if (q == 1 && (args.flags & 128)) {      // experiment only: measured slower (FMA pipe becomes the bound)
-                  e2 = ptx::ex2_poly2_d3(ptx::pack2u(v[c + 2 * q], v[c + 2 * q + 1]), scale2);
-                } else {
-                  float x0, x1;
-                  ptx::unpack2(ptx::mul2(ptx::pack2u(v[c + 2 * q], v[c + 2 * q + 1]), scale2), x0, x1);
-                  e2 = ptx::pack2(ptx::ex2(x0), ptx::ex2(x1));
-                }
+                // (MUFU only: a degree-3 polynomial on the FMA pipe for every second pair measured slower -- the FMA
+                // pipe becomes the bound)
+                float x0, x1;
+                ptx::unpack2(ptx::mul2(ptx::pack2u(v[c + 2 * q], v[c + 2 * q + 1]), scale2), x0, x1);
+                const uint64_t e2 = ptx::pack2(ptx::ex2(x0), ptx::ex2(x1));
                 const uint64_t c2 = ptx::add2(rcs2, q == 0 ? ptx::pack2(cc.x, cc.y) : ptx::pack2(cc.z, cc.w));
                 float w0, w1;
                 ptx::unpack2(ptx::mul2(e2, c2), w0, w1);
@@ -467,8 +460,6 @@ extern "C" int mscs_sim_backward_sets(const mscs_sim_job* job, const float* grad
             2 * (align_up(sizeof(WorkItem) * fwd_items, 64) + align_up(sizeof(int) * (fwd_items + 1), 64));
   BwdArgs args{};
   args.grad_out = grad_out;
-  static const int dbg_flags = [] { const char* e = getenv("MSCS_DEBUG_FLAGS"); return e ? atoi(e) : 0; }();
-  args.flags = dbg_flags;      // experiments only, read once per process
   const void* bases[MSCS_MAX_SCALES]; int nmaps = 0;
   auto map_of = [&](const void* base, int rows) -> int {
     for (int i = 0; i < nmaps; ++i) if (bases[i] == base) return i;

@@ -71,24 +71,15 @@ __host__ __device__ constexpr size_t fwd_smem_bytes(int KB) {
   return 1024 /*alignment slack*/ + (size_t)(2 * KB + kFwdStages) * kBlkBytes + 256 /*barriers*/;
 }
 
-// 32 unmasked logits -> partial sums of exp2(v * scale), TWO elements per instruction wherever the pipe allows it
-// (packed fp32x2 multiply / add / polynomial; MUFU.EX2 itself is scalar).  Bit ((c >> 1) & 7) of POLY selects the
-// element PAIRS whose exponential is evaluated as a degree-4 polynomial on the FMA pipe instead of MUFU.EX2: the MUFU
-// unit (16 results/clk/SM) is the epilogue's bottleneck next to the issue slots.  Per pair: MUFU path = FMUL2 + 2 MUFU
-// + FADD2 (2 issue slots per element), polynomial path = 7 FFMA2 + 2 (shift, add) per element + FADD2.
-template <int POLY>
+// 16 unmasked logits -> partial sums of exp2(v * scale), TWO elements per instruction wherever the pipe allows it
+// (packed fp32x2 multiply / add; MUFU.EX2 itself is scalar).  Per pair: FMUL2 + 2 MUFU + FADD2.  (Moving a share of
+// the exponentials to a polynomial on the FMA pipe measured no faster, DESIGN.md §4.)
 __device__ __forceinline__ void fast_chunk(const uint32_t (&cur)[16], uint64_t scale2, uint64_t& acc_a, uint64_t& acc_b) {
 #pragma unroll
   for (int c = 0; c < 16; c += 2) {
-    const uint64_t v2 = ptx::pack2u(cur[c], cur[c + 1]);
-    uint64_t e2;
-    if ((POLY >> ((c >> 1) & 7)) & 1) {
-      e2 = ptx::ex2_poly2(v2, scale2);
-    } else {
-      float x0, x1;
-      ptx::unpack2(ptx::mul2(v2, scale2), x0, x1);
-      e2 = ptx::pack2(ptx::ex2(x0), ptx::ex2(x1));
-    }
+    float x0, x1;
+    ptx::unpack2(ptx::mul2(ptx::pack2u(cur[c], cur[c + 1]), scale2), x0, x1);
+    const uint64_t e2 = ptx::pack2(ptx::ex2(x0), ptx::ex2(x1));
     if (c & 2) acc_b = ptx::add2(acc_b, e2); else acc_a = ptx::add2(acc_a, e2);
   }
 }
@@ -97,13 +88,12 @@ __device__ __forceinline__ void fast_chunk(const uint32_t (&cur)[16], uint64_t s
 // inside the key set), otherwise per-element masks.  (16 columns: two chunks in flight cost 32 registers, which
 // leaves the compiler room to overlap the MUFU latencies of neighbouring pairs; with 32-column chunks every pair
 // went through the same register pair.)
-template <int POLY>
 __device__ __forceinline__ void neg_chunk(const uint32_t (&cur)[16], int c0, int tN2, int wmin, int wmax, int p0,
                                           unsigned plen, float scale, uint64_t scale2, uint64_t& acc_a, uint64_t& acc_b,
                                           float& acc_m) {
   const bool fast = (c0 + 16 <= wmin || c0 >= wmax) && (c0 + 16 <= tN2);
   if (fast) {
-    fast_chunk<POLY>(cur, scale2, acc_a, acc_b);
+    fast_chunk(cur, scale2, acc_a, acc_b);
   } else if (c0 < tN2) {
 #pragma unroll
     for (int c = 0; c < 16; ++c) {
@@ -120,8 +110,7 @@ __device__ __forceinline__ void neg_chunk(const uint32_t (&cur)[16], int c0, int
 static __device__ unsigned long long g_cta_span[2][160][4];
 #endif
 
-// POLY: pair mask of fast_chunk (sweep 0 only): 0x88 = a quarter of the exponentials on the FMA pipe
-template <int KB, int MODE, int POLY>
+template <int KB, int MODE>
 __global__ void __launch_bounds__(kFwdThreads, 1) k_sim_fwd(const __grid_constant__ FwdArgs args) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -282,10 +271,10 @@ __global__ void __launch_bounds__(kFwdThreads, 1) k_sim_fwd(const __grid_constan
 #pragma unroll 1
             for (int c4 = 0; c4 < NC16; c4 += 2) {
               ptx::tmem_ld16(taddr + (c4 + 1) * 16, vb);
-              neg_chunk<POLY>(va, cb + c4 * 16, tN2, wmin, wmax, p0, plen, scale, scale2, acc_a, acc_b, acc0);
+              neg_chunk(va, cb + c4 * 16, tN2, wmin, wmax, p0, plen, scale, scale2, acc_a, acc_b, acc0);
               ptx::tmem_ld_wait16(vb);
               if (c4 + 2 < NC16) ptx::tmem_ld16(taddr + (c4 + 2) * 16, va);
-              neg_chunk<POLY>(vb, cb + (c4 + 1) * 16, tN2, wmin, wmax, p0, plen, scale, scale2, acc_a, acc_b, acc0);
+              neg_chunk(vb, cb + (c4 + 1) * 16, tN2, wmin, wmax, p0, plen, scale, scale2, acc_a, acc_b, acc0);
               if (c4 + 2 < NC16) ptx::tmem_ld_wait16(va);
             }
           }
@@ -513,34 +502,6 @@ int make_tensor_map(CUtensorMap* out, const void* base, int rows, int c_pad) {
   return 0;
 }
 
-// generic 2D tiled tensor map (no swizzle): `rows` x `cols` elements of `elem_bytes`, row pitch in bytes, box in elements
-int make_tensor_map_2d(CUtensorMap* out, int dtype, int elem_bytes, const void* base, unsigned long long cols,
-                       unsigned long long rows, unsigned long long row_pitch_bytes, unsigned box_cols, unsigned box_rows) {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qr;
-    MSCS_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr));
-    MSCS_CHECK_ARG(p != nullptr && qr == cudaDriverEntryPointSuccess, "cuTensorMapEncodeTiled not available");
-    fn = (EncodeTiledFn)p;
-  }
-  (void)elem_bytes;
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)row_pitch_bytes};
-  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = CUDA_SUCCESS;
-  for (int attempt = 0; attempt < 2; ++attempt) {
-    r = fn(out, (CUtensorMapDataType)dtype, 2, const_cast<void*>(base), dims, strides, box, estr,
-           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_ERROR_INVALID_CONTEXT) break;      // see make_tensor_map
-    MSCS_CUDA(cudaFree(nullptr));
-  }
-  MSCS_CHECK_ARG(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (2d) failed with CUresult %d", (int)r);
-  return 0;
-}
-
 int launch_build_work(const BuildArgs& b, cudaStream_t st) {
   MSCS_CUDA(launch_k(k_build_work, b.items1 ? 2 : 1, 1024, 0, st, b));
   MSCS_LAUNCH_CHECK();
@@ -565,14 +526,10 @@ int persistent_ctas() {
 }
 
 // environment switches of the tuning experiments, read ONCE per process (no getenv on the per-step path)
-struct FwdTuning { int poly, pad; bool timeline; };
+struct FwdTuning { int pad; bool timeline; };
 static const FwdTuning& fwd_tuning() {
   static const FwdTuning t = [] {
-    FwdTuning v{0, 0, false};
-    // share of the exponentials evaluated as a polynomial on the FMA pipe: 0 = none (default: measured fastest with the
-    // packed epilogue, r02: 0.302 ms for the forward stage against 0.308 (1/4), 0.308 (3/8), 0.313 (1/2)), 1 = 1/4,
-    // 2 = 3/8, 3 = 1/2
-    if (const char* e = getenv("MSCS_FWD_POLY")) v.poly = atoi(e);
+    FwdTuning v{0, false};
     if (const char* e = getenv("MSCS_FWD_PAD")) v.pad = atoi(e);
     v.timeline = getenv("MSCS_FWD_TIMELINE") != nullptr;
     return v;
@@ -580,15 +537,15 @@ static const FwdTuning& fwd_tuning() {
   return t;
 }
 
-template <int KB, int MODE, int POLY>
+template <int KB, int MODE>
 static int launch_fwd_k(const FwdArgs& args, cudaStream_t st) {
   const size_t smem = fwd_smem_bytes(KB);
   static bool attr_done = false;      // per instantiation
   if (!attr_done) {
-    MSCS_CUDA(cudaFuncSetAttribute(k_sim_fwd<KB, MODE, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MSCS_CUDA(cudaFuncSetAttribute(k_sim_fwd<KB, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_done = true;
   }
-  MSCS_CUDA(launch_k(k_sim_fwd<KB, MODE, POLY>, persistent_ctas(), kFwdThreads, smem, st, args));
+  MSCS_CUDA(launch_k(k_sim_fwd<KB, MODE>, persistent_ctas(), kFwdThreads, smem, st, args));
   MSCS_LAUNCH_CHECK();
   return 0;
 }
@@ -596,16 +553,7 @@ static int launch_fwd_k(const FwdArgs& args, cudaStream_t st) {
 template <int KB>
 static int launch_fwd(const FwdArgs& args, int mode, cudaStream_t st) {
   if (int rc = ensure_trap_buffer()) return rc;
-  if (mode == 1) return launch_fwd_k<KB, 1, 0>(args, st);
-  if (KB == 4) {      // the polynomial share is a tuning switch for the 256-channel kernels only
-    switch (fwd_tuning().poly) {
-      case 1: return launch_fwd_k<KB, 0, 0x88>(args, st);
-      case 2: return launch_fwd_k<KB, 0, 0x92>(args, st);
-      case 3: return launch_fwd_k<KB, 0, 0xAA>(args, st);
-      default: break;
-    }
-  }
-  return launch_fwd_k<KB, 0, 0x00>(args, st);
+  return mode == 1 ? launch_fwd_k<KB, 1>(args, st) : launch_fwd_k<KB, 0>(args, st);
 }
 
 }  // namespace mscs

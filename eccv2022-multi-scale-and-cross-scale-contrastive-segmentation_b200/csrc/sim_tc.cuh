@@ -77,8 +77,5 @@ int persistent_ctas();   // grid of the persistent tensor kernels (SM count minu
 
 // TMA tensor map for a row-major (rows, C_pad) bf16 matrix, box = {64 elements, 128 rows}, 128B swizzle
 int make_tensor_map(CUtensorMap* out, const void* base, int rows, int c_pad);
-// generic 2D tiled map without swizzle (dtype: a CUtensorMapDataType value)
-int make_tensor_map_2d(CUtensorMap* out, int dtype, int elem_bytes, const void* base, unsigned long long cols,
-                       unsigned long long rows, unsigned long long row_pitch_bytes, unsigned box_cols, unsigned box_rows);
 
 }  // namespace mscs

@@ -48,7 +48,7 @@ extern "C" int mscs_forward_chain(const mscs_forward_chain_args* a, void* sample
                                   mscs_scale_plan* plan_host) {
   MSCS_CHECK_ARG(a && a->cfg && a->labels && a->workspace && a->plan_dev && a->job && a->gather_items,
                  "null pointer argument");
-  MSCS_CHECK_ARG(a->gather_kind >= 0 && a->gather_kind <= 2, "gather_kind %d out of range", a->gather_kind);
+  MSCS_CHECK_ARG(a->gather_kind >= 0 && a->gather_kind <= 1, "gather_kind %d out of range", a->gather_kind);
   cudaStream_t ss = (cudaStream_t)sample_stream_, ms = (cudaStream_t)main_stream_;
   const int S = a->cfg->num_scales;
   const bool two = ss != ms;
@@ -76,11 +76,10 @@ extern "C" int mscs_forward_chain(const mscs_forward_chain_args* a, void* sample
     MSCS_CUDA(cudaStreamWaitEvent(ms, ev->to_main, 0));
   }
   CHAIN(mark(a->stage_events[2], ms));
-  switch (a->gather_kind) {
-    case 0: CHAIN(mscs_gather_normalize_sectors_batch((const mscs_gather_item*)a->gather_items, S, ms)); break;
-    case 1: CHAIN(mscs_gather_rows_nhwc_batch((const mscs_rows_item*)a->gather_items, S, ms)); break;
-    default: CHAIN(mscs_gather_normalize_tma_batch((const mscs_gather_item*)a->gather_items, S, ms)); break;
-  }
+  if (a->gather_kind == 0)
+    CHAIN(mscs_gather_normalize_sectors_batch((const mscs_gather_item*)a->gather_items, S, ms));
+  else
+    CHAIN(mscs_gather_rows_nhwc_batch((const mscs_rows_item*)a->gather_items, S, ms));
   CHAIN(mark(a->stage_events[3], ms));
   CHAIN(mscs_sim_forward(a->job, ms));
   CHAIN(mark(a->stage_events[4], ms));
@@ -90,12 +89,12 @@ extern "C" int mscs_forward_chain(const mscs_forward_chain_args* a, void* sample
 
 extern "C" int mscs_backward_chain(const mscs_sim_job* job, const float* grad_out, float* const* dF_sets,
                                    const int32_t* dF_ld, const mscs_scatter_item* items, const int32_t* rows, int count,
-                                   uint32_t* mask_scratch, void* const* stage_events, void* stream_) {
+                                   void* const* stage_events, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
   if (stage_events) CHAIN(mark(stage_events[0], st));
   CHAIN(mscs_sim_backward(job, grad_out, dF_sets, dF_ld, st));
   if (stage_events) CHAIN(mark(stage_events[1], st));
-  if (count > 0) CHAIN(mscs_scatter_dense_batch(items, rows, count, mask_scratch, st));
+  if (count > 0) CHAIN(mscs_scatter_dense_batch(items, rows, count, st));
   if (stage_events) CHAIN(mark(stage_events[2], st));
   return 0;
 }

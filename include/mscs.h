@@ -183,11 +183,8 @@ int mscs_gather_normalize(const float* feat, int n, int C, int plane, const int3
  * reads inside open DRAM pages; needs plane % 8 == 0 */
 int mscs_gather_normalize_sectors(const float* feat, int n, int C, int plane, const int32_t* slot, int N,
                                   void* anc_bf16, float* anc_f32, float* inv_norm, void* stream);
-/* Same with the row count read from device memory (e.g. &plan_dev[s].N); also zeroes the padding rows. */
-int mscs_gather_normalize_sectors_async(const float* feat, int n, int C, int plane, const int32_t* slot,
-                                        const int32_t* n_rows_dev, void* anc_bf16, float* anc_f32, float* inv_norm,
-                                        void* stream);
-/* every scale of a call in ONE launch (device-driven form, see above).  `dtype` (MSCS_DTYPE_*, last member: a
+/* every scale of a call in ONE launch, device-driven: the row count is read from device memory (`n_rows_dev`, e.g.
+ * &plan_dev[s].N) and the padding rows are zeroed inside the call.  `dtype` (MSCS_DTYPE_*, last member: a
  * zero-initialised item is fp32) is the element type of `feat`; scales of different dtypes may be mixed (one launch
  * per dtype present).  The outputs are the same for a half map and for its exact fp32 widening. */
 typedef struct {
@@ -196,10 +193,6 @@ typedef struct {
   int32_t dtype;
 } mscs_gather_item;
 int mscs_gather_normalize_sectors_batch(const mscs_gather_item* items, int count, void* stream);
-/* The same gather with the strided walk over the channel planes done by the TMA unit: one bulk-tensor copy of
- * {8 pixels x C channels} per octet of the slot map that holds a sampled pixel, staged in shared memory
- * (feature maps 16-byte aligned; fp32 items only). */
-int mscs_gather_normalize_tma_batch(const mscs_gather_item* items, int count, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * K3 / K4 -- fused similarity + loss forward and backward for every term of one call.
@@ -282,14 +275,12 @@ int mscs_scatter_grad(const float* dF, int ldF, const float* anc_f32, const floa
                       const int32_t* pix, int N, int n, int C, int plane, float* dfeat,
                       int zero_fill, void* stream);
 
-/* Fast path of the scatter when the caller has ALREADY zero-filled dfeat (the host side does that
+/* Scatter when the caller has ALREADY zero-filled dfeat (the host side does that
  * on a side stream while the tensor kernels run) and plane % 8 == 0:
- *   mscs_slot_map        slot[image*plane + pixel] = sorted anchor row sampled there, else -1
- *   mscs_scatter_sectors rewrites, with full 32-byte sector stores, only the sectors of dfeat that
- *                        hold a sampled pixel (same maths as mscs_scatter_grad). */
+ *   mscs_slot_map              slot[image*plane + pixel] = sorted anchor row sampled there, else -1
+ *   mscs_scatter_sectors_batch rewrites, with full 32-byte sector stores, only the sectors of dfeat that
+ *                              hold a sampled pixel (same maths as mscs_scatter_grad). */
 int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream);
-int mscs_scatter_sectors(const float* dF, int ldF, const float* anc_f32, const float* inv_norm,
-                         const int32_t* slot, int n, int C, int plane, float* dfeat, void* stream);
 /* every scale of a call in ONE launch.  `dtype` (MSCS_DTYPE_*): element type of `dfeat`; the gradient rows dF stay
  * fp32.  mscs_scatter_sectors_batch takes fp32 items only.  `n_rows_dev` (last member, mscs_scatter_dense_batch only):
  * NULL = `rows[s]` is the row count; else the count is read from device memory (e.g. &plan_dev[s].N) and `rows[s]` is
@@ -317,10 +308,8 @@ int mscs_scatter_rows_nhwc_batch(const mscs_rows_item* items, int count, void* s
 /* Dense gradients of every scale written in ONE streaming pass, zeros included (no pre-zeroed buffer needed):
  * dF rows are first turned into dx rows IN PLACE (rows[s] rows of item s), then every 16 bytes of every dfeat are
  * written once (4 fp32 or 8 half pixels of a channel plane per store).  plane must be a multiple of 4 (fp32) or 8
- * (bf16 / fp16), dfeat 16-byte aligned.  mask_scratch: sum over items of ceil(n*plane/32) uint32 words (one bit per
- * pixel: sampled or not, built inside the call). */
-int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count, uint32_t* mask_scratch,
-                             void* stream);
+ * (bf16 / fp16), dfeat 16-byte aligned. */
+int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * One forward / one backward of the single-process path in ONE call each (csrc/step.cu): the same entry points as
@@ -348,8 +337,8 @@ typedef struct {
   void* const* fill_ptrs; const int32_t* fill_values; const size_t* fill_bytes; int32_t n_fill;   /* mscs_fill_bytes */
   void* main_zero_ptr; size_t main_zero_bytes;   /* optional: cleared on main_stream while the sampling chain runs (the
                                       gradient-row accumulators of the backward) */
-  int32_t gather_kind;             /* 0: NCHW (mscs_gather_item[num_scales], lane loads), 1: channels-last rows
-                                      (mscs_rows_item[num_scales]), 2: NCHW through bulk-tensor copies */
+  int32_t gather_kind;             /* 0: NCHW (mscs_gather_item[num_scales]), 1: channels-last rows
+                                      (mscs_rows_item[num_scales]) */
   const void* gather_items;
   const mscs_sim_job* job;         /* forward job (upper bounds + device-resident row counts) */
   void* stage_events[5];           /* optional cudaEvent_t, recorded at: sampling start / end (sample stream), gather
@@ -360,8 +349,8 @@ int mscs_forward_chain(const mscs_forward_chain_args* args, void* sample_stream,
 /* backward: mscs_sim_backward, then mscs_scatter_dense_batch (count may be 0: no dense gradient wanted).
  * stage_events: NULL or 3 optional cudaEvent_t recorded before / between / after the two. */
 int mscs_backward_chain(const mscs_sim_job* job, const float* grad_out, float* const* dF_sets, const int32_t* dF_ld,
-                        const mscs_scatter_item* items, const int32_t* rows, int count, uint32_t* mask_scratch,
-                        void* const* stage_events, void* stream);
+                        const mscs_scatter_item* items, const int32_t* rows, int count, void* const* stage_events,
+                        void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Co-loss on the same label read (SURVEY.md 8f item 2).  The reference's LossWrapper evaluates a class-weighted

@@ -293,7 +293,7 @@ def _expect_bad(rc, lib):
 
 
 @pytest.mark.parametrize("bad", [-1, 3])
-def test_bad_dtype_in_items_is_rejected(bad):
+def test_bad_dtype_in_batched_items_is_rejected(bad):
     import mscs_b200
     from mscs_b200 import _lib
     lib = mscs_b200.load()
@@ -301,7 +301,6 @@ def test_bad_dtype_in_items_is_rejected(bad):
     g[0].feat = g[0].slot = g[0].n_rows_dev = g[0].anc_bf16 = g[0].anc_f32 = g[0].inv_norm = _FAKE
     g[0].n, g[0].C, g[0].plane, g[0].dtype = 1, 64, 8, bad
     _expect_bad(lib.mscs_gather_normalize_sectors_batch(g, 1, None), lib)
-    _expect_bad(lib.mscs_gather_normalize_tma_batch(g, 1, None), lib)
     r = (_lib.RowsItem * 1)()
     r[0].feat = r[0].pix = r[0].anc_bf16 = r[0].anc_f32 = r[0].inv_norm = r[0].dF = r[0].dfeat = _FAKE
     r[0].rows, r[0].C, r[0].ldF, r[0].dtype = 1, 64, 64, bad
@@ -311,7 +310,7 @@ def test_bad_dtype_in_items_is_rejected(bad):
     sc[0].dF = sc[0].anc_f32 = sc[0].inv_norm = sc[0].slot = sc[0].dfeat = _FAKE
     sc[0].ldF, sc[0].n, sc[0].C, sc[0].plane, sc[0].dtype = 64, 1, 64, 8, bad
     rows = (C.c_int32 * 1)(1)
-    _expect_bad(lib.mscs_scatter_dense_batch(sc, rows, 1, _FAKE, None), lib)
+    _expect_bad(lib.mscs_scatter_dense_batch(sc, rows, 1, None), lib)
     _expect_bad(lib.mscs_scatter_sectors_batch(sc, 1, None), lib)
 
 
@@ -323,14 +322,10 @@ def test_bad_dtype_in_ce_is_rejected(bad):
     _expect_bad(lib.mscs_ce_backward(_FAKE, _FAKE, 1, 19, 8, None, 19, _FAKE, _FAKE, _FAKE, None, bad), lib)
 
 
-def test_half_items_rejected_where_only_fp32_is_implemented():
+def test_half_items_rejected_by_fp32_sector_scatter():
     import mscs_b200
     from mscs_b200 import _lib
     lib = mscs_b200.load()
-    g = (_lib.GatherItem * 1)()
-    g[0].feat = g[0].slot = g[0].n_rows_dev = g[0].anc_bf16 = g[0].anc_f32 = g[0].inv_norm = _FAKE
-    g[0].n, g[0].C, g[0].plane, g[0].dtype = 1, 64, 8, _lib.DTYPE_BF16
-    assert lib.mscs_gather_normalize_tma_batch(g, 1, None) < 0 and b"fp32" in lib.mscs_last_error()
     sc = (_lib.ScatterItem * 1)()
     sc[0].dF = sc[0].anc_f32 = sc[0].inv_norm = sc[0].slot = sc[0].dfeat = _FAKE
     sc[0].ldF, sc[0].n, sc[0].C, sc[0].plane, sc[0].dtype = 64, 1, 64, 8, _lib.DTYPE_F16

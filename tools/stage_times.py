@@ -1,4 +1,4 @@
-"""Per-stage device times of cfg2 steps (run on the GPU box); honours MSCS_DEBUG_FLAGS experiments."""
+"""Per-stage device times of cfg2 steps (run on a GPU)."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -41,7 +41,7 @@ print(f"wall/step {t_all/50*1e3:.3f} ms; host blocked in the plan fetch {sum(_op
 _ops.TIMING = {}
 for _ in range(30): step()
 torch.cuda.synchronize()
-print(os.environ.get("MSCS_DEBUG_FLAGS", "0"), {k: round(sum(a.elapsed_time(b) for a, b in v) / len(v), 4) for k, v in _ops.TIMING.items()})
+print({k: round(sum(a.elapsed_time(b) for a, b in v) / len(v), 4) for k, v in _ops.TIMING.items()})
 
 if os.environ.get("MSCS_FWD_TIMELINE"):
     import ctypes, numpy as np
