@@ -224,8 +224,12 @@ typedef struct {
   /* Optional: the row counts live in DEVICE memory (e.g. &plan_dev[s].N).  N1 / N2 above are then UPPER BOUNDS (they
    * size grids, work tables and tensor maps) and the kernels read the actual counts, so the forward and the backward
    * can be enqueued before the host has seen the sampling plan (or without it ever doing so: CUDA graphs).  NULL = N1 /
-   * N2 are the actual counts.  The backward takes them for every term or for none; rows beyond the counts contribute
-   * nothing, and a count of 0 gives an empty pass. */
+   * N2 are the actual counts.  The backward takes them for every term or for none; a count of 0 gives an empty pass.
+   * Rows [count, count rounded up to 256) of the operand matrix must be ZERO, as the gathers write them: the kernels
+   * load whole 128-row tiles and 256-key blocks, and the backward keeps the row coefficient of a column at or beyond
+   * the count (W = e * cS_i != 0), so those columns add nothing only because their rows are zero.  Rows at or above
+   * the count rounded up to 256 are never read, and class ids at or above the count are never read.  Statistics and
+   * coefficients of rows at or above the count are not written, gradient rows there are not touched. */
   const int32_t* n1_dev; const int32_t* n2_dev;
 } mscs_term;
 
