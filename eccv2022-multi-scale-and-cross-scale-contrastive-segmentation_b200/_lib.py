@@ -133,9 +133,8 @@ _SIGNATURES = {
                                   C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "mscs_ce_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
-    "mscs_gather_rows_raw": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
-    "mscs_scatter_rows_raw": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
-                                        C.c_void_p]),
+    "mscs_gather_raw_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "mscs_gather_raw_rows_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "mscs_xchg_alloc": (C.c_int, [C.c_size_t, C.POINTER(C.c_void_p), C.c_char_p]),
     "mscs_xchg_open": (C.c_int, [C.c_char_p, C.POINTER(C.c_void_p)]),
     "mscs_xchg_close": (C.c_int, [C.c_void_p]),

@@ -865,12 +865,13 @@ def channels_last_ok(spec, world, feats):
 GRAPH_CALL_BASE = 2 ** 62
 
 
-def graph_mode(spec, world, single_scale, labels, feats, counter):
+def graph_mode(spec, world, single_scale, labels, feats, counter, plan_of=None):
     """Whether this call is being captured into a CUDA graph (``torch.cuda.graph``), which the single-process fast path
     with sampler='philox' supports: the call then enqueues work without ever waiting for the host (the row counts stay
     on the device, the Philox call index is read from ``counter``).  Everything that cannot be captured raises a
     RuntimeError here, before anything is enqueued, so that the capture still ends cleanly.  Outside a capture: False
-    (the eager path, unchanged)."""
+    (the eager path, unchanged).  ``plan_of(nhwc)``: the caller's cached plan of these inputs, or None before its first
+    eager call (default: the step plan of the loss classes)."""
     if not (feats[0].is_cuda and torch.cuda.is_current_stream_capturing()):      # (a CUDA tensor: a runtime exists)
         return False
 
@@ -891,8 +892,11 @@ def graph_mode(spec, world, single_scale, labels, feats, counter):
     nhwc = channels_last_ok(spec, world, feats)
     if not nhwc and any((f.shape[2] * f.shape[3]) % 8 for f in feats):
         refuse("feature planes that are not a multiple of 8 pixels take the host-driven path")
-    sp = _step_plan(feats[0].device, labels.shape, [tuple(f.shape) for f in feats], spec, single_scale, world, 0, nhwc,
-                    create=False)
+    if plan_of is None:
+        sp = _step_plan(feats[0].device, labels.shape, [tuple(f.shape) for f in feats], spec, single_scale, world, 0,
+                        nhwc, create=False)
+    else:
+        sp = plan_of(nhwc)
     if sp is None or counter is None or counter.device != feats[0].device:
         refuse("run one eager call with the same shapes and configuration before capturing (warm-up)")
     return True

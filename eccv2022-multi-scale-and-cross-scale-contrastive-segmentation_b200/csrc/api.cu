@@ -59,7 +59,7 @@ extern "C" int mscs_debug_trap_info(char* out, int len) {
   return n;
 }
 
-extern "C" const char* mscs_version(void) { return "mscs 0.4.0 (sm_100a, tcgen05/TMA; items carry dtype; device row counts)"; }
+extern "C" const char* mscs_version(void) { return "mscs 0.5.0 (sm_100a, tcgen05/TMA; items carry dtype; device row counts; batched raw rows)"; }
 extern "C" const char* mscs_last_error(void) { return mscs::get_error(); }
 extern "C" int mscs_device_ok(void) {
   int n = 0;

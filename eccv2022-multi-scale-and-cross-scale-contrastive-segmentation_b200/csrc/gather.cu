@@ -173,6 +173,16 @@ __global__ void __launch_bounds__(256) k_gather_sectors_batch(const __grid_const
                       g.n_rows_dev[s]);
 }
 
+// Projector-tail path: the sampled c-vectors as they are (no normalisation), same octet walk.  The slot map holds the
+// sampled rows only, so the row count is not needed; rows the call does not sample are not touched.
+template <typename T>
+__global__ void __launch_bounds__(256) k_gather_raw_batch(const __grid_constant__ GatherBatch g) {
+  int s = 0;
+  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  gather_sectors_body<T>(blockIdx.x - g.block0[s], g.block0[s + 1] - g.block0[s], static_cast<const T*>(g.feat[s]), g.C[s],
+                         0, g.plane[s], g.slot[s], g.n_oct[s], nullptr, g.f32[s], nullptr, nullptr);
+}
+
 // slot map: slot[image*plane + pixel] = sorted anchor row sampled there, or -1
 __global__ void k_slot_map(const int* __restrict__ pix, int N, int* __restrict__ slot) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -203,14 +213,6 @@ scatter_sectors_body(const float* __restrict__ dF, int ldF, const float* __restr
     const int row = __shfl_sync(0xffffffffu, s_mine, j);
     if (row >= 0) {                                   // warp-uniform
       const float* g = (pull ? pull->p[row / pull->rows_per_rank] : dF) + (size_t)row * ldF;
-      if (anc_f32 == nullptr) {      // raw mode (projector-tail path): the rows ARE the pixel gradients
-#pragma unroll
-        for (int q = 0; q < kMaxC / 32; ++q) {
-          const int c = lane + 32 * q;
-          dx[j][q] = (c < C) ? g[c] : 0.f;
-        }
-        continue;
-      }
       const float* f = anc_f32 + (size_t)row * C;
       float gv[kMaxC / 32], fv[kMaxC / 32], dot = 0.f;
 #pragma unroll
@@ -241,12 +243,6 @@ scatter_sectors_body(const float* __restrict__ dF, int ldF, const float* __restr
   }
 }
 
-__global__ void __launch_bounds__(256)
-k_scatter_sectors(const float* __restrict__ dF, int ldF, const float* __restrict__ anc_f32,
-                  const float* __restrict__ inv_norm, const int* __restrict__ slot, int n_octets, int C,
-                  int plane, float* __restrict__ dfeat, int block_base) {
-  scatter_sectors_body(dF, ldF, anc_f32, inv_norm, slot, n_octets, C, plane, dfeat, block_base);
-}
 __global__ void __launch_bounds__(256)
 k_scatter_sectors_pull(const __grid_constant__ PullRows pull, int ldF, const float* __restrict__ anc_f32,
                        const float* __restrict__ inv_norm, const int* __restrict__ slot, int n_octets, int C,
@@ -383,6 +379,29 @@ __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant
   }
 }
 
+// Projector-tail path, channels-last: raw row copies in both directions (warp per sorted row, rows below the count)
+//   gather: rows[row][:] = feat[pix[row]][:]  (fp32 rows)      store: dfeat[pix[row]][:] = rows[row][:]  (map's type)
+template <typename T, bool GATHER>
+__global__ void __launch_bounds__(256) k_rows_raw_nhwc(const __grid_constant__ RowsBatch g) {
+  int s = 0;
+  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int lane = threadIdx.x & 31;
+  const int row = ((int)blockIdx.x - g.block0[s]) * 8 + (threadIdx.x >> 5);
+  if (row >= g.rows[s] || (g.n_rows_dev[s] && row >= *g.n_rows_dev[s])) return;
+  const int gp = g.pix[s][row];
+  if (gp < 0) return;
+  const int C = g.C[s];
+  if (GATHER) {
+    const T* src = static_cast<const T*>(g.feat[s]) + (size_t)gp * C;
+    float* dst = g.f32[s] + (size_t)row * C;
+    for (int c = lane; c < C; c += 32) dst[c] = to_f32(__ldg(src + c));
+  } else {
+    const float* src = g.dF[s] + (size_t)row * g.ldF[s];
+    T* dst = static_cast<T*>(g.dfeat[s]) + (size_t)gp * C;
+    for (int c = lane; c < C; c += 32) dst[c] = from_f32<T>(src[c]);
+  }
+}
+
 // One-pass dense writer: a thread OWNS 4 consecutive pixels and walks the channel planes.
 // Its four slot entries are fetched once (one coalesced int4), so the sampled / not-sampled decision is loop
 // invariant: 97 % of the threads run a pure store loop, the others add up to four independent (predicated) loads of
@@ -446,31 +465,6 @@ extern "C" int mscs_gather_normalize_sectors(const float* feat, int n, int C, in
   return 0;
 }
 
-// Projector-tail path (SURVEY.md 8f item 1): the sampled pixels' c_in-vectors as they are (no normalisation), rows in
-// sorted-anchor order, and the matching scatter of row gradients into the pre-zeroed dense (n, c_in, h, w) gradient.
-extern "C" int mscs_gather_rows_raw(const float* feat, int n, int C, int plane, const int32_t* slot, float* rows,
-                                    void* stream_) {
-  MSCS_CHECK_ARG(feat && slot && rows, "null pointer argument");
-  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC, "C=%d unsupported (1..%d)", C, kMaxC);
-  MSCS_CHECK_ARG(n >= 1 && plane >= 8 && plane % 8 == 0, "bad sizes (plane must be a multiple of 8)");
-  const int n_oct = n * (plane / 8);
-  k_gather_sectors<<<ceil_div(n_oct, 8), 256, 0, (cudaStream_t)stream_>>>(feat, C, (C + 63) / 64 * 64, plane, slot, n_oct,
-                                                                          nullptr, rows, nullptr, nullptr);
-  MSCS_LAUNCH_CHECK();
-  return 0;
-}
-extern "C" int mscs_scatter_rows_raw(const float* drows, int ld, const int32_t* slot, int n, int C, int plane,
-                                     float* dfeat, void* stream_) {
-  MSCS_CHECK_ARG(drows && slot && dfeat, "null pointer argument");
-  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC && ld >= C, "C=%d / ld=%d unsupported", C, ld);
-  MSCS_CHECK_ARG(plane % 8 == 0, "plane %d is not a multiple of 8 pixels", plane);
-  const int n_oct = n * (plane / 8);
-  k_scatter_sectors<<<ceil_div(n_oct, 8), 256, 0, (cudaStream_t)stream_>>>(drows, ld, nullptr, nullptr, slot, n_oct, C,
-                                                                           plane, dfeat, 0);
-  MSCS_LAUNCH_CHECK();
-  return 0;
-}
-
 extern "C" int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream_) {
   MSCS_CHECK_ARG(pix && slot && N >= 1 && n_pixels >= 1, "bad arguments");
   cudaStream_t st = (cudaStream_t)stream_;
@@ -513,7 +507,7 @@ static int check_dtype(int s, int dtype, const void* p, int align, const char* w
 
 // the items of one element type, one launch
 template <typename T>
-static int gather_sectors_launch(const mscs_gather_item* items, int count, int dtype, cudaStream_t st) {
+static int gather_sectors_launch(const mscs_gather_item* items, int count, int dtype, cudaStream_t st, bool raw = false) {
   GatherBatch g{};
   int blocks = 0;
   for (int s = 0; s < count; ++s) {
@@ -527,10 +521,11 @@ static int gather_sectors_launch(const mscs_gather_item* items, int count, int d
   if (g.count == 0) return 0;
   for (int j = 0; j < g.count; ++j) {
     g.block0[j] = blocks;
-    blocks += ceil_div(g.n_oct[j], 8) + 1;      // + the block that zeroes the padding rows
+    blocks += ceil_div(g.n_oct[j], 8) + (raw ? 0 : 1);      // + the block that zeroes the padding rows
   }
   g.block0[g.count] = blocks;
-  k_gather_sectors_batch<T><<<blocks, 256, 0, st>>>(g);
+  if (raw) k_gather_raw_batch<T><<<blocks, 256, 0, st>>>(g);
+  else k_gather_sectors_batch<T><<<blocks, 256, 0, st>>>(g);
   MSCS_LAUNCH_CHECK();
   return 0;
 }
@@ -550,6 +545,22 @@ extern "C" int mscs_gather_normalize_sectors_batch(const mscs_gather_item* items
   if (int rc = gather_sectors_launch<float>(items, count, MSCS_DTYPE_F32, st)) return rc;
   if (int rc = gather_sectors_launch<__nv_bfloat16>(items, count, MSCS_DTYPE_BF16, st)) return rc;
   return gather_sectors_launch<__half>(items, count, MSCS_DTYPE_F16, st);
+}
+
+// Projector-tail path: the raw rows of every scale, one launch per element type (see mscs.h)
+extern "C" int mscs_gather_raw_batch(const mscs_gather_item* items, int count, void* stream_) {
+  MSCS_CHECK_ARG(items && count >= 1 && count <= MSCS_MAX_SCALES, "bad item count %d", count);
+  for (int s = 0; s < count; ++s) {
+    const mscs_gather_item& it = items[s];
+    MSCS_CHECK_ARG(it.feat && it.slot && it.anc_f32, "item %d: null pointer argument", s);
+    MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC, "item %d: C=%d unsupported (1..%d)", s, it.C, kMaxC);
+    MSCS_CHECK_ARG(it.n >= 1 && it.plane >= 8 && it.plane % 8 == 0, "item %d: plane must be a multiple of 8", s);
+    if (int rc = check_dtype(s, it.dtype, it.feat, 1, "feat")) return rc;
+  }
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (int rc = gather_sectors_launch<float>(items, count, MSCS_DTYPE_F32, st, true)) return rc;
+  if (int rc = gather_sectors_launch<__nv_bfloat16>(items, count, MSCS_DTYPE_BF16, st, true)) return rc;
+  return gather_sectors_launch<__half>(items, count, MSCS_DTYPE_F16, st, true);
 }
 
 struct ScatterBatch {
@@ -636,78 +647,103 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
   MSCS_CHECK_ARG(items && rows && count >= 1 && count <= MSCS_MAX_SCALES, "bad arguments");
   DenseBatch g{};
   g.count = count;
-  int rb = 0;
+  int rb = 0, n_raw = 0;
   for (int s = 0; s < count; ++s) {
     const mscs_scatter_item& it = items[s];
-    MSCS_CHECK_ARG(it.dF && it.anc_f32 && it.inv_norm && it.slot && it.dfeat, "item %d: null pointer argument", s);
+    MSCS_CHECK_ARG(it.dF && it.slot && it.dfeat, "item %d: null pointer argument", s);
+    MSCS_CHECK_ARG((it.anc_f32 == nullptr) == (it.inv_norm == nullptr),
+                   "item %d: anc_f32 and inv_norm must both be set or both be NULL (raw rows)", s);
+    const bool raw = it.anc_f32 == nullptr;
+    n_raw += raw;
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC && it.ldF >= it.C, "item %d: C=%d / ldF=%d unsupported", s, it.C, it.ldF);
     MSCS_CHECK_ARG(it.plane % 4 == 0 && rows[s] >= 0, "item %d: plane %d is not a multiple of 4 pixels", s, it.plane);
     if (int rc = check_dtype(s, it.dtype, it.dfeat, 16, "dfeat")) return rc;
     MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32 || it.plane % 8 == 0,
                    "item %d: half gradients need a plane that is a multiple of 8 pixels (plane %d)", s, it.plane);
     g.dF[s] = const_cast<float*>(it.dF); g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot;
-    g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = rows[s];
+    g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = raw ? 0 : rows[s];
     g.n_rows_dev[s] = it.n_rows_dev;
     MSCS_CHECK_ARG((long long)it.n * it.C * it.plane < (1ll << 32), "item %d: more than 2^32 gradient elements", s);
-    g.rowblk0[s] = rb; rb += ceil_div(rows[s], 8);
+    g.rowblk0[s] = rb; rb += ceil_div(g.rows[s], 8);      // raw rows are written as they are: no blocks
   }
   g.rowblk0[count] = rb;
   cudaStream_t st = (cudaStream_t)stream_;
-  k_dx_rows<<<rb > 0 ? rb : 1, 256, 0, st>>>(g);
-  MSCS_LAUNCH_CHECK();
+  if (n_raw < count) {
+    k_dx_rows<<<rb > 0 ? rb : 1, 256, 0, st>>>(g);
+    MSCS_LAUNCH_CHECK();
+  }
   if (int rc = dense_stream_launch<float>(g, items, MSCS_DTYPE_F32, st)) return rc;
   if (int rc = dense_stream_launch<__nv_bfloat16>(g, items, MSCS_DTYPE_BF16, st)) return rc;
   return dense_stream_launch<__half>(g, items, MSCS_DTYPE_F16, st);
 }
 
 // ---- channels-last (NHWC) row gather / scatter, every scale of one element type in one launch (see mscs.h) ----
-static int rows_check(const mscs_rows_item* items, int count, bool gather) {
+enum RowsKind { kRowsGather, kRowsScatter, kRowsGatherRaw };
+
+static int rows_check(const mscs_rows_item* items, int count, RowsKind kind) {
   MSCS_CHECK_ARG(items && count >= 1 && count <= MSCS_MAX_SCALES, "bad item count %d", count);
+  const bool gather = kind != kRowsScatter;
   for (int s = 0; s < count; ++s) {
     const mscs_rows_item& it = items[s];
-    MSCS_CHECK_ARG(it.pix && it.anc_f32 && it.inv_norm, "item %d: null pointer argument", s);
+    if (kind == kRowsScatter) {     // anc_f32 and inv_norm both NULL: the rows dF are stored as they are
+      MSCS_CHECK_ARG(it.pix, "item %d: null pointer argument", s);
+      MSCS_CHECK_ARG((it.anc_f32 == nullptr) == (it.inv_norm == nullptr),
+                     "item %d: anc_f32 and inv_norm must both be set or both be NULL (raw rows)", s);
+    } else {
+      MSCS_CHECK_ARG(it.pix && it.anc_f32 && (kind == kRowsGatherRaw || it.inv_norm), "item %d: null pointer argument", s);
+    }
     MSCS_CHECK_ARG(it.C >= 1 && it.C <= kMaxC && it.rows >= 0, "item %d: C=%d unsupported (1..%d)", s, it.C, kMaxC);
-    if (gather) MSCS_CHECK_ARG(it.feat && it.anc_bf16, "item %d: null pointer argument", s);
+    if (gather) MSCS_CHECK_ARG(it.feat && (kind == kRowsGatherRaw || it.anc_bf16), "item %d: null pointer argument", s);
     else MSCS_CHECK_ARG(it.dF && it.dfeat && it.ldF >= it.C, "item %d: bad gradient arguments", s);
     if (int rc = check_dtype(s, it.dtype, gather ? it.feat : it.dfeat, 1, gather ? "feat" : "dfeat")) return rc;
   }
   return 0;
 }
 
+// raw: the items without a normalisation (raw gather; scatter items with anc_f32 == NULL)
 template <typename T>
-static int rows_launch(const mscs_rows_item* items, int count, bool gather, int dtype, cudaStream_t st) {
+static int rows_launch(const mscs_rows_item* items, int count, RowsKind kind, bool raw, int dtype, cudaStream_t st) {
   RowsBatch g{};
   int blocks = 0;
   for (int s = 0; s < count; ++s) {
     const mscs_rows_item& it = items[s];
-    if (it.dtype != dtype) continue;
+    if (it.dtype != dtype || (kind == kRowsScatter && (it.anc_f32 == nullptr) != raw)) continue;
     const int j = g.count++;
     g.feat[j] = it.feat; g.pix[j] = it.pix; g.n_rows_dev[j] = it.n_rows_dev;
     g.bf16[j] = (__nv_bfloat16*)it.anc_bf16; g.f32[j] = it.anc_f32; g.inv[j] = it.inv_norm;
     g.dF[j] = it.dF; g.dfeat[j] = it.dfeat; g.C[j] = it.C; g.ldF[j] = it.ldF; g.rows[j] = it.rows;
     g.block0[j] = blocks;
-    blocks += ceil_div(gather ? (it.rows + 255) / 256 * 256 : it.rows, 8);
+    blocks += ceil_div(kind == kRowsGather ? (it.rows + 255) / 256 * 256 : it.rows, 8);
   }
   g.block0[g.count] = blocks;
   if (blocks == 0) return 0;
-  if (gather) k_gather_rows_nhwc<T><<<blocks, 256, 0, st>>>(g);
+  if (kind == kRowsGather) k_gather_rows_nhwc<T><<<blocks, 256, 0, st>>>(g);
+  else if (kind == kRowsGatherRaw) k_rows_raw_nhwc<T, true><<<blocks, 256, 0, st>>>(g);
+  else if (raw) k_rows_raw_nhwc<T, false><<<blocks, 256, 0, st>>>(g);
   else k_scatter_rows_nhwc<T><<<blocks, 256, 0, st>>>(g);
   MSCS_LAUNCH_CHECK();
   return 0;
 }
 
-static int rows_batch(const mscs_rows_item* items, int count, bool gather, void* stream_) {
-  if (int rc = rows_check(items, count, gather)) return rc;
+static int rows_batch(const mscs_rows_item* items, int count, RowsKind kind, bool raw, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
-  if (int rc = rows_launch<float>(items, count, gather, MSCS_DTYPE_F32, st)) return rc;
-  if (int rc = rows_launch<__nv_bfloat16>(items, count, gather, MSCS_DTYPE_BF16, st)) return rc;
-  return rows_launch<__half>(items, count, gather, MSCS_DTYPE_F16, st);
+  if (int rc = rows_launch<float>(items, count, kind, raw, MSCS_DTYPE_F32, st)) return rc;
+  if (int rc = rows_launch<__nv_bfloat16>(items, count, kind, raw, MSCS_DTYPE_BF16, st)) return rc;
+  return rows_launch<__half>(items, count, kind, raw, MSCS_DTYPE_F16, st);
 }
 
 extern "C" int mscs_gather_rows_nhwc_batch(const mscs_rows_item* items, int count, void* stream_) {
-  return rows_batch(items, count, true, stream_);
+  if (int rc = rows_check(items, count, kRowsGather)) return rc;
+  return rows_batch(items, count, kRowsGather, false, stream_);
+}
+
+extern "C" int mscs_gather_raw_rows_batch(const mscs_rows_item* items, int count, void* stream_) {
+  if (int rc = rows_check(items, count, kRowsGatherRaw)) return rc;
+  return rows_batch(items, count, kRowsGatherRaw, true, stream_);
 }
 
 extern "C" int mscs_scatter_rows_nhwc_batch(const mscs_rows_item* items, int count, void* stream_) {
-  return rows_batch(items, count, false, stream_);
+  if (int rc = rows_check(items, count, kRowsScatter)) return rc;
+  if (int rc = rows_batch(items, count, kRowsScatter, false, stream_)) return rc;
+  return rows_batch(items, count, kRowsScatter, true, stream_);
 }

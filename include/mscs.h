@@ -388,14 +388,20 @@ int mscs_ce_backward(const void* logits, const int16_t* lab16, int n, int K, int
 /* ---------------------------------------------------------------------------------------
  * Projector tail on the sampled rows only (SURVEY.md 8f item 1; models/Projector.py:49-72: the projector ends in
  * nn.Conv2d(c_prev, d, kernel_size=1), evaluated densely by the reference although the loss reads <= 10k pixels per
- * scale).  The 1x1 convolution of the sampled pixels is a plain (N x c_in) x (c_in x d) GEMM on the host side's
- * library of choice; these two calls move the rows.  plane % 8 == 0; slot = pixel -> sorted row map of K1.
- *   mscs_gather_rows_raw   rows[slot[b*plane+p]][:] = feat[b, :, p]           (no normalisation)
- *   mscs_scatter_rows_raw  dfeat[b, :, p] = drows[slot[b*plane+p]][:]          into a PRE-ZEROED dense gradient
+ * scale).  The 1x1 convolution of the sampled pixels is a plain (N x c_prev) x (c_prev x d) GEMM on the host side's
+ * library of choice; these calls move the rows, every scale in one launch per element type of the maps.  The rows are
+ * fp32 (N x C, row stride C) and not normalised: a half map gives the same rows as its exact fp32 widening.
+ *   mscs_gather_raw_batch       NCHW: rows[slot[b*plane+p]][:] = feat[b, :, p], in the address order of the slot map
+ *                               (mscs_gather_item: `anc_f32` receives the rows; anc_bf16, inv_norm and n_rows_dev are
+ *                               not used -- the slot map holds the sampled rows only; plane % 8 == 0)
+ *   mscs_gather_raw_rows_batch  channels-last: rows[r][:] = feat[pix[r]][:] for r below the count (mscs_rows_item:
+ *                               `anc_f32` receives the rows, `rows` / `n_rows_dev` as for mscs_gather_rows_nhwc_batch)
+ * The way back is the dense writers above: an item of mscs_scatter_dense_batch or mscs_scatter_rows_nhwc_batch whose
+ * anc_f32 and inv_norm are both NULL stores its rows dF as they are (no normalisation backward); exactly one of the two
+ * being NULL is rejected.
  * ------------------------------------------------------------------------------------- */
-int mscs_gather_rows_raw(const float* feat, int n, int C, int plane, const int32_t* slot, float* rows, void* stream);
-int mscs_scatter_rows_raw(const float* drows, int ld, const int32_t* slot, int n, int C, int plane, float* dfeat,
-                          void* stream);
+int mscs_gather_raw_batch(const mscs_gather_item* items, int count, void* stream);
+int mscs_gather_raw_rows_batch(const mscs_rows_item* items, int count, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * Pooled cross-batch mode -- the exchange between the GPUs of one box over NVLink peer memory.  (Not a reference
