@@ -9,6 +9,7 @@ import ctypes as C
 import os
 import struct
 import threading
+import time
 from dataclasses import dataclass, field
 from typing import List
 
@@ -41,7 +42,6 @@ def _seg(name, t0):
     """Adds the host time since t0 to segment `name`; returns the new time stamp (no-op when disabled)."""
     if HOST_SEG is None:
         return t0
-    import time
     t1 = time.perf_counter()
     HOST_SEG[name] = HOST_SEG.get(name, 0.0) + (t1 - t0)
     return t1
@@ -117,6 +117,12 @@ class ScaleSample:
 
     def ptr(self, k):
         return self._slab.data_ptr() + 4 * self._off[k]
+
+
+def _samples_from_plan(plan, islab, ioff, A):
+    """The ScaleSample of every scale from the host copy of the plan records; `ioff[s]`: offsets of the scale's five
+    index arrays in the int32 slab `islab`."""
+    return [ScaleSample(p.T, p.V, p.N, bool(p.log_flag), p.dl_h, p.dl_w, islab, off, A) for p, off in zip(plan, ioff)]
 
 
 _stream_override = [None, None]
@@ -405,8 +411,7 @@ def sample_anchors(labels, feat_hw, spec, mt_state=None, defer_rng=False):
             off += (x + 15) // 16 * 16
         offs.append(cur)
     slab = torch.empty(off, dtype=torch.int32, device=dev)
-    out = [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w,
-                       slab, offs[s], A) for s in range(S)]
+    out = _samples_from_plan(plan, slab, offs, A)
     arrs = [[out[s].ptr(k) for s in range(S)] for k in range(5)]
     _lib.check(lib.mscs_sample_select(C.byref(cfg), plan, ws.data_ptr(), draws.data_ptr(),
                                       *[_lib.ptr_array(a) for a in arrs], None, st), "mscs_sample_select")
@@ -460,10 +465,10 @@ class SimState:
     cs_logged: List[int]            # indices (into term_loss) of the cs terms that go to cs_losses
 
 
-def build_job(spec, samples, sets, single_scale):
-    """Terms of one call: one single-scale term per scale (V2.py:55 via _ms.py:53-59) and, when
+def _terms(spec, S, single_scale):
+    """Terms of one call, as (anchor set, key set, self term, weight, tau, key-side pass), and the indices of the
+    cross-scale terms that are logged: one single-scale term per scale (V2.py:55 via _ms.py:53-59) and, when
     cross_scale_contrast, scale 0 against the deepest and second-deepest scales (_ms.py:62-80)."""
-    S = len(sets)
     terms = [(s, s, True, spec.weights[s], spec.temperature, False) for s in range(S)]
     cs_logged = []
     if spec.cross_scale and not single_scale:
@@ -477,6 +482,13 @@ def build_job(spec, samples, sets, single_scale):
             cs_logged.append(len(terms) - 1)
     if len(terms) > _lib.MAX_TERMS:
         raise ValueError(f"{len(terms)} loss terms exceed the supported {_lib.MAX_TERMS}")
+    return terms, cs_logged
+
+
+def build_job(spec, samples, sets, single_scale):
+    """The similarity job of one call over the given anchor sets (terms: _terms)."""
+    S = len(sets)
+    terms, cs_logged = _terms(spec, S, single_scale)
     dev = sets[0].bf16.device
     n_rows = [sets[a].N for a, *_ in terms]
     stats = torch.zeros(3 * sum(n_rows), dtype=torch.float32, device=dev)
@@ -759,20 +771,7 @@ class _StepPlan:
             self.boff.append(off)
             off += al(self.Ncap[s], 256) * self.C_pad
         self.bslab_n = off
-        # terms (V2.py:55 via _ms.py:53-59; cross-scale _ms.py:62-80)
-        terms = [(s, s, True, spec.weights[s], spec.temperature, False) for s in range(S)]
-        self.cs_logged = []
-        if spec.cross_scale and not single_scale:
-            assert S > 1, "cross_scale_contrast needs at least two scales (_ms.py:63-64)"
-            need_dk = not spec.detach_deepest
-            terms.append((0, S - 1, False, spec.w_high_low, spec.cs_temperature, need_dk))
-            if not spec.detach_deepest:
-                self.cs_logged.append(len(terms) - 1)
-            if S > 2:
-                terms.append((0, S - 2, False, spec.w_high_mid, spec.cs_temperature, need_dk))
-                self.cs_logged.append(len(terms) - 1)
-        if len(terms) > _lib.MAX_TERMS:
-            raise ValueError(f"{len(terms)} loss terms exceed the supported {_lib.MAX_TERMS}")
+        terms, self.cs_logged = _terms(spec, S, single_scale)
         self.terms = terms
         self.soff, off = [], 0          # stats: neg, pos, S per term (zero-initialised)
         for a, *_ in terms:
@@ -839,9 +838,9 @@ def _step_plan(dev, label_shape, feat_shapes, spec, single_scale, world=1, rank=
 
 
 def fast_path_ok(spec, world):
-    """Single process and selection shared memory within limits: the device-driven order can be used."""
-    v_cap = min(spec.max_total, 16384) if spec.max_views == 1 else min(spec.max_views, spec.max_total, 16384)
-    return world == 1 and v_cap * 12 <= 200 * 1024
+    """Whether the device-driven order can be used: in a single process.  Its selection table always fits (at most 16384
+    views per pair, 192 KB; mscs_sample_select_async rejects more itself); `spec` is kept for the callers."""
+    return world == 1
 
 
 def half_io_ok(sp, world):
@@ -849,9 +848,7 @@ def half_io_ok(sp, world):
     written in the maps' dtype): the single-process fast path with the channels-last row gather, or with the NCHW octet
     gather and the one-pass dense writer.  Every other route -- pooled mode, planes that are not a multiple of 8
     pixels -- converts the maps to fp32 first and the gradients back afterwards."""
-    if not fast_path_ok(sp.spec, world):
-        return False
-    return sp.nhwc or all(sp.slot_sizes)
+    return fast_path_ok(sp.spec, world) and (sp.nhwc or all(sp.slot_sizes))
 
 
 def channels_last_ok(spec, world, feats):
@@ -885,8 +882,6 @@ def graph_mode(spec, world, single_scale, labels, feats, counter, plan_of=None):
                "use sampler='philox'")
     if single_scale and spec.cross_scale:
         refuse("DenseContrastiveLossV2 with cross_scale_contrast=True returns sampled features of a data-dependent shape")
-    if not fast_path_ok(spec, world):
-        refuse("the selection table of this configuration exceeds the device-driven path's shared memory")
     if any(f.device != feats[0].device for f in feats) or labels.device != feats[0].device:
         refuse("labels and feature maps must already be on the GPU")
     nhwc = channels_last_ok(spec, world, feats)
@@ -967,9 +962,7 @@ def fetch_graph_plan(state):
 def graph_samples(state, plan):
     """The ScaleSample list of a captured call's latest replay (views of the graph's workspace: the next replay
     overwrites them)."""
-    sp, e = state.sp, state.entry
-    return [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w, e.islab,
-                        sp.ioff[s], sp.A) for s in range(sp.S)]
+    return _samples_from_plan(plan, state.entry.islab, state.sp.ioff, state.sp.A)
 
 
 def _fill_job(job, sp, A, bbase, ibase, sbase, cbase, work_ptr):
@@ -1082,10 +1075,19 @@ class _Workspace:
         ch.gather_items, ch.job = C.addressof(self.gitems), C.addressof(self.job_fwd)
 
 
-class _StepState:
-    """Buffers of one call (kept alive for the backward)."""
-    entry = None
-    io_dtypes = None        # dtypes of the maps the kernels read and of the gradients they write (None: all fp32)
+class _DeviceState:
+    """A call in the device-driven order (the projector tail's; the loss classes extend it: _FastState).  It owns the
+    workspace taken from the step plan's pool and gives it back when it dies; a captured call's workspace belongs to its
+    graph.  ``samples``: set by _after_wait (None for a captured call).  ``dF_fresh``: the workspace's gradient rows
+    were cleared by this forward and no backward has used them yet."""
+
+    def __init__(self, sp, e, graph, out, gradbufs, dF_fresh):
+        self.sp, self.entry = sp, e        # first: from here on an exception returns the workspace to the pool
+        self.graph, self.gradbufs, self.dF_fresh = graph, gradbufs, dF_fresh
+        self.samples = None
+        self.job, self.stats, self.fslab = e.job_bwd, e.stats, e.fslab
+        self.scalars, self.term_loss = out, out[:len(sp.terms)]      # [term losses..., total, inf/NaN flag]
+        self.num_ms, self.cs_logged = sp.S, sp.cs_logged
 
     def __del__(self):
         e, self.entry = self.entry, None
@@ -1093,14 +1095,48 @@ class _StepState:
             self.sp.ws_pool.append(e)
 
 
+class _FastState(_DeviceState):
+    """A device-driven call of the loss classes: also the 0-d loss, the dtypes the kernels read and write the maps in,
+    and the dense-gradient slab the forward prepared for the NCHW backward."""
+
+    def __init__(self, sp, e, graph, out, gradbufs, dF_fresh, total, io_dtypes, grad_slab, grad_outs):
+        super().__init__(sp, e, graph, out, gradbufs, dF_fresh)
+        self.total, self.io_dtypes = total, io_dtypes
+        self.grad_slab, self.grad_outs = grad_slab, grad_outs
+        self.backward = _backward_rows if sp.nhwc else _backward_nchw
+
+
+class _HostState:
+    """A call in the host-driven order; ``keep``: the buffers the job and the samples point into."""
+
+    def __init__(self, sp, job, samples, gradbufs, slots, keep, stats, fslab, scalars, total):
+        self.sp, self.job, self.samples, self.gradbufs, self.slots = sp, job, samples, gradbufs, slots
+        self.keep, self.stats, self.fslab, self.total = keep, stats, fslab, total
+        self.scalars, self.term_loss = scalars, scalars[:len(sp.terms)]      # [term losses..., total, inf/NaN flag]
+        self.num_ms, self.cs_logged = sp.S, sp.cs_logged
+        self.backward = _backward_host
+
+
+class _PooledState(_HostState):
+    """A call of the pooled mode: also the exchange slab and the parity this step used.  ``dF_fresh``: as in
+    _DeviceState, for this parity's gradient rows in the exchange slab."""
+
+    def __init__(self, sp, job, samples, gradbufs, slots, keep, fslab, scalars, total, comm, xs, par, exchange_info):
+        super().__init__(sp, job, samples, gradbufs, slots, keep, None, fslab, scalars, total)
+        self.comm, self.xs, self.par, self.exchange_info = comm, xs, par, exchange_info
+        self.dF_fresh = gradbufs is not None
+        self.backward = _run_backward_pooled
+
+
 def run_forward(sp, labels, feats32, needs, comm=None, philox=None, graph=False):
     """philox: None (reference stream: torch CPU generator) or (seed, call index) of the opt-in counter-based stream.
     feats32: fp32 maps, or bf16 / fp16 ones where half_io_ok(sp, world) holds (fast path only).
-    graph: the call is captured into a CUDA graph (see graph_mode); philox is then (seed, int64 device call index)."""
+    graph: the call is captured into a CUDA graph (see graph_mode); philox is then (seed, int64 device call index).
+    The state returned knows the backward of the order that ran (run_backward)."""
     pooled = comm is not None and comm.world > 1
     # device-driven order (selection, gather and similarity forward enqueued before the host sees the plan): single
-    # process, every plane a multiple of 8 pixels (slot maps), selection shared memory within limits
-    if fast_path_ok(sp.spec, 1 if not pooled else comm.world) and (sp.nhwc or all(x != 0 for x in sp.slot_sizes)):
+    # process, every plane a multiple of 8 pixels (slot maps) or channels-last maps
+    if not pooled and (sp.nhwc or all(sp.slot_sizes)):
         return _run_forward_fast(sp, labels, feats32, needs, philox, graph)
     assert all(f.dtype == torch.float32 for f in feats32), "half maps are converted by the caller off the fast path"
     assert not sp.nhwc, "channels-last inputs are converted by the caller unless the fast path applies"
@@ -1125,6 +1161,64 @@ def _finish_rng(sp, dev, mt, pos, total, defer=False):
     _stream_cache(dev).release_and_prefetch(mt2, pos2, sp.max_draws + _MT_N, defer)
 
 
+# ---- the device-driven order: the parts the loss classes and the projector tail (projector.py) share --------------
+def _take_workspace(sp, graph, make, *args):
+    """The workspace of a device-driven call (under capture a fresh ``make(sp, *args, graph=True)`` that its graph
+    keeps, else one from the pool) and this call's scalars, entered into both similarity jobs: ``out`` = [term
+    losses..., total, inf/NaN flag] and the 0-d loss ``total_t``.  The loss has storage of its own: the reference's
+    LossWrapper multiplies it IN PLACE (``loss *= weight``, LossWrapper.py:90), which autograd forbids on a view created
+    inside a custom Function, and which must not change the logged (unweighted) scalars."""
+    cur = _cur_stream()
+    e = make(sp, *args, graph=True) if graph else (sp.ws_pool.pop() if sp.ws_pool else make(sp, *args))
+    if e.last_stream is not None and e.last_stream != cur:
+        cur.wait_stream(e.last_stream)          # reuse on another stream: order after its previous user
+    e.last_stream = cur
+    nt = len(sp.terms)
+    out = torch.empty(nt + 2, dtype=torch.float32, device=sp.dev)
+    total_t = torch.empty((), dtype=torch.float32, device=sp.dev)
+    for job in (e.job_fwd, e.job_bwd):
+        job.term_loss, job.total_loss = out.data_ptr(), out.data_ptr() + 4 * nt
+        job.total_out = total_t.data_ptr()
+    return e, out, total_t
+
+
+def _call_draws(sp, e, philox, graph, st_s):
+    """This call's random stream: (device address, event the sampling stream must wait for or None, the (mt, pos) of
+    the torch CPU generator or None).  MT19937: normally produced ahead of time during the previous step.  Philox: one
+    small kernel on `st_s`, which the caller has ordered after its stream; under capture the call index is read from
+    device memory and incremented behind the generator, so that every replay draws anew."""
+    if philox is None:
+        mt, pos = torch_mt_state()
+        cache = _stream_cache(sp.dev)
+        return cache.acquire_nowait(mt, pos, sp.max_draws + _MT_N).data_ptr(), cache.ready, (mt, pos)
+    if e.philox is None:
+        e.philox = torch.empty((sp.max_draws + 3) // 4 * 4 + 4, dtype=torch.int32, device=sp.dev)
+    lib, seed, draws = _lib.load(), int(philox[0]) & (2 ** 64 - 1), e.philox.data_ptr()
+    if graph:
+        _lib.check(lib.mscs_philox_stream_dev(seed, philox[1].data_ptr(), sp.max_draws, draws, st_s),
+                   "mscs_philox_stream_dev")
+    else:
+        _lib.check(lib.mscs_philox_stream(seed, int(philox[1]), sp.max_draws, draws, st_s), "mscs_philox_stream")
+    return draws, None, None
+
+
+def _after_wait(state, rng, defer, t0):
+    """Host work of an eager device-driven forward after its wait: the reference's errors (the state owns the workspace,
+    so an error returns it to the pool), the samples, the backward job's row counts, and the generator bookkeeping of
+    the reference sampler (`rng`: the (mt, pos) drawn from; `defer`: see _finish_rng).  t0: time of the wait's end."""
+    sp, e = state.sp, state.entry
+    plan = e.plan
+    _raise_plan_errors(plan, sp.S, sp.spec)
+    state.samples = samples = _samples_from_plan(plan, e.islab, sp.ioff, sp.A)
+    for i, (a, k, *_rest) in enumerate(sp.terms):
+        t = e.job_bwd.terms[i]
+        t.N1, t.N2 = samples[a].N, samples[k].N
+    t0 = _seg("fwd: after wait", t0)
+    if rng is not None:
+        _finish_rng(sp, sp.dev, *rng, sum(int(p.draws) for p in plan), defer)
+    _seg("fwd: rng advance + prefetch", t0)
+
+
 def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
     """Single process.  Selection, gather AND the similarity forward are driven by the DEVICE plan records and enqueued
     before the host looks at the plan: the one host wait of the forward pass (needed to raise the reference's errors
@@ -1134,48 +1228,19 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
     carry the upper bounds and the device-resident row counts; errors, sampling results and the logging flag stay in
     the device plan records (read by the caller after a replay: fetch_graph_plan)."""
     lib = _lib.load()
-    dev, S, A, spec = sp.dev, sp.S, sp.A, sp.spec
+    dev, S = sp.dev, sp.S
     st, cur = _stream(), _cur_stream()
-    import time
     _t = time.perf_counter() if HOST_SEG is not None else 0.0
-    if graph:
-        e = _Workspace(sp, graph=True)
-    else:
-        e = sp.ws_pool.pop() if sp.ws_pool else _Workspace(sp)
-    if e.last_stream is not None and e.last_stream != cur:
-        cur.wait_stream(e.last_stream)          # reuse on another stream: order after its previous user
-    e.last_stream = cur
-    nt = len(sp.terms)
-    out = torch.empty(nt + 2, dtype=torch.float32, device=dev)      # term losses, total, inf/NaN flag
-    # the 0-d loss handed to the caller: a tensor of its own (not a view of `out`) -- the reference's LossWrapper
-    # multiplies it IN PLACE (`loss *= weight`, LossWrapper.py:90), which autograd forbids on a view created inside
-    # a custom Function, and which must not change the logged (unweighted) scalars
-    total_t = torch.empty((), dtype=torch.float32, device=dev)
-    for job in (e.job_fwd, e.job_bwd):
-        job.term_loss, job.total_loss = out.data_ptr(), out.data_ptr() + 4 * nt
-        job.total_out = total_t.data_ptr()
+    e, out, total_t = _take_workspace(sp, graph, _Workspace)
     # the small, latency-bound sampling kernels run on a high-priority stream (see _hp_stream)
     hp = _hp_stream(dev) if _USE_HP_STREAM else None
     st_s = C.c_void_p(hp.cuda_stream) if hp is not None else st
     ch = e.chain
-    # MT19937 output stream of this call (normally produced ahead of time during the previous step): looked up
-    # first, so that nothing but kernels sits between the launches of the sampling chain
-    if philox is None:
-        mt, pos = torch_mt_state()
-        ch.draws = _stream_cache(dev).acquire_nowait(mt, pos, sp.max_draws + _MT_N).data_ptr()
-        ch.wait_event = _stream_cache(dev).ready.cuda_event
-    else:       # counter-based stream of this call: one small kernel in front of the chain, no generator state
-        if e.philox is None:
-            e.philox = torch.empty((sp.max_draws + 3) // 4 * 4 + 4, dtype=torch.int32, device=dev)
-        if hp is not None:
-            hp.wait_stream(cur)
-        ch.draws, ch.wait_event = e.philox.data_ptr(), None
-        if graph:       # call index in device memory, incremented behind the generator: every replay draws anew
-            _lib.check(lib.mscs_philox_stream_dev(int(philox[0]) & (2 ** 64 - 1), philox[1].data_ptr(), sp.max_draws,
-                                                  ch.draws, st_s), "mscs_philox_stream_dev")
-        else:
-            _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws, ch.draws,
-                                              st_s), "mscs_philox_stream")
+    if philox is not None and hp is not None:
+        hp.wait_stream(cur)     # the Philox kernel runs in front of the chain (which then orders the sampling stream)
+    # looked up (MT19937) or launched (Philox) first, so that nothing but kernels sits between the launches of the chain
+    ch.draws, ready, rng = _call_draws(sp, e, philox, graph, st_s)
+    ch.wait_event = None if ready is None else ready.cuda_event
     _t = _seg("fwd: rng state + stream acquire", _t)
     # channels-last dense gradients + gradient rows: pre-zeroed on a side stream, sampled rows written by the backward
     # (NCHW maps need no fill: the backward writes their dense gradients in one streaming pass, see gather.cu).
@@ -1215,11 +1280,10 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
             ch.stage_events[i] = None
     if HOST_WAIT is not None:
         _t0 = time.perf_counter()
-    plan = e.plan
     # ONE call: fills, hist -> tile scan -> plan -> select on the sampling stream (programmatic dependent launches; the
     # plan records travel to the host on a private stream), gather + similarity forward on the caller's stream, all
     # driven by the DEVICE plan records, then the one host wait of the forward pass (plan records only)
-    _lib.check(lib.mscs_forward_chain(C.byref(ch), st_s, st, None if graph else plan), "mscs_forward_chain")
+    _lib.check(lib.mscs_forward_chain(C.byref(ch), st_s, st, None if graph else e.plan), "mscs_forward_chain")
     if HOST_WAIT is not None:
         HOST_WAIT.append(time.perf_counter() - _t0)
     if evs is not None:
@@ -1227,39 +1291,17 @@ def _run_forward_fast(sp, labels, feats32, needs, philox=None, graph=False):
         TIMING.setdefault("gather", []).append((evs[2], evs[3]))
         TIMING.setdefault("sim_fwd", []).append((evs[3], evs[4]))
     _t = time.perf_counter() if HOST_SEG is not None else 0.0
-    state = _StepState()
-    state.sp, state.entry = sp, e          # (from here on an exception returns the workspace to the pool)
-    state.graph = graph
-    if graph:           # nothing is known on the host: the backward structures hold the device-count form already
-        samples = None
-    else:
-        _raise_plan_errors(plan, S, spec)
-        total = sum(int(plan[s].draws) for s in range(S))
-        samples = [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w,
-                               e.islab, sp.ioff[s], A) for s in range(S)]
-        for i, (a, k, *_rest) in enumerate(sp.terms):      # the backward is launched with the actual counts
-            t = e.job_bwd.terms[i]
-            t.N1, t.N2 = samples[a].N, samples[k].N
-    _t = _seg("fwd: after wait", _t)
-    if philox is None:
-        _finish_rng(sp, dev, mt, pos, total, defer=any(needs))
-    _t = _seg("fwd: rng advance + prefetch", _t)
-    state.job, state.samples, state.gradbufs, state.slots = e.job_bwd, samples, gradbufs, e.slots
-    state.keep, state.stats, state.fslab = out, e.stats, e.fslab
-    state.term_loss, state.total, state.scalars = out[:nt], total_t, out
-    state.num_ms, state.cs_logged, state.comm = S, sp.cs_logged, None
-    state.dF_ws = e.dF_ptr if dF_in_ws else None
-    state.grad_slab, state.grad_outs = grad_slab, grad_outs
-    state.io_dtypes = [f.dtype for f in feats32]
-    if not graph:
+    state = _FastState(sp, e, graph, out, gradbufs, dF_in_ws, total_t, [f.dtype for f in feats32], grad_slab, grad_outs)
+    if not graph:       # (a captured call: the backward structures hold the device-count form already)
+        _after_wait(state, rng, any(needs), _t)
         for s in range(S):
-            e.bw_rows[s] = samples[s].N
+            e.bw_rows[s] = state.samples[s].N
     return state
 
 
 def _run_forward_general(sp, labels, feats32, needs):
-    """Host-driven order on one stream: plan, fetch (host sync), select, gather, forward.  Single process, planes that
-    are not a multiple of 8 pixels (no slot maps) or selection shared memory beyond the fast path's limit."""
+    """Host-driven order on one stream: plan, fetch (host sync), select, gather, forward.  Single process, NCHW maps
+    with a plane that is not a multiple of 8 pixels (no slot map for that scale)."""
     lib = _lib.load()
     dev, S, A, spec = sp.dev, sp.S, sp.A, sp.spec
     st = _stream()
@@ -1305,8 +1347,7 @@ def _run_forward_general(sp, labels, feats32, needs):
         total = sum(int(plan[s].draws) for s in range(S))
         _lib.check(lib.mscs_sample_select(C.byref(sp.cfg), plan, ws.data_ptr(), draws.data_ptr(), *arrs, sarr, st),
                    "mscs_sample_select")
-    samples = [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w,
-                           islab, sp.ioff[s], A) for s in range(S)]
+    samples = _samples_from_plan(plan, islab, sp.ioff, A)
     with _timed("gather"):
         for s in range(S):
             n, Cc, h, w = sp.feat_shapes[s]
@@ -1325,15 +1366,8 @@ def _run_forward_general(sp, labels, feats32, needs):
     with _timed("sim_fwd"):
         _lib.check(lib.mscs_sim_forward(C.byref(job), st), "mscs_sim_forward")
     _finish_rng(sp, dev, mt, pos, total)
-    state = _StepState()
-    state.sp, state.job, state.samples, state.gradbufs, state.slots = sp, job, samples, gradbufs, slots
-    state.keep = (ws, islab, fslab, bslab, stats, misc, work, slot_slab)
-    state.stats = stats
-    state.fslab, state.term_loss = fslab, misc[sp.out_off:sp.out_off + nt]
-    state.total = total_t
-    state.scalars = misc[sp.out_off:sp.out_off + nt + 2]      # [term losses..., total, inf/NaN flag]: one copy for the logger
-    state.num_ms, state.cs_logged, state.comm = S, sp.cs_logged, None
-    return state
+    return _HostState(sp, job, samples, gradbufs, slots, (ws, islab, fslab, bslab, stats, misc, work, slot_slab), stats,
+                      fslab, misc[sp.out_off:sp.out_off + nt + 2], total_t)
 
 
 def _run_forward_pooled(sp, labels, feats32, needs, comm):
@@ -1410,32 +1444,22 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
             jb.total_out = total_t.data_ptr()
         # Selection and the peer-store gather are driven by the DEVICE plan records and enqueued before the host looks
         # at the plan: the one host wait of the forward (errors, row ranges) overlaps them instead of idling the GPU.
-        device_driven = sp.v_cap * 12 <= 200 * 1024
         plan_sz = C.sizeof(_lib.ScalePlan)
-        if device_driven:
-            _lib.check(lib.mscs_plan_fetch_begin(plan_dev.data_ptr(), S, st), "mscs_plan_fetch_begin")
-            _lib.check(lib.mscs_sample_select_async(C.byref(sp.cfg), plan_dev.data_ptr(), sp.v_cap, ws.data_ptr(),
-                                                    draws.data_ptr(), *arrs, sarr, st), "mscs_sample_select_async")
-        else:
-            _lib.check(lib.mscs_plan_fetch(plan_dev.data_ptr(), plan, S, st), "mscs_plan_fetch")     # the host sync
-            _raise_plan_errors(plan, S, spec)
-            _lib.check(lib.mscs_sample_select(C.byref(sp.cfg), plan, ws.data_ptr(), draws.data_ptr(), *arrs, sarr, st),
-                       "mscs_sample_select")
+        _lib.check(lib.mscs_plan_fetch_begin(plan_dev.data_ptr(), S, st), "mscs_plan_fetch_begin")
+        _lib.check(lib.mscs_sample_select_async(C.byref(sp.cfg), plan_dev.data_ptr(), sp.v_cap, ws.data_ptr(),
+                                                draws.data_ptr(), *arrs, sarr, st), "mscs_sample_select_async")
     with _timed("gather"):
         for s in range(S):
             n, Cc, h, w = sp.feat_shapes[s]
             _lib.check(lib.mscs_gather_normalize_p2p(
-                feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(), 0 if device_driven else plan[s].N,
-                plan_dev.data_ptr() + s * plan_sz + 8 if device_driven else None, xs.peers, world, rank,
-                xo["b"] + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1], st),
-                "mscs_gather_normalize_p2p")
+                feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(), 0, plan_dev.data_ptr() + s * plan_sz + 8,
+                xs.peers, world, rank, xo["b"] + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1],
+                st), "mscs_gather_normalize_p2p")
         comm.barrier(xs)                                   # A: every rank's key rows have landed here
-    if device_driven:
-        _lib.check(lib.mscs_plan_fetch_end(plan, S), "mscs_plan_fetch_end")       # the host wait (plan records only)
-        _raise_plan_errors(plan, S, spec)
+    _lib.check(lib.mscs_plan_fetch_end(plan, S), "mscs_plan_fetch_end")       # the host wait (plan records only)
+    _raise_plan_errors(plan, S, spec)
     total = sum(int(plan[s].draws) for s in range(S))
-    samples = [ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h, plan[s].dl_w,
-                           islab, sp.ioff[s], A) for s in range(S)]
+    samples = _samples_from_plan(plan, islab, sp.ioff, A)
     # this parity's gradient rows: only the 128-aligned row blocks this rank computes are accumulated into (and
     # pulled from): clear those (1/world of the slab), on the main stream, long before the backward
     if any(needs):
@@ -1470,17 +1494,8 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
         _lib.check(lib.mscs_sim_finalize(C.byref(job), st), "mscs_sim_finalize")
     if comm.owns_rng:
         _finish_rng(sp, dev, mt, pos, total)
-    state = _StepState()
-    state.sp, state.job, state.samples, state.gradbufs, state.slots = sp, job, samples, gradbufs, slots
-    state.keep = (ws, islab, fslab, misc, work, slot_slab, stats_priv)
-    state.stats = None
-    state.fslab, state.term_loss = fslab, misc[sp.out_off:sp.out_off + nt]
-    state.total = total_t
-    state.scalars = misc[sp.out_off:sp.out_off + nt + 2]      # [term losses..., total, inf/NaN flag]: one copy for the logger
-    state.num_ms, state.cs_logged, state.comm = S, sp.cs_logged, comm
-    state.xs, state.par = xs, par
     n_local = sum(int(samples[s].N) for s in range(S)) / world        # rows this rank owns, on average
-    state.exchange_info = {
+    exchange_info = {
         "transport": "NVLink peer stores / loads by the library's kernels (CUDA IPC slabs) + device-side flag barriers; "
                      "NCCL only for the class histograms",
         "barriers_per_step": 3,
@@ -1488,36 +1503,32 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
         "key_rows_stored_to_peers_bytes": int(n_local * sp.C_pad * 2 * (world - 1)),
         "row_statistics_pushed_bytes": int(sum(push_len) * 4 * (world - 1)),
         "gradient_rows_pulled_bytes": int(n_local * sp.C_pad * 4 * (world - 1) / world)}
-    return state
+    return _PooledState(sp, job, samples, gradbufs, slots, (ws, islab, fslab, misc, work, slot_slab, stats_priv), fslab,
+                        misc[sp.out_off:sp.out_off + nt + 2], total_t, comm, xs, par, exchange_info)
 
 
 def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
     """Pooled mode: every rank computes the COMPLETE gradient rows of its 128-aligned row block of every anchor set
     (one launch for all passes) into its exchange slab; after the barrier the scatter pulls the row of every LOCAL
-    pixel from the rank that computed it -- an eighth of the rows travels, once, to where it is needed."""
+    pixel from the rank that computed it -- an eighth of the rows travels, once, to where it is needed.  A second
+    backward through the same graph clears the rows again and zero-fills fresh dense gradients."""
     lib = _lib.load()
     sp, comm, xs = state.sp, state.comm, state.xs
     dev, S = sp.dev, sp.S
     st = _stream()
     xo = sp.x_off[state.par]
     gb = state.gradbufs
-    first = gb is not None and gb.ready is not None and not getattr(state, "bwd_done", False)
-    if first:
-        _cur_stream().wait_event(gb.ready)          # the side-stream zero fill (dense gradients + the slab's row region)
-    else:                                           # second backward through the same graph: clear the row region again
+    if state.dF_fresh:
+        _cur_stream().wait_event(gb.ready)          # the side-stream zero fill of the dense gradients
+    else:
         _lib.check(lib.mscs_fill_bytes(_lib.ptr_array([xs.local + xo["dF"]]), (C.c_int32 * 1)(0),
                                        (C.c_size_t * 1)(4 * sp.dF_n), 1, st), "mscs_fill_bytes")
         comm.barrier(xs)                            # nobody still pulls the previous rows
-    state.bwd_done = True
-    base = xs.local + xo["dF"]
-    ptrs = [0] * _lib.MAX_SCALES
-    lds = (C.c_int32 * _lib.MAX_SCALES)()
-    for s in range(S):
-        ptrs[s], lds[s] = base + 4 * sp.dF_off[s], sp.C_pad
-    g = grad_out.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
+    state.dF_fresh = False
+    _ptrs, ptrs_arr, lds = _row_accumulators(sp, xs.local + xo["dF"])
+    g = _as_f32(grad_out, dev)
     with _timed("sim_bwd"):
-        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), _lib.ptr_array(ptrs), lds, st),
-                   "mscs_sim_backward")
+        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st), "mscs_sim_backward")
         comm.barrier(xs)                            # C: every rank's gradient rows are complete
     grads = []
     fbase = state.fslab.data_ptr()
@@ -1540,150 +1551,167 @@ def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
     return grads
 
 
-def run_backward(state, grad_out, needs, shapes, dtypes):
+def _row_accumulators(sp, base):
+    """(addresses, pointer table, leading dimensions) of the gradient rows of every scale in the fp32 region at
+    `base` (layout: sp.dF_off)."""
+    ptrs = [base + 4 * sp.dF_off[s] for s in range(sp.S)] + [0] * (_lib.MAX_SCALES - sp.S)
+    return ptrs, _lib.ptr_array(ptrs), (C.c_int32 * _lib.MAX_SCALES)(*([sp.C_pad] * sp.S))
+
+
+def _as_f32(grad_out, dev):
+    """The incoming gradient of the loss as an fp32 device tensor (only its address is passed on)."""
+    if grad_out.dtype == torch.float32 and grad_out.device == dev and grad_out.is_contiguous():
+        return grad_out
+    return grad_out.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
+
+
+def _as_dtypes(grads, dtypes):
+    """The gradients in the dtypes of the inputs (converted where the kernels wrote another one)."""
+    return [g if g is None or g.dtype == dt else g.to(dt) for g, dt in zip(grads, dtypes)]
+
+
+def _backward_nchw(state, grad_out, needs, shapes, dtypes):
+    """NCHW maps after the device-driven forward: similarity backward, normalisation backward of the rows and the
+    one-pass dense writer in ONE C call.  The first backward accumulates into the workspace's gradient rows (cleared by
+    the forward chain) with the prebuilt argument structures, and writes the dense slab the forward allocated when
+    every map wants its gradient.  A second backward through the same graph takes fresh zeroed rows and a fresh slab."""
     lib = _lib.load()
-    sp = state.sp
+    sp, e = state.sp, state.entry
     dev, S = sp.dev, sp.S
     st = _stream()
-    if state.comm is not None:
-        return _run_backward_pooled(state, grad_out, needs, shapes, dtypes)
-    # gradient-row accumulators: cleared during the forward -- inside the workspace by the sampling chain's fills
-    # (default), or together with the pre-zeroed dense gradients on the side stream; a second backward through the
-    # same graph takes a fresh zeroed buffer
-    dF, base, e = None, None, getattr(state, "entry", None)
-    first = not getattr(state, "bwd_done", False)
-    state.bwd_done = True
-    if state.gradbufs is not None:
-        dF = state.gradbufs.take_dF()
-        if dF is not None:
-            _cur_stream().wait_event(state.gradbufs.ready)
-    elif first and getattr(state, "dF_ws", None):
-        base = state.dF_ws
-    in_ws = base is not None
-    if not in_ws:
-        if dF is None:
-            dF = torch.zeros(sp.dF_n, dtype=torch.float32, device=dev)
-        base = dF.data_ptr()
-    if in_ws:
-        ptrs_arr, lds = e.bw_ptrs, e.bw_lds
-        ptrs = [base + 4 * sp.dF_off[s] for s in range(S)]
+    fresh, state.dF_fresh = state.dF_fresh, False
+    if fresh:
+        ptrs, ptrs_arr, lds = [e.dF_ptr + 4 * sp.dF_off[s] for s in range(S)], e.bw_ptrs, e.bw_lds
     else:
-        ptrs = [0] * _lib.MAX_SCALES
-        lds = (C.c_int32 * _lib.MAX_SCALES)()
-        for s in range(S):
-            ptrs[s], lds[s] = base + 4 * sp.dF_off[s], sp.C_pad
-        ptrs_arr = _lib.ptr_array(ptrs)
-    if grad_out.dtype == torch.float32 and grad_out.device == dev and grad_out.is_contiguous():
-        g = grad_out                      # (only its address is used)
+        dF = torch.zeros(sp.dF_n, dtype=torch.float32, device=dev)
+        ptrs, ptrs_arr, lds = _row_accumulators(sp, dF.data_ptr())
+    g = _as_f32(grad_out, dev)
+    idx = [s for s in range(S) if needs[s]]
+    if fresh and state.grad_slab is not None and len(idx) == S:
+        # allocated and entered into the prebuilt structures by the forward
+        slab, items, rows, outs = state.grad_slab, e.bw_items, e.bw_rows, state.grad_outs
+        state.grad_slab = state.grad_outs = None
     else:
-        g = grad_out.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
-    grads = []
-    fbase = state.fslab.data_ptr()
-    io = state.io_dtypes or [torch.float32] * S         # dtypes the kernels write the dense gradients in
-    # a captured call: row counts only on the device (upper bounds on the host), no generator prefetch to launch
-    graph = getattr(state, "graph", False)
-    rows_dev = e.rows_dev if graph else [None] * S
-    n_rows = (lambda s: sp.Ncap[s]) if graph else (lambda s: state.samples[s].N)
-    dense = (not sp.nhwc) and state.gradbufs is None and \
-        all((not needs[s]) or (state.slots[s] is not None) for s in range(S))
-    if dense:
-        # default path: similarity backward + normalisation backward + one-pass dense writer in ONE C call
-        idx = [s for s in range(S) if needs[s]]
-        pre = getattr(state, "grad_slab", None) if (in_ws and len(idx) == S) else None
-        if pre is not None:                 # allocated and entered into the prebuilt structures by the forward
-            state.grad_slab = None
-            slab, items, rows = pre, e.bw_items, e.bw_rows
-            outs = dict(enumerate(state.grad_outs))
-            state.grad_outs = None
-        else:
-            slab, views, offs = _dense_grad_slab([shapes[s] for s in idx], [io[s] for s in idx], dev)
-            sbase = slab.data_ptr()
-            outs = {}
-            items = (_lib.ScatterItem * max(1, len(idx)))()
-            rows = (C.c_int32 * max(1, len(idx)))()
-            for j, s in enumerate(idx):
-                n, Cc, h, w = shapes[s]
-                outs[s] = views[j]
-                it = items[j]
-                it.dF, it.ldF, it.anc_f32, it.inv_norm = ptrs[s], sp.C_pad, fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
-                it.slot, it.n, it.C, it.plane = state.slots[s].data_ptr(), n, Cc, h * w
-                it.dfeat, it.dtype, it.n_rows_dev = sbase + offs[j], _DTYPE_CODE[io[s]], rows_dev[s]
-                rows[j] = n_rows(s)
-        evs, evp = None, None
-        if TIMING is not None:
-            evs = [torch.cuda.Event(enable_timing=True) for _ in range(3 if TIMING_ALL else 2)]
-            for ev in evs:
-                ev.record()         # creates the CUDA event; the chain records it again at its stage boundary
-            evp = _lib.ptr_array([ev.cuda_event for ev in evs] + [None] * (3 - len(evs)))
-        _lib.check(lib.mscs_backward_chain(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, items, rows,
-                                           len(idx), evp, st), "mscs_backward_chain")
-        if not graph:
-            _stream_cache(dev).flush()    # the deferred generator launch of the next call's stream
-        if evs is not None:
-            TIMING.setdefault("sim_bwd", []).append((evs[0], evs[1]))
-            if len(evs) == 3:
-                TIMING.setdefault("scatter", []).append((evs[1], evs[2]))
-        return [None if not needs[s] else (outs[s] if outs[s].dtype == dtypes[s] else outs[s].to(dtypes[s]))
-                for s in range(S)]
+        io = state.io_dtypes            # dtypes the kernels write the dense gradients in
+        slab, views, offs = _dense_grad_slab([shapes[s] for s in idx], [io[s] for s in idx], dev)
+        sbase, fbase = slab.data_ptr(), state.fslab.data_ptr()
+        outs = [None] * S
+        items = (_lib.ScatterItem * max(1, len(idx)))()
+        rows = (C.c_int32 * max(1, len(idx)))()
+        for j, s in enumerate(idx):
+            n, Cc, h, w = shapes[s]
+            outs[s] = views[j]
+            it = items[j]
+            it.dF, it.ldF, it.anc_f32, it.inv_norm = ptrs[s], sp.C_pad, fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
+            it.slot, it.n, it.C, it.plane = e.slots[s].data_ptr(), n, Cc, h * w
+            it.dfeat, it.dtype = sbase + offs[j], _DTYPE_CODE[io[s]]
+            # a captured call: row counts only on the device (upper bounds on the host)
+            it.n_rows_dev, rows[j] = (e.rows_dev[s], sp.Ncap[s]) if state.graph else (None, state.samples[s].N)
+    evs, evp = None, None
+    if TIMING is not None:
+        evs = [torch.cuda.Event(enable_timing=True) for _ in range(3 if TIMING_ALL else 2)]
+        for ev in evs:
+            ev.record()         # creates the CUDA event; the chain records it again at its stage boundary
+        evp = _lib.ptr_array([ev.cuda_event for ev in evs] + [None] * (3 - len(evs)))
+    _lib.check(lib.mscs_backward_chain(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, items, rows, len(idx), evp, st),
+               "mscs_backward_chain")
+    if not state.graph:
+        _stream_cache(dev).flush()    # the deferred generator launch of the next call's stream
+    if evs is not None:
+        TIMING.setdefault("sim_bwd", []).append((evs[0], evs[1]))
+        if len(evs) == 3:
+            TIMING.setdefault("scatter", []).append((evs[1], evs[2]))
+    return _as_dtypes(outs, dtypes)
+
+
+def _backward_rows(state, grad_out, needs, shapes, dtypes):
+    """Channels-last maps after the device-driven forward: similarity backward into the gradient rows, then one row
+    store per sampled pixel into the dense gradients.  Rows and dense gradients come pre-zeroed by the forward's fill;
+    a second backward through the same graph zero-fills fresh ones."""
+    lib = _lib.load()
+    sp, e, gb = state.sp, state.entry, state.gradbufs
+    dev, S = sp.dev, sp.S
+    st = _stream()
+    dF = gb.take_dF()
+    if dF is None:
+        dF = torch.zeros(sp.dF_n, dtype=torch.float32, device=dev)
+    _cur_stream().wait_event(gb.ready)
+    ptrs, ptrs_arr, lds = _row_accumulators(sp, dF.data_ptr())
+    g = _as_f32(grad_out, dev)
     with _timed("sim_bwd"):
-        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st),
-                   "mscs_sim_backward")
-    if not graph:
+        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st), "mscs_sim_backward")
+    if not state.graph:
         _stream_cache(dev).flush()        # the deferred generator launch of the next call's stream
-    if sp.nhwc:
-        with _timed("scatter"):
-            gb = state.gradbufs
-            if gb is not None:
-                _cur_stream().wait_event(gb.ready)
-            idx = [s for s in range(S) if needs[s]]
-            items = (_lib.RowsItem * max(1, len(idx)))()
-            outs = {}
-            for j, s in enumerate(idx):
-                n, Cc, h, w = shapes[s]
-                pre = gb.take(s) if gb is not None else None
-                if pre is None:      # second backward through the same graph
-                    pre = torch.zeros((n, h, w, Cc), dtype=io[s], device=dev).permute(0, 3, 1, 2)
-                outs[s] = pre
-                it = items[j]
-                it.pix = e.islab.data_ptr() + 4 * sp.ioff[s][2] if graph else state.samples[s].ptr(2)
-                it.rows, it.C, it.n_rows_dev = n_rows(s), Cc, rows_dev[s]
-                it.anc_f32, it.inv_norm = fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
-                it.dF, it.ldF, it.dfeat, it.dtype = ptrs[s], sp.C_pad, pre.data_ptr(), _DTYPE_CODE[io[s]]
-            if idx:
-                _lib.check(lib.mscs_scatter_rows_nhwc_batch(items, len(idx), st), "mscs_scatter_rows_nhwc_batch")
-            return [None if not needs[s] else (outs[s] if outs[s].dtype == dtypes[s] else outs[s].to(dtypes[s]))
-                    for s in range(S)]
+    io, fbase = state.io_dtypes, state.fslab.data_ptr()
     with _timed("scatter"):
-        gb = state.gradbufs
-        if gb is not None:
-            _cur_stream().wait_event(gb.ready)
-        batch = []
+        idx = [s for s in range(S) if needs[s]]
+        items = (_lib.RowsItem * max(1, len(idx)))()
+        outs = [None] * S
+        for j, s in enumerate(idx):
+            n, Cc, h, w = shapes[s]
+            pre = gb.take(s)
+            if pre is None:
+                pre = torch.zeros((n, h, w, Cc), dtype=io[s], device=dev).permute(0, 3, 1, 2)
+            outs[s] = pre
+            it = items[j]
+            it.pix, it.C = e.islab.data_ptr() + 4 * sp.ioff[s][2], Cc
+            # a captured call: row counts only on the device (upper bounds on the host)
+            it.n_rows_dev, it.rows = (e.rows_dev[s], sp.Ncap[s]) if state.graph else (None, state.samples[s].N)
+            it.anc_f32, it.inv_norm = fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
+            it.dF, it.ldF, it.dfeat, it.dtype = ptrs[s], sp.C_pad, pre.data_ptr(), _DTYPE_CODE[io[s]]
+        if idx:
+            _lib.check(lib.mscs_scatter_rows_nhwc_batch(items, len(idx), st), "mscs_scatter_rows_nhwc_batch")
+    return _as_dtypes(outs, dtypes)
+
+
+def _backward_host(state, grad_out, needs, shapes, dtypes):
+    """After the host-driven forward: similarity backward, then one batched sector scatter into the pre-zeroed gradients
+    of the scales with a slot map, and mscs_scatter_grad (which writes every element) for the others.  A second
+    backward through the same graph takes fresh zeroed rows and scatters every scale with mscs_scatter_grad."""
+    lib = _lib.load()
+    sp, gb = state.sp, state.gradbufs
+    dev, S = sp.dev, sp.S
+    st = _stream()
+    dF = gb.take_dF()
+    if dF is None:
+        dF = torch.zeros(sp.dF_n, dtype=torch.float32, device=dev)
+    _cur_stream().wait_event(gb.ready)
+    ptrs, ptrs_arr, lds = _row_accumulators(sp, dF.data_ptr())
+    g = _as_f32(grad_out, dev)
+    with _timed("sim_bwd"):
+        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st), "mscs_sim_backward")
+    _stream_cache(dev).flush()        # the deferred generator launch of the next call's stream
+    fbase = state.fslab.data_ptr()
+    grads, batch = [None] * S, []
+    with _timed("scatter"):
         for s in range(S):
             if not needs[s]:
-                grads.append(None)
                 continue
             n, Cc, h, w = shapes[s]
-            smp = state.samples[s]
-            pre, slot = (gb.take(s) if gb is not None else None), state.slots[s]
-            if pre is not None and slot is not None:
-                out = pre
-                # every scale in one launch (below)
-                batch.append((ptrs[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1], slot.data_ptr(),
-                              n, Cc, h * w, out.data_ptr()))
+            pre = gb.take(s)        # only scales with a slot map have one
+            if pre is not None:     # every such scale in one launch (below)
+                grads[s] = pre
+                batch.append((ptrs[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1], state.slots[s].data_ptr(),
+                              n, Cc, h * w, pre.data_ptr()))
             else:
-                out = torch.empty(shapes[s], dtype=torch.float32, device=dev)
+                grads[s] = torch.empty(shapes[s], dtype=torch.float32, device=dev)
+                smp = state.samples[s]
                 _lib.check(lib.mscs_scatter_grad(ptrs[s], sp.C_pad, fbase + 4 * sp.foff[s][0],
                                                  fbase + 4 * sp.foff[s][1], smp.ptr(2), smp.N, n, Cc, h * w,
-                                                 out.data_ptr(), 1, st), "mscs_scatter_grad")
-            grads.append(out)
+                                                 grads[s].data_ptr(), 1, st), "mscs_scatter_grad")
         if batch:
             items = (_lib.ScatterItem * len(batch))()
             for it, (dfp, f32p, invp, slotp, n, Cc, plane, outp) in zip(items, batch):
                 it.dF, it.ldF, it.anc_f32, it.inv_norm, it.slot = dfp, sp.C_pad, f32p, invp, slotp
                 it.n, it.C, it.plane, it.dfeat = n, Cc, plane, outp
             _lib.check(lib.mscs_scatter_sectors_batch(items, len(batch), st), "mscs_scatter_sectors_batch")
-        grads = [g_ if (g_ is None or dtypes[s] == torch.float32) else g_.to(dtypes[s]) for s, g_ in enumerate(grads)]
+        grads = _as_dtypes(grads, dtypes)
     return grads
+
+
+def run_backward(state, grad_out, needs, shapes, dtypes):
+    """The backward of the order the forward of `state` ran in (the state's `backward`)."""
+    return state.backward(state, grad_out, needs, shapes, dtypes)
 
 
 # ---- the autograd.Function ----------------------------------------------------------------

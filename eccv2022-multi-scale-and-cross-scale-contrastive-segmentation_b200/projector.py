@@ -26,6 +26,7 @@ dW_s and db_s exact.  Same loss, same gradients w.r.t. z_s, W_s and b_s as the d
 such module, so it sits next to the drop-in classes with its own, explicit interface.
 """
 import ctypes as C
+import time
 
 import torch
 import torch.nn as nn
@@ -146,38 +147,17 @@ class _ProjTailFn(torch.autograd.Function):
 
 def _forward(lib, sp, labels, maps, Ws, bs, c_prev, needs_z, any_grad, philox, graph):
     """One forward in the device-driven order (module docstring).  graph: captured call, nothing waits for the host."""
-    dev, S, A = sp.dev, sp.S, sp.A
+    dev, S = sp.dev, sp.S
     st, cur = _ops._stream(), _ops._cur_stream()
-    e = _TailWorkspace(sp, c_prev, graph=True) if graph else (sp.ws_pool.pop() if sp.ws_pool else _TailWorkspace(sp, c_prev))
-    if e.last_stream is not None and e.last_stream != cur:
-        cur.wait_stream(e.last_stream)          # reuse on another stream: order after its previous user
-    e.last_stream = cur
-    nt = len(sp.terms)
-    out = torch.empty(nt + 2, dtype=torch.float32, device=dev)      # term losses, total, inf/NaN flag
-    total_t = torch.empty((), dtype=torch.float32, device=dev)      # own buffer, not a view (see _ops._run_forward_fast)
-    for job in (e.job_fwd, e.job_bwd):
-        job.term_loss, job.total_loss = out.data_ptr(), out.data_ptr() + 4 * nt
-        job.total_out = total_t.data_ptr()
+    e, out, total_t = _ops._take_workspace(sp, graph, _TailWorkspace, c_prev)
     hp = _ops._hp_stream(dev) if _ops._USE_HP_STREAM else None
     ss = hp if hp is not None else cur
     st_s = C.c_void_p(ss.cuda_stream)
     if hp is not None:
         hp.wait_stream(cur)
-    if philox is None:          # MT19937 stream of the torch CPU generator (normally produced during the previous step)
-        mt, pos = _ops.torch_mt_state()
-        cache = _ops._stream_cache(dev)
-        draws = cache.acquire_nowait(mt, pos, sp.max_draws + _ops._MT_N).data_ptr()
-        ss.wait_event(cache.ready)
-    else:
-        if e.philox is None:
-            e.philox = torch.empty((sp.max_draws + 3) // 4 * 4 + 4, dtype=torch.int32, device=dev)
-        draws = e.philox.data_ptr()
-        if graph:
-            _lib.check(lib.mscs_philox_stream_dev(int(philox[0]) & (2 ** 64 - 1), philox[1].data_ptr(), sp.max_draws,
-                                                  draws, st_s), "mscs_philox_stream_dev")
-        else:
-            _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws, draws,
-                                              st_s), "mscs_philox_stream")
+    draws, ready, rng = _ops._call_draws(sp, e, philox, graph, st_s)
+    if ready is not None:       # the MT19937 stream, produced on the generator's side stream
+        ss.wait_event(ready)
     # channels-last dense gradients: pre-zeroed on a side stream, the sampled rows stored by the backward
     gradbufs = _ops._GradBuffers(maps, needs_z, True, 0) if (sp.nhwc and any(needs_z)) else None
     if gradbufs is not None:
@@ -208,24 +188,12 @@ def _forward(lib, sp, labels, maps, Ws, bs, c_prev, needs_z, any_grad, philox, g
             torch.addmm(bs[s].detach().float(), e.Z[s], W.t(), out=e.Pr[s])
     _lib.check(lib.mscs_gather_rows_nhwc_batch(e.pitems, S, st), "mscs_gather_rows_nhwc_batch")
     _lib.check(lib.mscs_sim_forward(C.byref(e.job_fwd), st), "mscs_sim_forward")
-    state = _ops._StepState()
-    state.sp, state.entry, state.graph = sp, e, graph     # (from here on an exception returns the workspace to the pool)
-    state.samples = None
+    # the state owns the workspace from here on (an exception returns it to the pool); the forward cleared the rows.
+    # The 0-d loss is not kept by the state: an output of the Function references its grad_fn, which owns the state
+    state = _ops._DeviceState(sp, e, graph, out, gradbufs, dF_fresh=True)
     if not graph:
-        plan = e.plan
-        _lib.check(lib.mscs_plan_fetch_end(plan, S), "mscs_plan_fetch_end")       # the one host wait
-        _ops._raise_plan_errors(plan, S, sp.spec)
-        state.samples = [_ops.ScaleSample(plan[s].T, plan[s].V, plan[s].N, bool(plan[s].log_flag), plan[s].dl_h,
-                                          plan[s].dl_w, e.islab, sp.ioff[s], A) for s in range(S)]
-        for i, (a, k, *_rest) in enumerate(sp.terms):      # the eager backward is launched with the actual counts
-            t = e.job_bwd.terms[i]
-            t.N1, t.N2 = state.samples[a].N, state.samples[k].N
-        if philox is None:
-            _ops._finish_rng(sp, dev, mt, pos, sum(int(plan[s].draws) for s in range(S)), defer=any_grad)
-    state.job, state.gradbufs = e.job_bwd, gradbufs
-    state.scalars, state.term_loss = out, out[:nt]
-    state.num_ms, state.cs_logged, state.comm = S, sp.cs_logged, None
-    # the 0-d loss is not kept by the state: an output of the Function references its grad_fn, which owns the state
+        _lib.check(lib.mscs_plan_fetch_end(e.plan, S), "mscs_plan_fetch_end")       # the one host wait
+        _ops._after_wait(state, rng, any_grad, time.perf_counter() if _ops.HOST_SEG is not None else 0.0)
     return state, total_t
 
 
@@ -233,10 +201,10 @@ def _backward(lib, state, grad_total, Ws, needs, dtypes):
     sp, e = state.sp, state.entry
     dev, S = sp.dev, sp.S
     st, cur = _ops._stream(), _ops._cur_stream()
-    if getattr(state, "bwd_done", False):       # a second backward through the same graph: fresh accumulators
+    if not state.dF_fresh:       # a second backward through the same graph: fresh accumulators
         _lib.check(lib.mscs_fill_bytes(e.tail_fill[0], e.tail_fill[1], e.tail_fill[2], 1, st), "mscs_fill_bytes")
-    state.bwd_done = True
-    g = grad_total.detach().to(device=dev, dtype=torch.float32).reshape(1).contiguous()
+    state.dF_fresh = False
+    g = _ops._as_f32(grad_total, dev)
     _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), e.bw_ptrs, e.bw_lds, st), "mscs_sim_backward")
     if not state.graph:
         _ops._stream_cache(dev).flush()        # the deferred generator launch of the next call's stream
@@ -282,10 +250,7 @@ def _backward(lib, state, grad_total, Ws, needs, dtypes):
             it.dfeat, it.dtype = views[j].data_ptr(), _ops._DTYPE_CODE[io[s]]
             rows[j] = sp.Ncap[s]
         _lib.check(lib.mscs_scatter_dense_batch(items, rows, len(idx), st), "mscs_scatter_dense_batch")
-    for s in idx:
-        if gz[s].dtype != dtypes[s]:
-            gz[s] = gz[s].to(dtypes[s])
-    return gz, gW, gb
+    return _ops._as_dtypes(gz, dtypes[:S]), gW, gb
 
 
 class ProjectorTailContrastive_ms(_GraphReadout, nn.Module):

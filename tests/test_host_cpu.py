@@ -175,7 +175,8 @@ def test_plan_errors_map_to_the_reference_exceptions():
 
 
 def test_fast_path_gate():
-    """Device-driven order: single process and a selection table (12 B per view) within 200 KB of shared memory."""
+    """Device-driven order: a single process.  The selection table (12 B per view) always fits the 200 KB of shared
+    memory, because V is capped at 16384 views (192 KB)."""
     mk = lambda **kw: _ops.LossSpec(num_classes=20, temperature=0.1, cs_temperature=0.1, **kw)
     assert _ops.fast_path_ok(mk(), 1)                                   # reference defaults: V <= 2500
     assert not _ops.fast_path_ok(mk(), 2)                               # pooled mode takes the host-driven order
