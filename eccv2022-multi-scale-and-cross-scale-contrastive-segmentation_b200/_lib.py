@@ -143,9 +143,13 @@ _SIGNATURES = {
     "mscs_xchg_push": (C.c_int, [_PTRS, C.c_int, C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64),
                                  C.POINTER(C.c_int32), C.c_int, C.c_void_p]),
     "mscs_gather_normalize_p2p": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, _PTRS,
-                                            C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
+                                            C.c_int, C.c_int, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "mscs_scatter_sectors_pull": (C.c_int, [_PTRS, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
-                                            C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+                                            C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "mscs_gather_rows_p2p": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, _PTRS, C.c_int, C.c_int,
+                                       C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
+    "mscs_scatter_rows_pull": (C.c_int, [_PTRS, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -845,17 +845,17 @@ def fast_path_ok(spec, world):
 
 def half_io_ok(sp, world):
     """Whether bf16 / fp16 feature maps are handed to the kernels as they are (no fp32 copy; the dense gradients are
-    written in the maps' dtype): the single-process fast path with the channels-last row gather, or with the NCHW octet
-    gather and the one-pass dense writer.  Every other route -- pooled mode, planes that are not a multiple of 8
-    pixels -- converts the maps to fp32 first and the gradients back afterwards."""
-    return fast_path_ok(sp.spec, world) and (sp.nhwc or all(sp.slot_sizes))
+    written in the maps' dtype), in a single process or in the pooled mode (any `world`): channels-last maps (row
+    gather), or NCHW maps whose planes are all a multiple of 8 pixels (octet gather over the slot maps).  The host-driven
+    path for other planes converts the maps to fp32 first and the gradients back afterwards."""
+    return sp.nhwc or all(sp.slot_sizes)
 
 
 def channels_last_ok(spec, world, feats):
-    """Channels-last feature maps (memory order [n][h][w][C]) are consumed as they are by the single-process fast path:
-    an anchor is then one contiguous row (gather / scatter become row copies)."""
-    return fast_path_ok(spec, world) and all(
-        f.dim() == 4 and f.is_contiguous(memory_format=torch.channels_last) and not f.is_contiguous() for f in feats)
+    """Channels-last feature maps (memory order [n][h][w][C]) are consumed as they are, in a single process or in the
+    pooled mode (any `world`): an anchor is then one contiguous row (gather / scatter become row copies)."""
+    return all(f.dim() == 4 and f.is_contiguous(memory_format=torch.channels_last) and not f.is_contiguous()
+               for f in feats)
 
 
 # first call index of graph replays: eager calls count up from 0 and never get here
@@ -1118,19 +1118,21 @@ class _HostState:
 
 
 class _PooledState(_HostState):
-    """A call of the pooled mode: also the exchange slab and the parity this step used.  ``dF_fresh``: as in
-    _DeviceState, for this parity's gradient rows in the exchange slab."""
+    """A call of the pooled mode: also the exchange slab and the parity this step used, and the dtypes the kernels read
+    and write the maps in.  ``dF_fresh``: as in _DeviceState, for this parity's gradient rows in the exchange slab."""
 
-    def __init__(self, sp, job, samples, gradbufs, slots, keep, fslab, scalars, total, comm, xs, par, exchange_info):
+    def __init__(self, sp, job, samples, gradbufs, slots, keep, fslab, scalars, total, comm, xs, par, exchange_info,
+                 io_dtypes):
         super().__init__(sp, job, samples, gradbufs, slots, keep, None, fslab, scalars, total)
         self.comm, self.xs, self.par, self.exchange_info = comm, xs, par, exchange_info
+        self.io_dtypes = io_dtypes
         self.dF_fresh = gradbufs is not None
         self.backward = _run_backward_pooled
 
 
 def run_forward(sp, labels, feats32, needs, comm=None, philox=None, graph=False):
     """philox: None (reference stream: torch CPU generator) or (seed, call index) of the opt-in counter-based stream.
-    feats32: fp32 maps, or bf16 / fp16 ones where half_io_ok(sp, world) holds (fast path only).
+    feats32: fp32 maps, or bf16 / fp16 ones where half_io_ok(sp, world) holds.
     graph: the call is captured into a CUDA graph (see graph_mode); philox is then (seed, int64 device call index).
     The state returned knows the backward of the order that ran (run_backward)."""
     pooled = comm is not None and comm.world > 1
@@ -1138,13 +1140,12 @@ def run_forward(sp, labels, feats32, needs, comm=None, philox=None, graph=False)
     # process, every plane a multiple of 8 pixels (slot maps) or channels-last maps
     if not pooled and (sp.nhwc or all(sp.slot_sizes)):
         return _run_forward_fast(sp, labels, feats32, needs, philox, graph)
-    assert all(f.dtype == torch.float32 for f in feats32), "half maps are converted by the caller off the fast path"
-    assert not sp.nhwc, "channels-last inputs are converted by the caller unless the fast path applies"
-    if philox is not None:
-        raise NotImplementedError("sampler='philox' is implemented for the single-process path with feature planes "
-                                  "that are a multiple of 8 pixels (or channels-last inputs)")
     if pooled:
-        return _run_forward_pooled(sp, labels, feats32, needs, comm)
+        return _run_forward_pooled(sp, labels, feats32, needs, comm, philox)
+    assert all(f.dtype == torch.float32 for f in feats32), "half maps are converted by the caller off the fast path"
+    if philox is not None:
+        raise NotImplementedError("sampler='philox' is implemented for feature planes that are a multiple of 8 pixels "
+                                  "(or channels-last inputs)")
     return _run_forward_general(sp, labels, feats32, needs)
 
 
@@ -1370,7 +1371,7 @@ def _run_forward_general(sp, labels, feats32, needs):
                       fslab, misc[sp.out_off:sp.out_off + nt + 2], total_t)
 
 
-def _run_forward_pooled(sp, labels, feats32, needs, comm):
+def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
     """POOLED cross-batch mode (one process per GPU, each with its own images): the reference loss of the concatenated
     batch of all ranks.  Control plane over NCCL (class histograms: a few KB); data plane by the library's own kernels
     over NVLink peer memory (csrc/xchg.cu), ordered by three device-side barriers per step:
@@ -1381,13 +1382,18 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
       K3 sweeps over this rank's anchor-row range against all keys -> its row statistics pushed to every peer ->
       barrier B -> finalise on all rows (every rank then holds the global loss and the coefficients of every row, so
       the backward needs no reduce-scatter) -> [backward: K4 over the rank's row range -> barrier C -> the scatter
-      PULLS each gradient row of a local pixel from the rank that computed it]."""
+      PULLS each gradient row of a local pixel from the rank that computed it].
+
+    The maps are read in their dtype (fp32 / bf16 / fp16) and layout: NCHW through the slot maps (planes a multiple of
+    8 pixels), channels-last as rows (no slot maps).  philox: (seed, call index) -- every rank generates the same
+    stream of the whole batch's draws and the torch CPU generator is not touched."""
     lib = _lib.load()
     dev, S, A, spec = sp.dev, sp.S, sp.A, sp.spec
     st = _stream()
     i32, f32, u8 = torch.int32, torch.float32, torch.uint8
-    if not all(sp.slot_sizes):
-        raise NotImplementedError("pooled mode needs feature planes that are a multiple of 8 pixels")
+    if not sp.nhwc and not all(sp.slot_sizes):
+        raise NotImplementedError("pooled mode needs NCHW feature planes that are a multiple of 8 pixels "
+                                  "(or channels-last maps)")
     if sp.xslab is None:
         sp.xslab = comm.symmetric(sp.x_bytes, dev)           # collective, first call only
     xs = sp.xslab
@@ -1408,28 +1414,35 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
         cptr = _lib.ptr_array([counts_g[s].data_ptr() for s in range(S)])
         _lib.check(lib.mscs_sample_plan_from_counts(C.byref(sp.cfg), cptr, ws.data_ptr(), plan_dev.data_ptr(), st),
                    "mscs_sample_plan_from_counts")
-        sizes = sp.slot_sizes
         islab = torch.empty(sp.islab_n, dtype=i32, device=dev)
         fslab = torch.empty(sp.fslab_n, dtype=f32, device=dev)
         misc = torch.empty(sp.misc_n, dtype=f32, device=dev)
         work = torch.empty(sp.work_bytes, dtype=u8, device=dev)
-        slot_slab = torch.full((sum(sizes),), -1, dtype=i32, device=dev)
-        slots, off = [], 0
-        for x in sizes:
-            slots.append(slot_slab[off:off + x])
-            off += x
-        # dense gradients (local): zero-filled on the side stream.  Row statistics: the sweeps accumulate them (one
-        # atomic per row, quarter and tile) in PRIVATE memory; pushed to every rank's slab afterwards
-        gradbufs = _GradBuffers(feats32, needs, False, 0) if any(needs) else None
+        slot_slab, slots, sarr = None, [None] * S, None      # channels-last maps: rows are gathered through `pix`
+        if not sp.nhwc:
+            slot_slab = torch.full((sum(sp.slot_sizes),), -1, dtype=i32, device=dev)
+            slots, off = [], 0
+            for x in sp.slot_sizes:
+                slots.append(slot_slab[off:off + x])
+                off += x
+            sarr = _lib.ptr_array([x.data_ptr() for x in slots])
+        # dense gradients (local, in the maps' dtype and layout): zero-filled on the side stream.  Row statistics: the
+        # sweeps accumulate them (one atomic per row, quarter and tile) in PRIVATE memory; pushed to every rank's slab
+        # afterwards
+        gradbufs = _GradBuffers(feats32, needs, sp.nhwc, 0) if any(needs) else None
         if gradbufs is not None:
             gradbufs.start_fill()
         stats_priv = torch.zeros(sp.stats_n, dtype=f32, device=dev)
-        mt, pos = torch_mt_state()
-        draws = _stream_cache(dev).acquire(mt, pos, sp.max_draws + _MT_N)
+        if philox is None:
+            mt, pos = torch_mt_state()
+            draws = _stream_cache(dev).acquire(mt, pos, sp.max_draws + _MT_N)
+        else:       # the same stream on every rank: sp.max_draws covers the draws of all ranks' images
+            draws = torch.empty((sp.max_draws + 3) // 4 * 4 + 4, dtype=i32, device=dev)
+            _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws,
+                                              draws.data_ptr(), st), "mscs_philox_stream")
         plan = (_lib.ScalePlan * S)()
         ibase = islab.data_ptr()
         arrs = [_lib.ptr_array([ibase + 4 * sp.ioff[s][k] for s in range(S)]) for k in range(5)]
-        sarr = _lib.ptr_array([x.data_ptr() for x in slots])
         fbase, bbase = fslab.data_ptr(), xs.local + xo["b"]
         # two views of the same terms: `job_sw` (sweeps: statistics in private memory) and `job` (finalise and
         # backward: statistics of ALL rows in the exchange slab)
@@ -1451,10 +1464,16 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
     with _timed("gather"):
         for s in range(S):
             n, Cc, h, w = sp.feat_shapes[s]
-            _lib.check(lib.mscs_gather_normalize_p2p(
-                feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(), 0, plan_dev.data_ptr() + s * plan_sz + 8,
-                xs.peers, world, rank, xo["b"] + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1],
-                st), "mscs_gather_normalize_p2p")
+            n_dev, code = plan_dev.data_ptr() + s * plan_sz + 8, _DTYPE_CODE[feats32[s].dtype]
+            boff, f32p, invp = xo["b"] + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
+            if sp.nhwc:         # the grid covers the row bound; the count is read on the device
+                _lib.check(lib.mscs_gather_rows_p2p(feats32[s].data_ptr(), Cc, ibase + 4 * sp.ioff[s][2], sp.Ncap[s],
+                                                    n_dev, xs.peers, world, rank, boff, f32p, invp, st, code),
+                           "mscs_gather_rows_p2p")
+            else:
+                _lib.check(lib.mscs_gather_normalize_p2p(feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(), 0,
+                                                         n_dev, xs.peers, world, rank, boff, f32p, invp, st, code),
+                           "mscs_gather_normalize_p2p")
         comm.barrier(xs)                                   # A: every rank's key rows have landed here
     _lib.check(lib.mscs_plan_fetch_end(plan, S), "mscs_plan_fetch_end")       # the host wait (plan records only)
     _raise_plan_errors(plan, S, spec)
@@ -1492,7 +1511,7 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
                                       len(push_off), st), "mscs_xchg_push")
         comm.barrier(xs)                                   # B: the statistics of every row are complete here
         _lib.check(lib.mscs_sim_finalize(C.byref(job), st), "mscs_sim_finalize")
-    if comm.owns_rng:
+    if philox is None and comm.owns_rng:
         _finish_rng(sp, dev, mt, pos, total)
     n_local = sum(int(samples[s].N) for s in range(S)) / world        # rows this rank owns, on average
     exchange_info = {
@@ -1503,15 +1522,18 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm):
         "key_rows_stored_to_peers_bytes": int(n_local * sp.C_pad * 2 * (world - 1)),
         "row_statistics_pushed_bytes": int(sum(push_len) * 4 * (world - 1)),
         "gradient_rows_pulled_bytes": int(n_local * sp.C_pad * 4 * (world - 1) / world)}
-    return _PooledState(sp, job, samples, gradbufs, slots, (ws, islab, fslab, misc, work, slot_slab, stats_priv), fslab,
-                        misc[sp.out_off:sp.out_off + nt + 2], total_t, comm, xs, par, exchange_info)
+    return _PooledState(sp, job, samples, gradbufs, slots, (ws, islab, fslab, misc, work, slot_slab, stats_priv, draws),
+                        fslab, misc[sp.out_off:sp.out_off + nt + 2], total_t, comm, xs, par, exchange_info,
+                        [f.dtype for f in feats32])
 
 
 def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
     """Pooled mode: every rank computes the COMPLETE gradient rows of its 128-aligned row block of every anchor set
     (one launch for all passes) into its exchange slab; after the barrier the scatter pulls the row of every LOCAL
-    pixel from the rank that computed it -- an eighth of the rows travels, once, to where it is needed.  A second
-    backward through the same graph clears the rows again and zero-fills fresh dense gradients."""
+    pixel from the rank that computed it -- an eighth of the rows travels, once, to where it is needed.  The dense
+    gradients are written by the scatter in the maps' dtype and layout (sector scatter for NCHW maps, row scatter for
+    channels-last ones).  A second backward through the same graph clears the rows again and zero-fills fresh dense
+    gradients."""
     lib = _lib.load()
     sp, comm, xs = state.sp, state.comm, state.xs
     dev, S = sp.dev, sp.S
@@ -1531,7 +1553,7 @@ def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
         _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st), "mscs_sim_backward")
         comm.barrier(xs)                            # C: every rank's gradient rows are complete
     grads = []
-    fbase = state.fslab.data_ptr()
+    io, fbase = state.io_dtypes, state.fslab.data_ptr()
     with _timed("scatter"):
         for s in range(S):
             if not needs[s]:
@@ -1540,15 +1562,20 @@ def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
             n, Cc, h, w = shapes[s]
             pre = gb.take(s) if gb is not None else None
             if pre is None:
-                pre = torch.zeros(shapes[s], dtype=torch.float32, device=dev)
+                pre = torch.zeros((n, h, w, Cc), dtype=io[s], device=dev).permute(0, 3, 1, 2) if sp.nhwc else \
+                    torch.zeros(shapes[s], dtype=io[s], device=dev)
             N = state.samples[s].N
             per = ((N + 127) // 128 + comm.world - 1) // comm.world * 128
-            _lib.check(lib.mscs_scatter_sectors_pull(xs.peers, comm.world, xo["dF"] + 4 * sp.dF_off[s], per, sp.C_pad,
-                                                     fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1],
-                                                     state.slots[s].data_ptr(), n, Cc, h * w, pre.data_ptr(), st),
-                       "mscs_scatter_sectors_pull")
-            grads.append(pre if dtypes[s] == torch.float32 else pre.to(dtypes[s]))
-    return grads
+            args = (xs.peers, comm.world, xo["dF"] + 4 * sp.dF_off[s], per, sp.C_pad, fbase + 4 * sp.foff[s][0],
+                    fbase + 4 * sp.foff[s][1])
+            if sp.nhwc:
+                _lib.check(lib.mscs_scatter_rows_pull(*args, state.samples[s].ptr(2), N, Cc, pre.data_ptr(), st,
+                                                      _DTYPE_CODE[io[s]]), "mscs_scatter_rows_pull")
+            else:
+                _lib.check(lib.mscs_scatter_sectors_pull(*args, state.slots[s].data_ptr(), n, Cc, h * w, pre.data_ptr(),
+                                                         st, _DTYPE_CODE[io[s]]), "mscs_scatter_sectors_pull")
+            grads.append(pre)
+    return _as_dtypes(grads, dtypes)
 
 
 def _row_accumulators(sp, base):
@@ -1735,8 +1762,8 @@ class MsCsContrastiveFn(torch.autograd.Function):
             if not _lib.load().mscs_device_ok():
                 raise RuntimeError("mscs_b200 needs a compute-capability 10.x (B200) device; no fallback exists")
             _device_checked[0] = True
-        # channels-last feature maps (memory order [n][h][w][C]) are consumed as they are by the single-process fast
-        # path: an anchor is then one contiguous row (gather / scatter become row copies)
+        # channels-last feature maps (memory order [n][h][w][C]) are consumed as they are: an anchor is then one
+        # contiguous row (gather / scatter become row copies)
         nhwc = channels_last_ok(spec, world, feats)
         for f in feats:
             _require_device(f)

@@ -129,4 +129,15 @@ static inline int dtype_bytes(int dtype) {
   return dtype == MSCS_DTYPE_F32 ? 4 : (dtype == MSCS_DTYPE_BF16 || dtype == MSCS_DTYPE_F16) ? 2 : 0;
 }
 
+// host side, element-type checks of the entry points: a known MSCS_DTYPE_* code and an address aligned to `align`
+// bytes (at least the element size).  `s`: the item of a batched call the message names, -1 for an unbatched call.
+static inline int check_dtype(int s, int dtype, const void* p, int align, const char* what) {
+  char item[24] = "";
+  if (s >= 0) snprintf(item, sizeof(item), "item %d: ", s);
+  MSCS_CHECK_ARG(dtype_bytes(dtype) > 0, "%sdtype %d unknown (MSCS_DTYPE_F32 / _BF16 / _F16)", item, dtype);
+  const int a = align > dtype_bytes(dtype) ? align : dtype_bytes(dtype);
+  MSCS_CHECK_ARG((uintptr_t)p % a == 0, "%s%s must be %d-byte aligned", item, what, a);
+  return 0;
+}
+
 }  // namespace mscs

@@ -196,10 +196,13 @@ __global__ void k_slot_map(const int* __restrict__ pix, int N, int* __restrict__
 // (n == 0: every row is local, `dF` is used)
 struct PullRows { const float* p[MSCS_MAX_RANKS]; int n, rows_per_rank; };
 
+// T: element type of the dense gradient.  fp32: two float4 stores per lane and channel; half: the octet's 8 values
+// rounded (nearest even) into one 16-byte store.
+template <typename T>
 __device__ __forceinline__ void
 scatter_sectors_body(const float* __restrict__ dF, int ldF, const float* __restrict__ anc_f32,
                   const float* __restrict__ inv_norm, const int* __restrict__ slot, int n_octets, int C,
-                  int plane, float* __restrict__ dfeat, int block_base, const PullRows* pull = nullptr) {
+                  int plane, T* __restrict__ dfeat, int block_base, const PullRows* pull = nullptr) {
   const int lane = threadIdx.x & 31;
   const int oct = ((int)blockIdx.x - block_base) * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (oct >= n_octets) return;
@@ -236,18 +239,58 @@ scatter_sectors_body(const float* __restrict__ dF, int ldF, const float* __restr
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
     if (c < C) {
-      float4* dst = reinterpret_cast<float4*>(dfeat + ((size_t)b * C + c) * plane + p);
-      dst[0] = make_float4(dx[0][q], dx[1][q], dx[2][q], dx[3][q]);
-      dst[1] = make_float4(dx[4][q], dx[5][q], dx[6][q], dx[7][q]);
+      T* dst = dfeat + ((size_t)b * C + c) * plane + p;
+      if constexpr (sizeof(T) == 4) {
+        float4* d4 = reinterpret_cast<float4*>(dst);
+        d4[0] = make_float4(dx[0][q], dx[1][q], dx[2][q], dx[3][q]);
+        d4[1] = make_float4(dx[4][q], dx[5][q], dx[6][q], dx[7][q]);
+      } else {
+        *reinterpret_cast<uint4*>(dst) = make_uint4(pack2(dst, dx[0][q], dx[1][q]), pack2(dst, dx[2][q], dx[3][q]),
+                                                    pack2(dst, dx[4][q], dx[5][q]), pack2(dst, dx[6][q], dx[7][q]));
+      }
     }
   }
 }
 
+template <typename T>
 __global__ void __launch_bounds__(256)
 k_scatter_sectors_pull(const __grid_constant__ PullRows pull, int ldF, const float* __restrict__ anc_f32,
                        const float* __restrict__ inv_norm, const int* __restrict__ slot, int n_octets, int C,
-                       int plane, float* __restrict__ dfeat) {
-  scatter_sectors_body(nullptr, ldF, anc_f32, inv_norm, slot, n_octets, C, plane, dfeat, 0, &pull);
+                       int plane, T* __restrict__ dfeat) {
+  scatter_sectors_body<T>(nullptr, ldF, anc_f32, inv_norm, slot, n_octets, C, plane, dfeat, 0, &pull);
+}
+
+// Channels-last pooled scatter: one warp per sorted row with pix >= 0, gradient row read from the slab of rank
+// row / rows_per_rank, then the normalisation backward and row store of k_scatter_rows_nhwc (below) into the
+// pre-zeroed channels-last dense gradient
+template <typename T>
+__global__ void __launch_bounds__(256)
+k_scatter_rows_pull(const __grid_constant__ PullRows pull, int ldF, const float* __restrict__ anc_f32,
+                    const float* __restrict__ inv_norm, const int* __restrict__ pix, int N, int C, T* __restrict__ dfeat) {
+  const int lane = threadIdx.x & 31;
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (row >= N) return;
+  const int gp = pix[row];
+  if (gp < 0) return;
+  const float* gr = pull.p[row / pull.rows_per_rank] + (size_t)row * ldF;
+  const float* f = anc_f32 + (size_t)row * C;
+  float gv[kMaxC / 32], fv[kMaxC / 32], dot = 0.f;
+#pragma unroll
+  for (int q = 0; q < kMaxC / 32; ++q) {
+    const int c = lane + 32 * q;
+    gv[q] = (c < C) ? gr[c] : 0.f;
+    fv[q] = (c < C) ? f[c] : 0.f;
+    dot = fmaf(gv[q], fv[q], dot);
+  }
+  dot = warp_sum(dot);
+  const float inv = inv_norm[row];
+  const bool clamped = inv >= 1e12f;        // ||x|| <= eps: F.normalize divides by the constant eps
+  T* dst = dfeat + (size_t)gp * C;
+#pragma unroll
+  for (int q = 0; q < kMaxC / 32; ++q) {
+    const int c = lane + 32 * q;
+    if (c < C) dst[c] = from_f32<T>((clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv);
+  }
 }
 
 
@@ -474,34 +517,62 @@ extern "C" int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* s
   return 0;
 }
 
+// pooled mode: the gradient rows of every rank's slab at dF_byte_off (row i: rank i / rows_per_rank)
+static int pull_rows(PullRows* pull, void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank) {
+  MSCS_CHECK_ARG(slabs, "null pointer argument");
+  MSCS_CHECK_ARG(world >= 1 && world <= MSCS_MAX_RANKS && rows_per_rank >= 1, "bad world %d / rows per rank %d", world,
+                 rows_per_rank);
+  pull->n = world; pull->rows_per_rank = rows_per_rank;
+  for (int r = 0; r < world; ++r) {
+    MSCS_CHECK_ARG(slabs[r] != nullptr, "peer %d: null slab pointer", r);
+    pull->p[r] = reinterpret_cast<const float*>((const char*)slabs[r] + dF_byte_off);
+  }
+  return 0;
+}
+
 // pooled mode: the same scatter with every gradient row read from the rank that computed it (row / rows_per_rank)
 extern "C" int mscs_scatter_sectors_pull(void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank, int ldF,
                                          const float* anc_f32, const float* inv_norm, const int32_t* slot, int n, int C,
-                                         int plane, float* dfeat, void* stream_) {
+                                         int plane, void* dfeat, void* stream_, int dtype) {
   MSCS_CHECK_ARG(slabs && anc_f32 && inv_norm && slot && dfeat, "null pointer argument");
-  MSCS_CHECK_ARG(world >= 1 && world <= MSCS_MAX_RANKS && rows_per_rank >= 1, "bad world %d / rows per rank %d", world,
-                 rows_per_rank);
+  PullRows pull{};
+  if (int rc = pull_rows(&pull, slabs, world, dF_byte_off, rows_per_rank)) return rc;
   MSCS_CHECK_ARG(C >= 1 && C <= kMaxC && ldF >= C, "C=%d / ldF=%d unsupported", C, ldF);
   MSCS_CHECK_ARG(plane % 8 == 0, "plane %d is not a multiple of 8 pixels", plane);
-  PullRows pull{};
-  pull.n = world; pull.rows_per_rank = rows_per_rank;
-  for (int r = 0; r < world; ++r) {
-    MSCS_CHECK_ARG(slabs[r] != nullptr, "peer %d: null slab pointer", r);
-    pull.p[r] = reinterpret_cast<const float*>((const char*)slabs[r] + dF_byte_off);
-  }
-  const int n_oct = n * (plane / 8);
-  k_scatter_sectors_pull<<<ceil_div(n_oct, 8), 256, 0, (cudaStream_t)stream_>>>(pull, ldF, anc_f32, inv_norm, slot,
-                                                                                n_oct, C, plane, dfeat);
+  if (int rc = check_dtype(-1, dtype, dfeat, 16, "dfeat")) return rc;
+  const int n_oct = n * (plane / 8), grid = ceil_div(n_oct, 8);
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (dtype == MSCS_DTYPE_F32)
+    k_scatter_sectors_pull<float><<<grid, 256, 0, st>>>(pull, ldF, anc_f32, inv_norm, slot, n_oct, C, plane, (float*)dfeat);
+  else if (dtype == MSCS_DTYPE_BF16)
+    k_scatter_sectors_pull<__nv_bfloat16><<<grid, 256, 0, st>>>(pull, ldF, anc_f32, inv_norm, slot, n_oct, C, plane,
+                                                                (__nv_bfloat16*)dfeat);
+  else
+    k_scatter_sectors_pull<__half><<<grid, 256, 0, st>>>(pull, ldF, anc_f32, inv_norm, slot, n_oct, C, plane, (__half*)dfeat);
   MSCS_LAUNCH_CHECK();
   return 0;
 }
 
-// element-type checks shared by the batched entry points: a known MSCS_DTYPE_* code and an address aligned to `align`
-// bytes (at least the element size)
-static int check_dtype(int s, int dtype, const void* p, int align, const char* what) {
-  MSCS_CHECK_ARG(dtype_bytes(dtype) > 0, "item %d: dtype %d unknown (MSCS_DTYPE_F32 / _BF16 / _F16)", s, dtype);
-  const int a = align > dtype_bytes(dtype) ? align : dtype_bytes(dtype);
-  MSCS_CHECK_ARG((uintptr_t)p % a == 0, "item %d: %s must be %d-byte aligned", s, what, a);
+// pooled mode, channels-last: the row scatter with every gradient row read from the rank that computed it
+extern "C" int mscs_scatter_rows_pull(void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank, int ldF,
+                                      const float* anc_f32, const float* inv_norm, const int32_t* pix, int N, int C,
+                                      void* dfeat, void* stream_, int dtype) {
+  MSCS_CHECK_ARG(slabs && anc_f32 && inv_norm && pix && dfeat, "null pointer argument");
+  PullRows pull{};
+  if (int rc = pull_rows(&pull, slabs, world, dF_byte_off, rows_per_rank)) return rc;
+  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC && ldF >= C && N >= 0, "C=%d / ldF=%d / %d rows unsupported", C, ldF, N);
+  if (int rc = check_dtype(-1, dtype, dfeat, 1, "dfeat")) return rc;
+  const int grid = ceil_div(N, 8);
+  if (grid == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (dtype == MSCS_DTYPE_F32)
+    k_scatter_rows_pull<float><<<grid, 256, 0, st>>>(pull, ldF, anc_f32, inv_norm, pix, N, C, (float*)dfeat);
+  else if (dtype == MSCS_DTYPE_BF16)
+    k_scatter_rows_pull<__nv_bfloat16><<<grid, 256, 0, st>>>(pull, ldF, anc_f32, inv_norm, pix, N, C,
+                                                             (__nv_bfloat16*)dfeat);
+  else
+    k_scatter_rows_pull<__half><<<grid, 256, 0, st>>>(pull, ldF, anc_f32, inv_norm, pix, N, C, (__half*)dfeat);
+  MSCS_LAUNCH_CHECK();
   return 0;
 }
 
@@ -572,8 +643,8 @@ struct ScatterBatch {
 __global__ void __launch_bounds__(256) k_scatter_sectors_batch(const __grid_constant__ ScatterBatch g) {
   int s = 0;
   while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
-  scatter_sectors_body(g.dF[s], g.ldF[s], g.f32[s], g.inv[s], g.slot[s], g.n_oct[s], g.C[s], g.plane[s], g.dfeat[s],
-                       g.block0[s]);
+  scatter_sectors_body<float>(g.dF[s], g.ldF[s], g.f32[s], g.inv[s], g.slot[s], g.n_oct[s], g.C[s], g.plane[s],
+                              g.dfeat[s], g.block0[s]);
 }
 
 extern "C" int mscs_scatter_sectors_batch(const mscs_scatter_item* items, int count, void* stream_) {

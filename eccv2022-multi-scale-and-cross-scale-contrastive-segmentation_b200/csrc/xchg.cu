@@ -9,6 +9,7 @@
 //   k_gather_p2p        K2 fused with the all-gather: every normalised bf16 anchor row is stored -- 16 bytes per lane,
 //                       one 512-byte row per warp instruction -- straight into the SAME sorted row of the operand
 //                       matrix of every rank (its own included).  No packing, no collective, no zero slab.
+//   k_gather_rows_p2p   the same for channels-last maps: one warp per sorted row of this rank.
 //   k_push_ranges       row statistics of this rank's anchor-row range (accumulated in PRIVATE memory: the sweeps'
 //                       per-tile atomics into the peer-mapped slab itself ran sweep 0 1.7x slower) -> the same rows
 //                       of every rank's slab.
@@ -74,12 +75,15 @@ __global__ void __launch_bounds__(256) k_push_ranges(const __grid_constant__ Pus
 // K2 + all-gather.  One warp per 8-pixel octet of the slot map (address order, like k_gather_sectors); lane l owns
 // channels [8l, 8l+8): eight strided sector reads, then ONE 16-byte store per destination matrix.
 struct GatherP2P {
-  const float* feat; const int* slot; float* anc_f32; float* inv_norm;
+  const void* feat; const int* slot; float* anc_f32; float* inv_norm;
   PeerPtrs bf16;            // the operand matrix of this scale in every rank's slab (same sorted row index everywhere)
   int C, C_pad, plane, n_octets, rank;
   int n_rows;               // N: the local padding rows [N, N_pad) are zeroed by the extra last block
   const int* n_rows_dev;    // optional: N lives in device memory (the launch then does not wait for the host)
 };
+// T: element type of the map (float / bf16 / fp16).  Loads widen exactly to fp32 (to_f32) and everything after them is
+// the fp32 arithmetic, so a half map gives the rows of its fp32 widening bit for bit.
+template <typename T>
 __global__ void __launch_bounds__(256) k_gather_p2p(const __grid_constant__ GatherP2P g) {
   const int lane = threadIdx.x & 31;
   if (blockIdx.x == gridDim.x - 1) {      // padding rows of the LOCAL matrix (the TMA tiles read them)
@@ -96,17 +100,17 @@ __global__ void __launch_bounds__(256) k_gather_p2p(const __grid_constant__ Gath
   if (act == 0) return;
   const int C = g.C, plane = g.plane;
   const int b = gp / plane, p = gp - b * plane;
-  const float* src0 = g.feat + ((size_t)b * C) * plane + p;
+  const T* src0 = static_cast<const T*>(g.feat) + ((size_t)b * C) * plane + p;
   const int c0 = lane * 8;
   while (act) {
     const int j = __ffs(act) - 1;
     act &= act - 1;
     const int row = __shfl_sync(0xffffffffu, s_mine, j);
-    const float* src = src0 + j;
+    const T* src = src0 + j;
     float v[8];
     float ss = 0.f;
 #pragma unroll
-    for (int q = 0; q < 8; ++q) v[q] = (c0 + q < C) ? __ldg(src + (size_t)(c0 + q) * plane) : 0.f;
+    for (int q = 0; q < 8; ++q) v[q] = (c0 + q < C) ? to_f32(__ldg(src + (size_t)(c0 + q) * plane)) : 0.f;
 #pragma unroll
     for (int q = 0; q < 8; ++q) ss = fmaf(v[q], v[q], ss);
     ss = warp_sum(ss);
@@ -125,6 +129,58 @@ __global__ void __launch_bounds__(256) k_gather_p2p(const __grid_constant__ Gath
       const uint4 w = make_uint4(pk[0], pk[1], pk[2], pk[3]);
       for (int r = 0; r < g.bf16.n; ++r)
         *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(g.bf16.p[r]) + (size_t)row * g.C_pad + c0) = w;
+    }
+  }
+}
+
+// Channels-last maps: one warp per sorted row with pix >= 0; lane l owns the channels l + 32 q, the lane / channel
+// assignment of k_gather_rows_nhwc, so the unit rows, inverse norms and operand rows equal the single-process ones bit
+// for bit.  The fp32 row and inverse norm stay local, the bf16 row is stored into every rank's operand matrix.
+// Rows with pix < 0 are NOT written: they belong to other ranks, whose peer stores land in this slab concurrently.
+// Only the local padding rows [N, N_pad) are zeroed.
+struct GatherRowsP2P {
+  const void* feat; const int* pix; float* anc_f32; float* inv_norm;
+  PeerPtrs bf16;            // as GatherP2P
+  int C, C_pad, rank;
+  int n_rows;               // N, or its upper bound when n_rows_dev is set (sizes the grid)
+  const int* n_rows_dev;
+};
+template <typename T>
+__global__ void __launch_bounds__(256) k_gather_rows_p2p(const __grid_constant__ GatherRowsP2P g) {
+  const int lane = threadIdx.x & 31;
+  const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  const int N = g.n_rows_dev ? *g.n_rows_dev : g.n_rows, N_pad = (N + 255) / 256 * 256;
+  if (row >= N_pad) return;
+  const int C = g.C, C_pad = g.C_pad;
+  if (row >= N) {
+    __nv_bfloat16* orow = reinterpret_cast<__nv_bfloat16*>(g.bf16.p[g.rank]) + (size_t)row * C_pad;
+    for (int c = lane; c < C_pad; c += 32) orow[c] = __float2bfloat16(0.f);
+    return;
+  }
+  const int gp = g.pix[row];
+  if (gp < 0) return;
+  const T* src = static_cast<const T*>(g.feat) + (size_t)gp * C;
+  float v[kMaxC / 32];
+  float ss = 0.f;
+#pragma unroll
+  for (int q = 0; q < kMaxC / 32; ++q) {
+    const int c = lane + 32 * q;
+    v[q] = (c < C) ? to_f32(__ldg(src + c)) : 0.f;
+  }
+#pragma unroll
+  for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q], v[q], ss);
+  ss = warp_sum(ss);
+  const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
+  if (lane == 0) g.inv_norm[row] = inv;
+#pragma unroll
+  for (int q = 0; q < kMaxC / 32; ++q) {
+    const int c = lane + 32 * q;
+    const float f = v[q] * inv;
+    if (c < C) g.anc_f32[(size_t)row * C + c] = f;
+    if (c < C_pad) {
+      const __nv_bfloat16 h = __float2bfloat16(c < C ? f : 0.f);
+      for (int r = 0; r < g.bf16.n; ++r)
+        reinterpret_cast<__nv_bfloat16*>(g.bf16.p[r])[(size_t)row * C_pad + c] = h;
     }
   }
 }
@@ -205,17 +261,43 @@ extern "C" int mscs_xchg_push(void* const* slabs, int world, const float* src, c
   return 0;
 }
 
-extern "C" int mscs_gather_normalize_p2p(const float* feat, int n, int C, int plane, const int32_t* slot, int N,
+extern "C" int mscs_gather_normalize_p2p(const void* feat, int n, int C, int plane, const int32_t* slot, int N,
                                          const int32_t* n_rows_dev, void* const* slabs, int world, int rank,
-                                         size_t bf16_byte_off, float* anc_f32, float* inv_norm, void* stream_) {
+                                         size_t bf16_byte_off, float* anc_f32, float* inv_norm, void* stream_, int dtype) {
   MSCS_CHECK_ARG(feat && slot && anc_f32 && inv_norm, "null pointer argument");
   MSCS_CHECK_ARG(C >= 1 && C <= kMaxC && plane % 8 == 0 && n >= 1 && N >= 0, "unsupported shape (C %d, plane %d)", C, plane);
   MSCS_CHECK_ARG(rank >= 0 && rank < world && bf16_byte_off % 16 == 0, "bad rank / offset");
+  if (int rc = check_dtype(-1, dtype, feat, 1, "feat")) return rc;
   GatherP2P g{};
   if (int rc = fill_peers(&g.bf16, slabs, world, bf16_byte_off)) return rc;
   g.feat = feat; g.slot = slot; g.anc_f32 = anc_f32; g.inv_norm = inv_norm;
   g.C = C; g.C_pad = (C + 63) / 64 * 64; g.plane = plane; g.n_octets = n * plane / 8; g.rank = rank; g.n_rows = N; g.n_rows_dev = n_rows_dev;
-  k_gather_p2p<<<ceil_div(g.n_octets, 8) + 1, 256, 0, (cudaStream_t)stream_>>>(g);
+  const int grid = ceil_div(g.n_octets, 8) + 1;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (dtype == MSCS_DTYPE_F32) k_gather_p2p<float><<<grid, 256, 0, st>>>(g);
+  else if (dtype == MSCS_DTYPE_BF16) k_gather_p2p<__nv_bfloat16><<<grid, 256, 0, st>>>(g);
+  else k_gather_p2p<__half><<<grid, 256, 0, st>>>(g);
+  MSCS_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int mscs_gather_rows_p2p(const void* feat, int C, const int32_t* pix, int N, const int32_t* n_rows_dev,
+                                    void* const* slabs, int world, int rank, size_t bf16_byte_off, float* anc_f32,
+                                    float* inv_norm, void* stream_, int dtype) {
+  MSCS_CHECK_ARG(feat && pix && anc_f32 && inv_norm, "null pointer argument");
+  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC && N >= 0, "unsupported shape (C %d, %d rows)", C, N);
+  MSCS_CHECK_ARG(rank >= 0 && rank < world && bf16_byte_off % 16 == 0, "bad rank / offset");
+  if (int rc = check_dtype(-1, dtype, feat, 1, "feat")) return rc;
+  GatherRowsP2P g{};
+  if (int rc = fill_peers(&g.bf16, slabs, world, bf16_byte_off)) return rc;
+  g.feat = feat; g.pix = pix; g.anc_f32 = anc_f32; g.inv_norm = inv_norm;
+  g.C = C; g.C_pad = (C + 63) / 64 * 64; g.rank = rank; g.n_rows = N; g.n_rows_dev = n_rows_dev;
+  const int grid = ceil_div((N + 255) / 256 * 256, 8);
+  if (grid == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream_;
+  if (dtype == MSCS_DTYPE_F32) k_gather_rows_p2p<float><<<grid, 256, 0, st>>>(g);
+  else if (dtype == MSCS_DTYPE_BF16) k_gather_rows_p2p<__nv_bfloat16><<<grid, 256, 0, st>>>(g);
+  else k_gather_rows_p2p<__half><<<grid, 256, 0, st>>>(g);
   MSCS_LAUNCH_CHECK();
   return 0;
 }

@@ -155,8 +155,10 @@ class DenseContrastiveLossV2_ms(_GraphReadout, nn.Module):
 
     ``comm`` (not a reference argument) switches on the POOLED cross-batch mode: the loss is then the
     reference loss of the concatenated batch of all ranks (one process per GPU, each passing its local
-    images); anchor rows are sharded over the ranks, the normalised key set is exchanged over NCCL.
-    Pass ``mscs_b200.TorchDistComm(process_group)``; every rank's CPU generator must be in the same state."""
+    images); anchor rows are sharded over the ranks, the normalised key set is exchanged over NVLink peer memory.
+    Pass ``mscs_b200.TorchDistComm(process_group)``.  With ``sampler='reference'`` every rank's CPU generator must be in
+    the same state; with ``sampler='philox'`` the generators need not agree, but every rank's module must have been
+    called the same number of times (the call index keys the stream)."""
 
     def __init__(self, config, comm=None):
         super().__init__()

@@ -427,16 +427,33 @@ int mscs_xchg_push(void* const* slabs, int world, const float* src, const int64_
                    const int64_t* float_off, const int32_t* len, int count, void* stream);
 /* K2 fused with the all-gather of the normalised key set: as mscs_gather_normalize_sectors, but every bf16 anchor row
  * is stored into the operand matrix at byte offset bf16_byte_off of EVERY rank's slab (same sorted row everywhere: the
- * plan is global); fp32 rows and inverse norms stay local.  Also zeroes the local padding rows [N, N_pad). */
-int mscs_gather_normalize_p2p(const float* feat, int n, int C, int plane, const int32_t* slot, int N,
+ * plan is global); fp32 rows and inverse norms stay local.  Also zeroes the local padding rows [N, N_pad).
+ * `dtype` (MSCS_DTYPE_*): element type of `feat` (aligned to its size); a half map gives the rows of its exact fp32
+ * widening bit for bit. */
+int mscs_gather_normalize_p2p(const void* feat, int n, int C, int plane, const int32_t* slot, int N,
                               const int32_t* n_rows_dev /* optional: N read on the device, e.g. &plan_dev[s].N */,
                               void* const* slabs, int world, int rank, size_t bf16_byte_off, float* anc_f32,
-                              float* inv_norm, void* stream);
+                              float* inv_norm, void* stream, int dtype);
 /* as mscs_scatter_sectors, with gradient row i read from rank (i / rows_per_rank)'s slab at dF_byte_off (the rank
- * that computed it: anchor rows are sharded in 128-aligned blocks of rows_per_rank rows) */
+ * that computed it: anchor rows are sharded in 128-aligned blocks of rows_per_rank rows).  `dtype` (MSCS_DTYPE_*):
+ * element type of the pre-zeroed NCHW `dfeat` (16-byte aligned); the gradient rows stay fp32. */
 int mscs_scatter_sectors_pull(void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank, int ldF,
                               const float* anc_f32, const float* inv_norm, const int32_t* slot, int n, int C, int plane,
-                              float* dfeat, void* stream);
+                              void* dfeat, void* stream, int dtype);
+/* Channels-last maps (memory order [n][h][w][C]), one scale per call:
+ *   mscs_gather_rows_p2p    as mscs_gather_rows_nhwc_batch for the rows with pix[r] >= 0 (bit-identical rows), with the
+ *                           bf16 row stored into every rank's slab as mscs_gather_normalize_p2p does.  Rows with
+ *                           pix[r] < 0 are not written (another rank stores them, concurrently); the local padding rows
+ *                           [N, N_pad) are zeroed.  N: the row count, or its upper bound when n_rows_dev is set.
+ *   mscs_scatter_rows_pull  as mscs_scatter_rows_nhwc_batch for the N rows, with gradient row i read as in
+ *                           mscs_scatter_sectors_pull; stores into the pre-zeroed channels-last `dfeat`.
+ * `dtype` (MSCS_DTYPE_*): element type of `feat` / `dfeat` (aligned to its size). */
+int mscs_gather_rows_p2p(const void* feat, int C, const int32_t* pix, int N, const int32_t* n_rows_dev,
+                         void* const* slabs, int world, int rank, size_t bf16_byte_off, float* anc_f32, float* inv_norm,
+                         void* stream, int dtype);
+int mscs_scatter_rows_pull(void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank, int ldF,
+                           const float* anc_f32, const float* inv_norm, const int32_t* pix, int N, int C, void* dfeat,
+                           void* stream, int dtype);
 
 #ifdef __cplusplus
 }

@@ -1,6 +1,11 @@
 """2+ GPU check of the pooled mode under torchrun: every rank compares its pooled loss / gradients
-with the single-process loss of the concatenated batch computed locally."""
-import os, sys
+with the single-process loss of the concatenated batch computed locally.
+
+  torchrun --nproc-per-node N tools/pooled_check.py [cfg5] [--dtype bf16] [--layout channels_last] [--sampler philox]
+
+--dtype / --layout / --sampler: element type and memory format of the feature maps (both runs get the same maps) and
+the sampler.  cfg5: also BASELINE config 5 (fp32 NCHW maps, reference sampler) against the fp64-oracle fixture."""
+import argparse, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
@@ -8,37 +13,48 @@ import torch.distributed as dist
 import mscs_b200
 from mscs_b200 import synth
 
+ap = argparse.ArgumentParser()
+ap.add_argument("mode", nargs="?", choices=["cfg5"])
+ap.add_argument("--dtype", choices=["fp32", "bf16", "fp16"], default="fp32")
+ap.add_argument("--layout", choices=["nchw", "channels_last"], default="nchw")
+ap.add_argument("--sampler", choices=["reference", "philox"], default="reference")
+args = ap.parse_args()
+dtype = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}[args.dtype]
+fmt = torch.channels_last if args.layout == "channels_last" else torch.contiguous_format
+
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
 dev = torch.device("cuda", local)
 dist.init_process_group("nccl", device_id=dev)
 cfg = dict(dataset="CITYSCAPES", experiment=1, temperature=0.1, scales=3, weights=[1.0, 0.7, 0.4],
            cross_scale_contrast=True, w_high_low=0.5, w_high_mid=0.25, min_views_per_class=5,
-           max_views_per_class=50, max_features_total=3000)
+           max_views_per_class=50, max_features_total=3000, sampler=args.sampler, sampler_seed=11)
 n = 2 * world
 labels = synth.synth_labels(n, 128, 256, 19, 7, 16, 0.05, 21)
 feats = synth.synth_features(n, 64, 128, 256, [4, 8, 16], 22)
 full = mscs_b200.DenseContrastiveLossV2_ms(dict(cfg))
-fg = [f.to(dev).requires_grad_(True) for f in feats]
+fg = [f.to(dev).to(dtype).contiguous(memory_format=fmt).requires_grad_(True) for f in feats]
 torch.manual_seed(5)
 loss_full = full(labels.to(dev), fg)
 loss_full.backward()
 nl = n // world
 mod = mscs_b200.DenseContrastiveLossV2_ms(dict(cfg), comm=mscs_b200.TorchDistComm())
-fl = [f[rank * nl:(rank + 1) * nl].to(dev).requires_grad_(True) for f in feats]
+fl = [f[rank * nl:(rank + 1) * nl].to(dev).to(dtype).contiguous(memory_format=fmt).requires_grad_(True) for f in feats]
 torch.manual_seed(5)
 loss = mod(labels[rank * nl:(rank + 1) * nl].to(dev), fl)
 loss.backward()
 torch.cuda.synchronize()
 ok = abs(float(loss) - float(loss_full)) < 2e-5 * abs(float(loss_full))
 for s in range(len(fl)):
-    g, w = fl[s].grad.cpu().numpy().ravel().astype(np.float64), fg[s].grad[rank * nl:(rank + 1) * nl].cpu().numpy().ravel().astype(np.float64)
+    ok = ok and fl[s].grad.dtype == dtype and fl[s].grad.stride() == fl[s].stride()
+    g, w = (x.float().cpu().numpy().ravel().astype(np.float64) for x in (fl[s].grad, fg[s].grad[rank * nl:(rank + 1) * nl]))
     cos = float(g @ w / np.sqrt((g @ g) * (w @ w)))
     ok = ok and cos > 0.99999 and np.array_equal(g != 0, w != 0)
     print(f"rank {rank} scale {s}: cosine {cos:.8f} max-abs {np.abs(g - w).max():.3e}", flush=True)
-print(f"rank {rank}: pooled loss {float(loss):.6f} single-process {float(loss_full):.6f} -> {'OK' if ok else 'MISMATCH'}", flush=True)
+print(f"rank {rank} ({args.dtype}, {args.layout}, sampler {args.sampler}): pooled loss {float(loss):.6f} single-process "
+      f"{float(loss_full):.6f} -> {'OK' if ok else 'MISMATCH'}", flush=True)
 
-if len(sys.argv) > 1 and sys.argv[1] == "cfg5":
+if args.mode == "cfg5":
     # BASELINE config 5 over real ranks against the fp64-oracle fixture (tests/golden/cfg5.npz): loss, term losses and
     # the recorded gradient rows of the pixels this rank owns
     import json
