@@ -105,8 +105,6 @@ _SIGNATURES = {
     "mscs_philox_stream_dev": (C.c_int, [C.c_uint64, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]),
     "mscs_sample_select": (C.c_int, [C.POINTER(SampleCfg), C.POINTER(ScalePlan), C.c_void_p, C.c_void_p,
                                      _PTRS, _PTRS, _PTRS, _PTRS, _PTRS, _PTRS, C.c_void_p]),
-    "mscs_gather_normalize_sectors": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,
-                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mscs_mt19937_advance_host": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.c_uint64]),
     "mscs_gather_normalize": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
                                         C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -123,7 +121,6 @@ _SIGNATURES = {
     "mscs_debug_sim_forward_simt": (C.c_int, [C.POINTER(SimJob), _PTRS, C.c_void_p]),
     "mscs_debug_sim_backward_simt": (C.c_int, [C.POINTER(SimJob), _PTRS, C.c_void_p, _PTRS, C.POINTER(C.c_int32),
                                                C.c_void_p]),
-    "mscs_slot_map": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "mscs_scatter_grad": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                     C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p]),
     "mscs_label_pass": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

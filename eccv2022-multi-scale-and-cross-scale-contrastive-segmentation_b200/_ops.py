@@ -1350,14 +1350,21 @@ def _run_forward_general(sp, labels, feats32, needs):
                    "mscs_sample_select")
     samples = _samples_from_plan(plan, islab, sp.ioff, A)
     with _timed("gather"):
+        # the scales with a slot map in one launch, which reads their row counts from the device plan records
+        sect = [s for s in range(S) if slots[s] is not None]
+        if sect:
+            items = (_lib.GatherItem * len(sect))()
+            for it, s in zip(items, sect):
+                n, Cc, h, w = sp.feat_shapes[s]
+                it.feat, it.n, it.C, it.plane, it.slot = feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr()
+                it.n_rows_dev = plan_dev.data_ptr() + s * C.sizeof(_lib.ScalePlan) + 8      # &plan_dev[s].N
+                it.anc_bf16, it.anc_f32 = bbase + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0]
+                it.inv_norm, it.dtype = fbase + 4 * sp.foff[s][1], _lib.DTYPE_F32
+            _lib.check(lib.mscs_gather_normalize_sectors_batch(items, len(sect), st),
+                       "mscs_gather_normalize_sectors_batch")
         for s in range(S):
-            n, Cc, h, w = sp.feat_shapes[s]
-            if slots[s] is not None:
-                _lib.check(lib.mscs_gather_normalize_sectors(feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(),
-                                                             samples[s].N, bbase + 2 * sp.boff[s],
-                                                             fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1], st),
-                           "mscs_gather_normalize_sectors")
-            else:
+            if slots[s] is None:
+                n, Cc, h, w = sp.feat_shapes[s]
                 _lib.check(lib.mscs_gather_normalize(feats32[s].data_ptr(), n, Cc, h * w, samples[s].ptr(2),
                                                      samples[s].N, bbase + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0],
                                                      fbase + 4 * sp.foff[s][1], st), "mscs_gather_normalize")

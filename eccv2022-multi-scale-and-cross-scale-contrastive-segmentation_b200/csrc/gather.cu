@@ -5,11 +5,9 @@
 //             a dense zero (n,C,h,w) gradient at the sampled pixels.
 // HBM-bound byte movers: NCHW means one anchor is C scalars `plane` floats apart (one 32 B
 // sector per useful 4 B), so one warp owns one anchor and keeps 8 independent loads in flight.
-#include "common.cuh"
+#include "rows.cuh"
 
 namespace mscs {
-
-constexpr int kMaxC = 256;
 
 __global__ void __launch_bounds__(256)
 k_gather_normalize(const float* __restrict__ feat, int C, int C_pad, int plane, const int* __restrict__ pix,
@@ -32,24 +30,14 @@ k_gather_normalize(const float* __restrict__ feat, int C, int C_pad, int plane, 
   const int b = gp / plane, p = gp - b * plane;
   const float* src = feat + ((size_t)b * C) * plane + p;
   float v[kMaxC / 32];
-  float ss = 0.f;
 #pragma unroll
-  for (int j = 0; j < kMaxC / 32; ++j) {
-    int c = lane + 32 * j;
-    v[j] = (c < C) ? __ldg(src + (size_t)c * plane) : 0.f;
+  for (int q = 0; q < kMaxC / 32; ++q) {
+    const int c = lane + 32 * q;
+    v[q] = (c < C) ? __ldg(src + (size_t)c * plane) : 0.f;
   }
-#pragma unroll
-  for (int j = 0; j < kMaxC / 32; ++j) ss = fmaf(v[j], v[j], ss);
-  ss = warp_sum(ss);
-  const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
+  const float inv = inv_norm_of(v);
   if (lane == 0) inv_norm[row] = inv;
-#pragma unroll
-  for (int j = 0; j < kMaxC / 32; ++j) {
-    int c = lane + 32 * j;
-    float f = v[j] * inv;
-    if (c < C) anc_f32[(size_t)row * C + c] = f;
-    if (c < C_pad) orow[c] = __float2bfloat16(c < C ? f : 0.f);
-  }
+  store_unit_row(v, inv, C, C_pad, anc_f32 + (size_t)row * C, orow);
 }
 
 __global__ void __launch_bounds__(256)
@@ -59,28 +47,16 @@ k_scatter_grad(const float* __restrict__ dF, int ldF, const float* __restrict__ 
   const int lane = threadIdx.x & 31;
   const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= N) return;
-  const float* g = dF + (size_t)row * ldF;
-  const float* f = anc_f32 + (size_t)row * C;
-  float gv[kMaxC / 32], fv[kMaxC / 32];
-  float dot = 0.f;
-#pragma unroll
-  for (int j = 0; j < kMaxC / 32; ++j) {
-    int c = lane + 32 * j;
-    gv[j] = (c < C) ? g[c] : 0.f;
-    fv[j] = (c < C) ? f[c] : 0.f;
-    dot = fmaf(gv[j], fv[j], dot);
-  }
-  dot = warp_sum(dot);
-  const float inv = inv_norm[row];
-  const bool clamped = inv >= 1e12f;        // ||x|| <= eps: F.normalize divides by the constant eps
+  float dx[kMaxC / 32];
+  dx_row(dF + (size_t)row * ldF, anc_f32 + (size_t)row * C, inv_norm, row, C, dx);
   const int gp = pix[row];
   if (gp < 0) return;
   const int b = gp / plane, p = gp - b * plane;
   float* dst = dfeat + ((size_t)b * C) * plane + p;
 #pragma unroll
-  for (int j = 0; j < kMaxC / 32; ++j) {
-    int c = lane + 32 * j;
-    if (c < C) dst[(size_t)c * plane] = (clamped ? gv[j] : (gv[j] - fv[j] * dot)) * inv;
+  for (int q = 0; q < kMaxC / 32; ++q) {
+    const int c = lane + 32 * q;
+    if (c < C) dst[(size_t)c * plane] = dx[q];
   }
 }
 
@@ -115,14 +91,11 @@ gather_sectors_body(int block, int nblocks, const T* __restrict__ feat, int C, i
     const int row = __shfl_sync(0xffffffffu, s_mine, j);
     const T* src = src0 + j;
     float v[kMaxC / 32];
-    float ss = 0.f;
 #pragma unroll
     for (int q = 0; q < kMaxC / 32; ++q) {
       const int c = lane + 32 * q;
       v[q] = (c < C) ? to_f32(__ldg(src + (size_t)c * plane)) : 0.f;
     }
-#pragma unroll
-    for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q], v[q], ss);
     if (anc_bf16 == nullptr) {      // raw mode (projector-tail path): the sampled rows as they are, no normalisation
 #pragma unroll
       for (int q = 0; q < kMaxC / 32; ++q) {
@@ -131,27 +104,10 @@ gather_sectors_body(int block, int nblocks, const T* __restrict__ feat, int C, i
       }
       continue;
     }
-    ss = warp_sum(ss);
-    const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
+    const float inv = inv_norm_of(v);
     if (lane == 0) inv_norm[row] = inv;
-    __nv_bfloat16* orow = anc_bf16 + (size_t)row * C_pad;
-#pragma unroll
-    for (int q = 0; q < kMaxC / 32; ++q) {
-      const int c = lane + 32 * q;
-      const float f = v[q] * inv;
-      if (c < C) anc_f32[(size_t)row * C + c] = f;
-      if (c < C_pad) orow[c] = __float2bfloat16(c < C ? f : 0.f);
-    }
+    store_unit_row(v, inv, C, C_pad, anc_f32 + (size_t)row * C, anc_bf16 + (size_t)row * C_pad);
   }
-}
-
-__global__ void __launch_bounds__(256)
-k_gather_sectors(const float* __restrict__ feat, int C, int C_pad, int plane, const int* __restrict__ slot,
-                 int n_octets, __nv_bfloat16* __restrict__ anc_bf16, float* __restrict__ anc_f32,
-                 float* __restrict__ inv_norm, const int* __restrict__ n_rows_dev) {
-  pdl_trigger();
-  gather_sectors_body<float>(blockIdx.x, gridDim.x, feat, C, C_pad, plane, slot, n_octets, anc_bf16, anc_f32, inv_norm,
-                      n_rows_dev);
 }
 
 // all scales of a call in ONE launch (the per-scale launches of the small scales do not fill the GPU and each
@@ -166,8 +122,7 @@ struct GatherBatch {
 template <typename T>
 __global__ void __launch_bounds__(256) k_gather_sectors_batch(const __grid_constant__ GatherBatch g) {
   pdl_trigger();      // the next kernel of the forward (k_row_ranges) is launched programmatically, see common.cuh
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int s = batch_item(g.block0, g.count);
   gather_sectors_body<T>(blockIdx.x - g.block0[s], g.block0[s + 1] - g.block0[s], static_cast<const T*>(g.feat[s]), g.C[s],
                       (g.C[s] + 63) / 64 * 64, g.plane[s], g.slot[s], g.n_oct[s], g.bf16[s], g.f32[s], g.inv[s],
                       g.n_rows_dev[s]);
@@ -177,16 +132,9 @@ __global__ void __launch_bounds__(256) k_gather_sectors_batch(const __grid_const
 // sampled rows only, so the row count is not needed; rows the call does not sample are not touched.
 template <typename T>
 __global__ void __launch_bounds__(256) k_gather_raw_batch(const __grid_constant__ GatherBatch g) {
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int s = batch_item(g.block0, g.count);
   gather_sectors_body<T>(blockIdx.x - g.block0[s], g.block0[s + 1] - g.block0[s], static_cast<const T*>(g.feat[s]), g.C[s],
                          0, g.plane[s], g.slot[s], g.n_oct[s], nullptr, g.f32[s], nullptr, nullptr);
-}
-
-// slot map: slot[image*plane + pixel] = sorted anchor row sampled there, or -1
-__global__ void k_slot_map(const int* __restrict__ pix, int N, int* __restrict__ slot) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < N && pix[i] >= 0) slot[pix[i]] = i;      // negative: row owned by another rank (pooled mode)
 }
 
 // Sector writer: the dense gradient is already zero; one warp per 8-pixel octet (= one 32-byte
@@ -216,20 +164,7 @@ scatter_sectors_body(const float* __restrict__ dF, int ldF, const float* __restr
     const int row = __shfl_sync(0xffffffffu, s_mine, j);
     if (row >= 0) {                                   // warp-uniform
       const float* g = (pull ? pull->p[row / pull->rows_per_rank] : dF) + (size_t)row * ldF;
-      const float* f = anc_f32 + (size_t)row * C;
-      float gv[kMaxC / 32], fv[kMaxC / 32], dot = 0.f;
-#pragma unroll
-      for (int q = 0; q < kMaxC / 32; ++q) {
-        const int c = lane + 32 * q;
-        gv[q] = (c < C) ? g[c] : 0.f;
-        fv[q] = (c < C) ? f[c] : 0.f;
-        dot = fmaf(gv[q], fv[q], dot);
-      }
-      dot = warp_sum(dot);
-      const float inv = inv_norm[row];
-      const bool clamped = inv >= 1e12f;
-#pragma unroll
-      for (int q = 0; q < kMaxC / 32; ++q) dx[j][q] = (clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv;
+      dx_row(g, anc_f32 + (size_t)row * C, inv_norm, row, C, dx[j]);
     } else {
 #pragma unroll
       for (int q = 0; q < kMaxC / 32; ++q) dx[j][q] = 0.f;
@@ -272,24 +207,13 @@ k_scatter_rows_pull(const __grid_constant__ PullRows pull, int ldF, const float*
   if (row >= N) return;
   const int gp = pix[row];
   if (gp < 0) return;
-  const float* gr = pull.p[row / pull.rows_per_rank] + (size_t)row * ldF;
-  const float* f = anc_f32 + (size_t)row * C;
-  float gv[kMaxC / 32], fv[kMaxC / 32], dot = 0.f;
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) {
-    const int c = lane + 32 * q;
-    gv[q] = (c < C) ? gr[c] : 0.f;
-    fv[q] = (c < C) ? f[c] : 0.f;
-    dot = fmaf(gv[q], fv[q], dot);
-  }
-  dot = warp_sum(dot);
-  const float inv = inv_norm[row];
-  const bool clamped = inv >= 1e12f;        // ||x|| <= eps: F.normalize divides by the constant eps
+  float dx[kMaxC / 32];
+  dx_row(pull.p[row / pull.rows_per_rank] + (size_t)row * ldF, anc_f32 + (size_t)row * C, inv_norm, row, C, dx);
   T* dst = dfeat + (size_t)gp * C;
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
-    if (c < C) dst[c] = from_f32<T>((clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv);
+    if (c < C) dst[c] = from_f32<T>(dx[q]);
   }
 }
 
@@ -310,30 +234,19 @@ struct DenseBatch {
 };
 
 __global__ void __launch_bounds__(256) k_dx_rows(const __grid_constant__ DenseBatch g) {
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.rowblk0[s + 1]) ++s;
+  const int s = batch_item(g.rowblk0, g.count);
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.rowblk0[s]) * 8 + (threadIdx.x >> 5);
   // rows[s] sizes the grid; with a device-resident count it is an upper bound and the rows beyond the count are stale
   if (row >= g.rows[s] || (g.n_rows_dev[s] && row >= *g.n_rows_dev[s])) return;
   const int C = g.C[s];
   float* gr = g.dF[s] + (size_t)row * g.ldF[s];
-  const float* f = g.f32[s] + (size_t)row * C;
-  float gv[kMaxC / 32], fv[kMaxC / 32], dot = 0.f;
+  float dx[kMaxC / 32];
+  dx_row(gr, g.f32[s] + (size_t)row * C, g.inv[s], row, C, dx);
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
-    gv[q] = (c < C) ? gr[c] : 0.f;
-    fv[q] = (c < C) ? f[c] : 0.f;
-    dot = fmaf(gv[q], fv[q], dot);
-  }
-  dot = warp_sum(dot);
-  const float inv = g.inv[s][row];
-  const bool clamped = inv >= 1e12f;        // ||x|| <= eps: F.normalize divides by the constant eps
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) {
-    const int c = lane + 32 * q;
-    if (c < C) gr[c] = (clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv;
+    if (c < C) gr[c] = dx[q];
   }
 }
 
@@ -355,8 +268,7 @@ struct RowsBatch {
 template <typename T>
 __global__ void __launch_bounds__(256) k_gather_rows_nhwc(const __grid_constant__ RowsBatch g) {
   pdl_trigger();
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int s = batch_item(g.block0, g.count);
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.block0[s]) * 8 + (threadIdx.x >> 5);
   const int N = g.n_rows_dev[s] ? *g.n_rows_dev[s] : g.rows[s], N_pad = (N + 255) / 256 * 256;
@@ -370,55 +282,33 @@ __global__ void __launch_bounds__(256) k_gather_rows_nhwc(const __grid_constant_
   }
   const T* src = static_cast<const T*>(g.feat[s]) + (size_t)gp * C;
   float v[kMaxC / 32];
-  float ss = 0.f;
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
     v[q] = (c < C) ? to_f32(__ldg(src + c)) : 0.f;
   }
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q], v[q], ss);
-  ss = warp_sum(ss);
-  const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
+  const float inv = inv_norm_of(v);
   if (lane == 0) g.inv[s][row] = inv;
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) {
-    const int c = lane + 32 * q;
-    const float f = v[q] * inv;
-    if (c < C) g.f32[s][(size_t)row * C + c] = f;
-    if (c < C_pad) orow[c] = __float2bfloat16(c < C ? f : 0.f);
-  }
+  store_unit_row(v, inv, C, C_pad, g.f32[s] + (size_t)row * C, orow);
 }
 
 // normalisation backward + row store into the (pre-zeroed) channels-last dense gradient
 template <typename T>
 __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant__ RowsBatch g) {
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int s = batch_item(g.block0, g.count);
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.block0[s]) * 8 + (threadIdx.x >> 5);
   if (row >= g.rows[s] || (g.n_rows_dev[s] && row >= *g.n_rows_dev[s])) return;      // (as k_dx_rows)
   const int gp = g.pix[s][row];
   if (gp < 0) return;
   const int C = g.C[s];
-  const float* gr = g.dF[s] + (size_t)row * g.ldF[s];
-  const float* f = g.f32[s] + (size_t)row * C;
-  float gv[kMaxC / 32], fv[kMaxC / 32], dot = 0.f;
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) {
-    const int c = lane + 32 * q;
-    gv[q] = (c < C) ? gr[c] : 0.f;
-    fv[q] = (c < C) ? f[c] : 0.f;
-    dot = fmaf(gv[q], fv[q], dot);
-  }
-  dot = warp_sum(dot);
-  const float inv = g.inv[s][row];
-  const bool clamped = inv >= 1e12f;        // ||x|| <= eps: F.normalize divides by the constant eps
+  float dx[kMaxC / 32];
+  dx_row(g.dF[s] + (size_t)row * g.ldF[s], g.f32[s] + (size_t)row * C, g.inv[s], row, C, dx);
   T* dst = static_cast<T*>(g.dfeat[s]) + (size_t)gp * C;
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
-    if (c < C) dst[c] = from_f32<T>((clamped ? gv[q] : (gv[q] - fv[q] * dot)) * inv);
+    if (c < C) dst[c] = from_f32<T>(dx[q]);
   }
 }
 
@@ -426,8 +316,7 @@ __global__ void __launch_bounds__(256) k_scatter_rows_nhwc(const __grid_constant
 //   gather: rows[row][:] = feat[pix[row]][:]  (fp32 rows)      store: dfeat[pix[row]][:] = rows[row][:]  (map's type)
 template <typename T, bool GATHER>
 __global__ void __launch_bounds__(256) k_rows_raw_nhwc(const __grid_constant__ RowsBatch g) {
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int s = batch_item(g.block0, g.count);
   const int lane = threadIdx.x & 31;
   const int row = ((int)blockIdx.x - g.block0[s]) * 8 + (threadIdx.x >> 5);
   if (row >= g.rows[s] || (g.n_rows_dev[s] && row >= *g.n_rows_dev[s])) return;
@@ -460,8 +349,7 @@ struct DenseStream {
 template <typename T>
 __global__ void __launch_bounds__(128) k_dense_stream(const __grid_constant__ DenseStream g) {
   constexpr int P = 16 / sizeof(T);      // pixels per thread: one 16-byte store per channel plane
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.blk0[s + 1]) ++s;
+  const int s = batch_item(g.blk0, g.count);
   const int lin = (((int)blockIdx.x - g.blk0[s]) * 128 + (int)threadIdx.x) * P;
   if (lin >= g.npix[s]) return;
   const int plane = g.plane[s], C = g.C[s], ld = g.ld[s];
@@ -490,32 +378,6 @@ __global__ void __launch_bounds__(128) k_dense_stream(const __grid_constant__ De
 }  // namespace mscs
 
 using namespace mscs;
-
-extern "C" int mscs_gather_normalize_sectors(const float* feat, int n, int C, int plane, const int32_t* slot, int N,
-                                             void* anc_bf16, float* anc_f32, float* inv_norm, void* stream_) {
-  MSCS_CHECK_ARG(feat && slot && anc_bf16 && anc_f32 && inv_norm, "null pointer argument");
-  MSCS_CHECK_ARG(C >= 1 && C <= kMaxC, "C=%d unsupported (1..%d)", C, kMaxC);
-  MSCS_CHECK_ARG(n >= 1 && plane >= 8 && plane % 8 == 0 && N >= 1, "bad sizes (plane must be a multiple of 8)");
-  cudaStream_t st = (cudaStream_t)stream_;
-  const int C_pad = (C + 63) / 64 * 64, N_pad = (N + 255) / 256 * 256;
-  if (N_pad > N)      // zero padding rows of the operand matrix (TMA tiles read them)
-    MSCS_CUDA(cudaMemsetAsync((__nv_bfloat16*)anc_bf16 + (size_t)N * C_pad, 0,
-                              sizeof(__nv_bfloat16) * (size_t)(N_pad - N) * C_pad, st));
-  const int n_oct = n * (plane / 8);
-  k_gather_sectors<<<ceil_div(n_oct, 8), 256, 0, st>>>(feat, C, C_pad, plane, slot, n_oct, (__nv_bfloat16*)anc_bf16,
-                                                       anc_f32, inv_norm, nullptr);
-  MSCS_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream_) {
-  MSCS_CHECK_ARG(pix && slot && N >= 1 && n_pixels >= 1, "bad arguments");
-  cudaStream_t st = (cudaStream_t)stream_;
-  MSCS_CUDA(cudaMemsetAsync(slot, 0xff, sizeof(int) * (size_t)n_pixels, st));
-  k_slot_map<<<ceil_div(N, 256), 256, 0, st>>>(pix, N, slot);
-  MSCS_LAUNCH_CHECK();
-  return 0;
-}
 
 // pooled mode: the gradient rows of every rank's slab at dF_byte_off (row i: rank i / rows_per_rank)
 static int pull_rows(PullRows* pull, void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank) {
@@ -641,8 +503,7 @@ struct ScatterBatch {
   int count;
 };
 __global__ void __launch_bounds__(256) k_scatter_sectors_batch(const __grid_constant__ ScatterBatch g) {
-  int s = 0;
-  while (s + 1 < g.count && (int)blockIdx.x >= g.block0[s + 1]) ++s;
+  const int s = batch_item(g.block0, g.count);
   scatter_sectors_body<float>(g.dF[s], g.ldF[s], g.f32[s], g.inv[s], g.slot[s], g.n_oct[s], g.C[s], g.plane[s],
                               g.dfeat[s], g.block0[s]);
 }

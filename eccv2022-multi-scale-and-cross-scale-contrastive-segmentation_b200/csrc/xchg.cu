@@ -18,11 +18,9 @@
 //   scatter (pull)      gather.cu: the scatter reads every gradient row from the rank that computed it.
 // Slabs are double-buffered by step parity, so a rank that runs ahead never writes into a buffer a slower rank is
 // still reading (DESIGN.md section 6 has the argument).
-#include "common.cuh"
+#include "rows.cuh"
 
 namespace mscs {
-
-constexpr int kMaxC = 256;
 
 struct PeerPtrs { void* p[MSCS_MAX_RANKS]; int n; };
 
@@ -72,8 +70,8 @@ __global__ void __launch_bounds__(256) k_push_ranges(const __grid_constant__ Pus
   }
 }
 
-// K2 + all-gather.  One warp per 8-pixel octet of the slot map (address order, like k_gather_sectors); lane l owns
-// channels [8l, 8l+8): eight strided sector reads, then ONE 16-byte store per destination matrix.
+// K2 + all-gather.  One warp per 8-pixel octet of the slot map (address order, like k_gather_sectors_batch); lane l
+// owns channels [8l, 8l+8): eight strided sector reads, then ONE 16-byte store per destination matrix.
 struct GatherP2P {
   const void* feat; const int* slot; float* anc_f32; float* inv_norm;
   PeerPtrs bf16;            // the operand matrix of this scale in every rank's slab (same sorted row index everywhere)
@@ -108,13 +106,9 @@ __global__ void __launch_bounds__(256) k_gather_p2p(const __grid_constant__ Gath
     const int row = __shfl_sync(0xffffffffu, s_mine, j);
     const T* src = src0 + j;
     float v[8];
-    float ss = 0.f;
 #pragma unroll
     for (int q = 0; q < 8; ++q) v[q] = (c0 + q < C) ? to_f32(__ldg(src + (size_t)(c0 + q) * plane)) : 0.f;
-#pragma unroll
-    for (int q = 0; q < 8; ++q) ss = fmaf(v[q], v[q], ss);
-    ss = warp_sum(ss);
-    const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
+    const float inv = inv_norm_of(v);
     if (lane == 0) g.inv_norm[row] = inv;
     uint32_t pk[4];
 #pragma unroll
@@ -161,28 +155,16 @@ __global__ void __launch_bounds__(256) k_gather_rows_p2p(const __grid_constant__
   if (gp < 0) return;
   const T* src = static_cast<const T*>(g.feat) + (size_t)gp * C;
   float v[kMaxC / 32];
-  float ss = 0.f;
 #pragma unroll
   for (int q = 0; q < kMaxC / 32; ++q) {
     const int c = lane + 32 * q;
     v[q] = (c < C) ? to_f32(__ldg(src + c)) : 0.f;
   }
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) ss = fmaf(v[q], v[q], ss);
-  ss = warp_sum(ss);
-  const float inv = 1.f / fmaxf(sqrtf(ss), 1e-12f);
+  const float inv = inv_norm_of(v);
   if (lane == 0) g.inv_norm[row] = inv;
-#pragma unroll
-  for (int q = 0; q < kMaxC / 32; ++q) {
-    const int c = lane + 32 * q;
-    const float f = v[q] * inv;
-    if (c < C) g.anc_f32[(size_t)row * C + c] = f;
-    if (c < C_pad) {
-      const __nv_bfloat16 h = __float2bfloat16(c < C ? f : 0.f);
-      for (int r = 0; r < g.bf16.n; ++r)
-        reinterpret_cast<__nv_bfloat16*>(g.bf16.p[r])[(size_t)row * C_pad + c] = h;
-    }
-  }
+  store_unit_row(v, inv, C, C_pad, g.anc_f32 + (size_t)row * C, [&](int c, __nv_bfloat16 h) {
+    for (int r = 0; r < g.bf16.n; ++r) reinterpret_cast<__nv_bfloat16*>(g.bf16.p[r])[(size_t)row * C_pad + c] = h;
+  });
 }
 
 }  // namespace mscs

@@ -179,14 +179,12 @@ int mscs_mt19937_advance_host(uint32_t* mt_state_host, int* mt_pos, uint64_t k);
  * ------------------------------------------------------------------------------------- */
 int mscs_gather_normalize(const float* feat, int n, int C, int plane, const int32_t* pix, int N,
                           void* anc_bf16, float* anc_f32, float* inv_norm, void* stream);
-/* same result, driven by the slot map (pixel -> row) in ADDRESS order, which keeps the strided sector
- * reads inside open DRAM pages; needs plane % 8 == 0 */
-int mscs_gather_normalize_sectors(const float* feat, int n, int C, int plane, const int32_t* slot, int N,
-                                  void* anc_bf16, float* anc_f32, float* inv_norm, void* stream);
-/* every scale of a call in ONE launch, device-driven: the row count is read from device memory (`n_rows_dev`, e.g.
- * &plan_dev[s].N) and the padding rows are zeroed inside the call.  `dtype` (MSCS_DTYPE_*, last member: a
- * zero-initialised item is fp32) is the element type of `feat`; scales of different dtypes may be mixed (one launch
- * per dtype present).  The outputs are the same for a half map and for its exact fp32 widening. */
+/* same result, driven by the slot map (pixel -> row) in ADDRESS order, which keeps the strided sector reads inside
+ * open DRAM pages; needs plane % 8 == 0.  Every scale of a call in ONE launch, device-driven: the row count is read
+ * from device memory (`n_rows_dev`, e.g. &plan_dev[s].N) and the padding rows are zeroed inside the call.  `dtype`
+ * (MSCS_DTYPE_*, last member: a zero-initialised item is fp32) is the element type of `feat`; scales of different
+ * dtypes may be mixed (one launch per dtype present).  The outputs are the same for a half map and for its exact fp32
+ * widening. */
 typedef struct {
   const void* feat; int32_t n, C, plane; const int32_t* slot; const int32_t* n_rows_dev;
   void* anc_bf16; float* anc_f32; float* inv_norm;
@@ -279,12 +277,10 @@ int mscs_scatter_grad(const float* dF, int ldF, const float* anc_f32, const floa
                       const int32_t* pix, int N, int n, int C, int plane, float* dfeat,
                       int zero_fill, void* stream);
 
-/* Scatter when the caller has ALREADY zero-filled dfeat (the host side does that
- * on a side stream while the tensor kernels run) and plane % 8 == 0:
- *   mscs_slot_map              slot[image*plane + pixel] = sorted anchor row sampled there, else -1
- *   mscs_scatter_sectors_batch rewrites, with full 32-byte sector stores, only the sectors of dfeat that
- *                              hold a sampled pixel (same maths as mscs_scatter_grad). */
-int mscs_slot_map(const int32_t* pix, int N, int n_pixels, int32_t* slot, void* stream);
+/* Scatter when the caller has ALREADY zero-filled dfeat (the host side does that on a side stream while the tensor
+ * kernels run) and plane % 8 == 0: mscs_scatter_sectors_batch rewrites, with full 32-byte sector stores, only the
+ * sectors of dfeat that hold a sampled pixel (same maths as mscs_scatter_grad), driven by the slot maps
+ * (slot[image*plane + pixel] = sorted anchor row sampled there, else -1) that the selection fills. */
 /* every scale of a call in ONE launch.  `dtype` (MSCS_DTYPE_*): element type of `dfeat`; the gradient rows dF stay
  * fp32.  mscs_scatter_sectors_batch takes fp32 items only.  `n_rows_dev` (last member, mscs_scatter_dense_batch only):
  * NULL = `rows[s]` is the row count; else the count is read from device memory (e.g. &plan_dev[s].N) and `rows[s]` is
@@ -425,9 +421,9 @@ int mscs_xchg_barrier(void* const* slabs, int world, int rank, uint32_t epoch, d
  * of its anchor rows, accumulated by the sweeps) to float offset float_off[j] of EVERY rank's slab, its own included */
 int mscs_xchg_push(void* const* slabs, int world, const float* src, const int64_t* src_float_off,
                    const int64_t* float_off, const int32_t* len, int count, void* stream);
-/* K2 fused with the all-gather of the normalised key set: as mscs_gather_normalize_sectors, but every bf16 anchor row
- * is stored into the operand matrix at byte offset bf16_byte_off of EVERY rank's slab (same sorted row everywhere: the
- * plan is global); fp32 rows and inverse norms stay local.  Also zeroes the local padding rows [N, N_pad).
+/* K2 fused with the all-gather of the normalised key set: as mscs_gather_normalize_sectors_batch for one scale, but
+ * every bf16 anchor row is stored into the operand matrix at byte offset bf16_byte_off of EVERY rank's slab (same
+ * sorted row everywhere: the plan is global); fp32 rows and inverse norms stay local.  Also zeroes the local padding rows [N, N_pad).
  * `dtype` (MSCS_DTYPE_*): element type of `feat` (aligned to its size); a half map gives the rows of its exact fp32
  * widening bit for bit. */
 int mscs_gather_normalize_p2p(const void* feat, int n, int C, int plane, const int32_t* slot, int N,

@@ -446,6 +446,6 @@ def test_pooled_entry_points_keep_rank_checks():
     assert b"world" in lib.mscs_last_error()
 
 
-def test_version_is_0_6_0():
+def test_version_is_0_7_0():
     import mscs_b200
-    assert mscs_b200.load().mscs_version().startswith(b"mscs 0.6.0 ")
+    assert mscs_b200.load().mscs_version().startswith(b"mscs 0.7.0 ")
