@@ -592,6 +592,8 @@ extern "C" int mscs_scatter_dense_batch(const mscs_scatter_item* items, const in
     if (int rc = check_dtype(s, it.dtype, it.dfeat, 16, "dfeat")) return rc;
     MSCS_CHECK_ARG(it.dtype == MSCS_DTYPE_F32 || it.plane % 8 == 0,
                    "item %d: half gradients need a plane that is a multiple of 8 pixels (plane %d)", s, it.plane);
+    // k_dense_stream reads a thread's slot entries as int4
+    MSCS_CHECK_ARG((uintptr_t)it.slot % 16 == 0, "item %d: the slot map must be 16-byte aligned", s);
     g.dF[s] = const_cast<float*>(it.dF); g.f32[s] = it.anc_f32; g.inv[s] = it.inv_norm; g.slot[s] = it.slot;
     g.ldF[s] = it.ldF; g.C[s] = it.C; g.plane[s] = it.plane; g.n[s] = it.n; g.rows[s] = raw ? 0 : rows[s];
     g.n_rows_dev[s] = it.n_rows_dev;

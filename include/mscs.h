@@ -284,7 +284,8 @@ int mscs_scatter_grad(const float* dF, int ldF, const float* anc_f32, const floa
 /* every scale of a call in ONE launch.  `dtype` (MSCS_DTYPE_*): element type of `dfeat`; the gradient rows dF stay
  * fp32.  mscs_scatter_sectors_batch takes fp32 items only.  `n_rows_dev` (last member, mscs_scatter_dense_batch only):
  * NULL = `rows[s]` is the row count; else the count is read from device memory (e.g. &plan_dev[s].N) and `rows[s]` is
- * its upper bound.  A zero-initialised tail is an fp32 item with a host count. */
+ * its upper bound.  A zero-initialised tail is an fp32 item with a host count.  `slot` (n * plane entries): 16-byte
+ * aligned for mscs_scatter_dense_batch, which reads it 4 entries at a time (the call returns < 0 otherwise). */
 typedef struct {
   const float* dF; int32_t ldF; const float* anc_f32; const float* inv_norm; const int32_t* slot;
   int32_t n, C, plane; void* dfeat;
@@ -308,7 +309,7 @@ int mscs_scatter_rows_nhwc_batch(const mscs_rows_item* items, int count, void* s
 /* Dense gradients of every scale written in ONE streaming pass, zeros included (no pre-zeroed buffer needed):
  * dF rows are first turned into dx rows IN PLACE (rows[s] rows of item s), then every 16 bytes of every dfeat are
  * written once (4 fp32 or 8 half pixels of a channel plane per store).  plane must be a multiple of 4 (fp32) or 8
- * (bf16 / fp16), dfeat 16-byte aligned. */
+ * (bf16 / fp16), dfeat and slot 16-byte aligned, n * C * plane below 2^32. */
 int mscs_scatter_dense_batch(const mscs_scatter_item* items, const int32_t* rows, int count, void* stream);
 
 /* ---------------------------------------------------------------------------------------
