@@ -147,6 +147,8 @@ _SIGNATURES = {
                                        C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "mscs_scatter_rows_pull": (C.c_int, [_PTRS, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "mscs_local_rows_batch": (C.c_int, [_PTRS, _PTRS, C.POINTER(C.c_int32), _PTRS, _PTRS, _PTRS, C.c_void_p, C.c_int,
+                                        C.c_void_p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -1122,11 +1122,11 @@ class _PooledState(_HostState):
     and write the maps in.  ``dF_fresh``: as in _DeviceState, for this parity's gradient rows in the exchange slab."""
 
     def __init__(self, sp, job, samples, gradbufs, slots, keep, fslab, scalars, total, comm, xs, par, exchange_info,
-                 io_dtypes):
+                 io_dtypes, dF_fresh):
         super().__init__(sp, job, samples, gradbufs, slots, keep, None, fslab, scalars, total)
         self.comm, self.xs, self.par, self.exchange_info = comm, xs, par, exchange_info
         self.io_dtypes = io_dtypes
-        self.dF_fresh = gradbufs is not None
+        self.dF_fresh = dF_fresh
         self.backward = _run_backward_pooled
 
 
@@ -1378,7 +1378,7 @@ def _run_forward_general(sp, labels, feats32, needs):
                       fslab, misc[sp.out_off:sp.out_off + nt + 2], total_t)
 
 
-def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
+def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None, tail=None):
     """POOLED cross-batch mode (one process per GPU, each with its own images): the reference loss of the concatenated
     batch of all ranks.  Control plane over NCCL (class histograms: a few KB); data plane by the library's own kernels
     over NVLink peer memory (csrc/xchg.cu), ordered by three device-side barriers per step:
@@ -1393,11 +1393,17 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
 
     The maps are read in their dtype (fp32 / bf16 / fp16) and layout: NCHW through the slot maps (planes a multiple of
     8 pixels), channels-last as rows (no slot maps).  philox: (seed, call index) -- every rank generates the same
-    stream of the whole batch's draws and the torch CPU generator is not touched."""
+    stream of the whole batch's draws and the torch CPU generator is not touched.
+
+    tail: the projector tail (projector.py) in place of K2 and the plan fetch, called after the selection as
+    ``tail(plan_dev, islab, slots, fslab address, exchange slab, this parity's offsets)``: it projects this rank's rows,
+    stores their normalised rows into every rank's slab, passes barrier A and returns the host plan records.  `needs`
+    are then the maps' gradients and ``tail.any_grad`` says whether a backward will run (the weights may want one)."""
     lib = _lib.load()
     dev, S, A, spec = sp.dev, sp.S, sp.A, sp.spec
     st = _stream()
     i32, f32, u8 = torch.int32, torch.float32, torch.uint8
+    grad_rows = any(needs) if tail is None else tail.any_grad
     if not sp.nhwc and not all(sp.slot_sizes):
         raise NotImplementedError("pooled mode needs NCHW feature planes that are a multiple of 8 pixels "
                                   "(or channels-last maps)")
@@ -1409,7 +1415,8 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
     xo = sp.x_off[par]
     world, rank = comm.world, comm.rank
     ws = torch.empty(sp.ws_bytes, dtype=u8, device=dev)
-    plan_dev = torch.empty(S * C.sizeof(_lib.ScalePlan), dtype=u8, device=dev)
+    # the tail's local row counts follow the plan records: one copy brings both to the host
+    plan_dev = torch.empty(S * C.sizeof(_lib.ScalePlan) + (4 * S if tail is not None else 0), dtype=u8, device=dev)
     with _timed("sample"):
         # local histograms -> all-gather of the (image, class) counts -> identical global plan on every rank
         fn, fname = _plan_entry(lib, labels, hist_only=True)
@@ -1436,7 +1443,8 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
         # dense gradients (local, in the maps' dtype and layout): zero-filled on the side stream.  Row statistics: the
         # sweeps accumulate them (one atomic per row, quarter and tile) in PRIVATE memory; pushed to every rank's slab
         # afterwards
-        gradbufs = _GradBuffers(feats32, needs, sp.nhwc, 0) if any(needs) else None
+        # (the tail's NCHW dense gradients are written whole by the one-pass writer: no fill)
+        gradbufs = _GradBuffers(feats32, needs, sp.nhwc, 0) if any(needs) and (tail is None or sp.nhwc) else None
         if gradbufs is not None:
             gradbufs.start_fill()
         stats_priv = torch.zeros(sp.stats_n, dtype=f32, device=dev)
@@ -1447,7 +1455,6 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
             draws = torch.empty((sp.max_draws + 3) // 4 * 4 + 4, dtype=i32, device=dev)
             _lib.check(lib.mscs_philox_stream(int(philox[0]) & (2 ** 64 - 1), int(philox[1]), sp.max_draws,
                                               draws.data_ptr(), st), "mscs_philox_stream")
-        plan = (_lib.ScalePlan * S)()
         ibase = islab.data_ptr()
         arrs = [_lib.ptr_array([ibase + 4 * sp.ioff[s][k] for s in range(S)]) for k in range(5)]
         fbase, bbase = fslab.data_ptr(), xs.local + xo["b"]
@@ -1464,31 +1471,20 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
             jb.total_out = total_t.data_ptr()
         # Selection and the peer-store gather are driven by the DEVICE plan records and enqueued before the host looks
         # at the plan: the one host wait of the forward (errors, row ranges) overlaps them instead of idling the GPU.
-        plan_sz = C.sizeof(_lib.ScalePlan)
-        _lib.check(lib.mscs_plan_fetch_begin(plan_dev.data_ptr(), S, st), "mscs_plan_fetch_begin")
+        if tail is None:
+            _lib.check(lib.mscs_plan_fetch_begin(plan_dev.data_ptr(), S, st), "mscs_plan_fetch_begin")
         _lib.check(lib.mscs_sample_select_async(C.byref(sp.cfg), plan_dev.data_ptr(), sp.v_cap, ws.data_ptr(),
                                                 draws.data_ptr(), *arrs, sarr, st), "mscs_sample_select_async")
-    with _timed("gather"):
-        for s in range(S):
-            n, Cc, h, w = sp.feat_shapes[s]
-            n_dev, code = plan_dev.data_ptr() + s * plan_sz + 8, _DTYPE_CODE[feats32[s].dtype]
-            boff, f32p, invp = xo["b"] + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
-            if sp.nhwc:         # the grid covers the row bound; the count is read on the device
-                _lib.check(lib.mscs_gather_rows_p2p(feats32[s].data_ptr(), Cc, ibase + 4 * sp.ioff[s][2], sp.Ncap[s],
-                                                    n_dev, xs.peers, world, rank, boff, f32p, invp, st, code),
-                           "mscs_gather_rows_p2p")
-            else:
-                _lib.check(lib.mscs_gather_normalize_p2p(feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(), 0,
-                                                         n_dev, xs.peers, world, rank, boff, f32p, invp, st, code),
-                           "mscs_gather_normalize_p2p")
-        comm.barrier(xs)                                   # A: every rank's key rows have landed here
-    _lib.check(lib.mscs_plan_fetch_end(plan, S), "mscs_plan_fetch_end")       # the host wait (plan records only)
+    if tail is not None:
+        plan = tail(plan_dev, islab, slots, fbase, xs, xo)
+    else:
+        plan = _gather_pooled(lib, sp, feats32, plan_dev, ibase, slots, fbase, comm, xs, xo, st)
     _raise_plan_errors(plan, S, spec)
     total = sum(int(plan[s].draws) for s in range(S))
     samples = _samples_from_plan(plan, islab, sp.ioff, A)
     # this parity's gradient rows: only the 128-aligned row blocks this rank computes are accumulated into (and
     # pulled from): clear those (1/world of the slab), on the main stream, long before the backward
-    if any(needs):
+    if grad_rows:
         zp, zb = [], []
         for s in range(S):
             rb, re_ = shard_rows(samples[s].N, world, rank)
@@ -1531,7 +1527,30 @@ def _run_forward_pooled(sp, labels, feats32, needs, comm, philox=None):
         "gradient_rows_pulled_bytes": int(n_local * sp.C_pad * 4 * (world - 1) / world)}
     return _PooledState(sp, job, samples, gradbufs, slots, (ws, islab, fslab, misc, work, slot_slab, stats_priv, draws),
                         fslab, misc[sp.out_off:sp.out_off + nt + 2], total_t, comm, xs, par, exchange_info,
-                        [f.dtype for f in feats32])
+                        [f.dtype for f in feats32], grad_rows)
+
+
+def _gather_pooled(lib, sp, feats32, plan_dev, ibase, slots, fbase, comm, xs, xo, st):
+    """K2 of the pooled mode fused with the all-gather of the key rows, barrier A, then the one host wait of the forward
+    (the plan records, whose copy was begun before the selection).  Returns the host plan records."""
+    S, world, rank, plan_sz = sp.S, comm.world, comm.rank, C.sizeof(_lib.ScalePlan)
+    with _timed("gather"):
+        for s in range(S):
+            n, Cc, h, w = sp.feat_shapes[s]
+            n_dev, code = plan_dev.data_ptr() + s * plan_sz + 8, _DTYPE_CODE[feats32[s].dtype]
+            boff, f32p, invp = xo["b"] + 2 * sp.boff[s], fbase + 4 * sp.foff[s][0], fbase + 4 * sp.foff[s][1]
+            if sp.nhwc:         # the grid covers the row bound; the count is read on the device
+                _lib.check(lib.mscs_gather_rows_p2p(feats32[s].data_ptr(), Cc, ibase + 4 * sp.ioff[s][2], sp.Ncap[s],
+                                                    n_dev, xs.peers, world, rank, boff, f32p, invp, st, code),
+                           "mscs_gather_rows_p2p")
+            else:
+                _lib.check(lib.mscs_gather_normalize_p2p(feats32[s].data_ptr(), n, Cc, h * w, slots[s].data_ptr(), 0,
+                                                         n_dev, xs.peers, world, rank, boff, f32p, invp, st, code),
+                           "mscs_gather_normalize_p2p")
+        comm.barrier(xs)                                   # A: every rank's key rows have landed here
+    plan = (_lib.ScalePlan * S)()
+    _lib.check(lib.mscs_plan_fetch_end(plan, S), "mscs_plan_fetch_end")       # the host wait (plan records only)
+    return plan
 
 
 def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
@@ -1547,18 +1566,7 @@ def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
     st = _stream()
     xo = sp.x_off[state.par]
     gb = state.gradbufs
-    if state.dF_fresh:
-        _cur_stream().wait_event(gb.ready)          # the side-stream zero fill of the dense gradients
-    else:
-        _lib.check(lib.mscs_fill_bytes(_lib.ptr_array([xs.local + xo["dF"]]), (C.c_int32 * 1)(0),
-                                       (C.c_size_t * 1)(4 * sp.dF_n), 1, st), "mscs_fill_bytes")
-        comm.barrier(xs)                            # nobody still pulls the previous rows
-    state.dF_fresh = False
-    _ptrs, ptrs_arr, lds = _row_accumulators(sp, xs.local + xo["dF"])
-    g = _as_f32(grad_out, dev)
-    with _timed("sim_bwd"):
-        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st), "mscs_sim_backward")
-        comm.barrier(xs)                            # C: every rank's gradient rows are complete
+    _sim_backward_pooled(lib, state, grad_out)
     grads = []
     io, fbase = state.io_dtypes, state.fslab.data_ptr()
     with _timed("scatter"):
@@ -1583,6 +1591,27 @@ def _run_backward_pooled(state, grad_out, needs, shapes, dtypes):
                                                          st, _DTYPE_CODE[io[s]]), "mscs_scatter_sectors_pull")
             grads.append(pre)
     return _as_dtypes(grads, dtypes)
+
+
+def _sim_backward_pooled(lib, state, grad_out):
+    """K4 of the pooled mode over this rank's row range into this parity's gradient rows, then barrier C.  A second
+    backward through the same graph clears the rows first (and waits until nobody still pulls the previous ones)."""
+    sp, comm, xs = state.sp, state.comm, state.xs
+    st = _stream()
+    xo = sp.x_off[state.par]
+    if state.dF_fresh:
+        if state.gradbufs is not None:
+            _cur_stream().wait_event(state.gradbufs.ready)      # the side-stream zero fill of the dense gradients
+    else:
+        _lib.check(lib.mscs_fill_bytes(_lib.ptr_array([xs.local + xo["dF"]]), (C.c_int32 * 1)(0),
+                                       (C.c_size_t * 1)(4 * sp.dF_n), 1, st), "mscs_fill_bytes")
+        comm.barrier(xs)                            # nobody still pulls the previous rows
+    state.dF_fresh = False
+    _ptrs, ptrs_arr, lds = _row_accumulators(sp, xs.local + xo["dF"])
+    g = _as_f32(grad_out, sp.dev)
+    with _timed("sim_bwd"):
+        _lib.check(lib.mscs_sim_backward(C.byref(state.job), g.data_ptr(), ptrs_arr, lds, st), "mscs_sim_backward")
+        comm.barrier(xs)                            # C: every rank's gradient rows are complete
 
 
 def _row_accumulators(sp, base):

@@ -167,9 +167,74 @@ __global__ void __launch_bounds__(256) k_gather_rows_p2p(const __grid_constant__
   });
 }
 
+// Projector tail in the pooled mode: this rank's rows in compact order.  One CTA per scale scans the sorted rows 1024
+// at a time; a row below the device count with pix >= 0 is local and gets k = the number of local rows before it, so
+// the compact order is the global row order restricted to the local rows (no atomics: deterministic).
+struct LocalRows {
+  const int* pix[MSCS_MAX_SCALES]; const int* n_rows_dev[MSCS_MAX_SCALES]; int* crow[MSCS_MAX_SCALES];
+  int* cpix[MSCS_MAX_SCALES]; int* slot[MSCS_MAX_SCALES]; int rows[MSCS_MAX_SCALES]; int* n_local_dev;
+};
+__global__ void __launch_bounds__(1024) k_local_rows(const __grid_constant__ LocalRows a) {
+  const int s = blockIdx.x;
+  const int* __restrict__ pix = a.pix[s];
+  int* __restrict__ crow = a.crow[s];
+  int* __restrict__ cpix = a.cpix[s];
+  int* __restrict__ slot = a.slot[s];
+  const int rows = a.rows[s];
+  __shared__ int warp_total[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int N = max(0, min(*a.n_rows_dev[s], rows));      // pix entries at and above the count are stale
+  int base = 0;
+  for (int r0 = 0; r0 < rows; r0 += 1024) {
+    const int r = r0 + (int)threadIdx.x;
+    const int p = r < N ? pix[r] : -1;
+    const unsigned m = __ballot_sync(0xffffffffu, p >= 0);
+    if (lane == 0) warp_total[warp] = __popc(m);
+    __syncthreads();
+    int before = 0, total = 0;
+    for (int w = 0; w < 32; ++w) {
+      const int t = warp_total[w];
+      before += w < warp ? t : 0;
+      total += t;
+    }
+    const int k = base + before + __popc(m & ((1u << lane) - 1u));
+    if (r < rows) crow[r] = p >= 0 ? k : -1;
+    if (p >= 0) {
+      cpix[k] = p;
+      if (slot) slot[p] = k;
+    }
+    base += total;
+    __syncthreads();      // warp_total is rewritten by the next chunk
+  }
+  if (threadIdx.x == 0) a.n_local_dev[s] = base;
+}
+
 }  // namespace mscs
 
 using namespace mscs;
+
+extern "C" int mscs_local_rows_batch(const int32_t* const* pix, const int32_t* const* n_rows_dev, const int32_t* rows,
+                                     int32_t* const* crow, int32_t* const* cpix, int32_t* const* slot,
+                                     int32_t* n_local_dev, int count, void* stream_) {
+  MSCS_CHECK_ARG(count >= 1 && count <= MSCS_MAX_SCALES, "bad scale count %d", count);
+  MSCS_CHECK_ARG(pix && n_rows_dev && rows && crow && cpix && n_local_dev, "null pointer argument");
+  MSCS_CHECK_ARG((uintptr_t)n_local_dev % 4 == 0, "n_local_dev must be 4-byte aligned");
+  LocalRows a{};
+  a.n_local_dev = n_local_dev;
+  for (int s = 0; s < count; ++s) {
+    MSCS_CHECK_ARG(pix[s] && n_rows_dev[s] && crow[s] && cpix[s], "scale %d: null pointer argument", s);
+    MSCS_CHECK_ARG(rows[s] >= 0, "scale %d: %d rows", s, rows[s]);
+    const int32_t* sl = slot ? slot[s] : nullptr;
+    for (const void* p : {(const void*)pix[s], (const void*)n_rows_dev[s], (const void*)crow[s], (const void*)cpix[s],
+                          (const void*)sl})
+      MSCS_CHECK_ARG((uintptr_t)p % 4 == 0, "scale %d: int32 arrays must be 4-byte aligned", s);
+    a.pix[s] = pix[s]; a.n_rows_dev[s] = n_rows_dev[s]; a.crow[s] = crow[s]; a.cpix[s] = cpix[s];
+    a.slot[s] = const_cast<int*>(sl); a.rows[s] = rows[s];
+  }
+  k_local_rows<<<count, 1024, 0, (cudaStream_t)stream_>>>(a);
+  MSCS_LAUNCH_CHECK();
+  return 0;
+}
 
 static int fill_peers(PeerPtrs* out, void* const* ptrs, int n, size_t byte_off) {
   MSCS_CHECK_ARG(ptrs && n >= 1 && n <= MSCS_MAX_RANKS, "bad peer table (%d ranks, at most %d)", n, MSCS_MAX_RANKS);

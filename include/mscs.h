@@ -451,6 +451,24 @@ int mscs_gather_rows_p2p(const void* feat, int C, const int32_t* pix, int N, con
 int mscs_scatter_rows_pull(void* const* slabs, int world, size_t dF_byte_off, int rows_per_rank, int ldF,
                            const float* anc_f32, const float* inv_norm, const int32_t* pix, int N, int C, void* dfeat,
                            void* stream, int dtype);
+/* Projector tail in the pooled mode: this rank's rows in compact order, every scale in one launch (one CTA per scale),
+ * the row counts read on the device.  Global sorted row r of scale s (r < N_s = min(*n_rows_dev[s], rows[s])) is local
+ * when pix[s][r] >= 0; its compact index k = the number of local rows before it (the global row order restricted to
+ * the local rows).  Per scale s < count (arrays of `count` entries):
+ *   pix, n_rows_dev, rows  the selection's pix array, its row count in device memory (e.g. &plan_dev[s].N) and the
+ *                          count's upper bound; pix entries at and above the count are not read
+ *   crow                   out, rows[s] entries: k of global row r, -1 for another rank's row and for r >= N_s
+ *   cpix                   out, n_local entries: local pixel of compact row k (the pix entry of its row)
+ *   slot                   optional (the array or an entry may be NULL), NCHW: the selection's slot map, rewritten in
+ *                          place to compact ids: slot[cpix[k]] = k; no other entry is touched
+ *   n_local_dev            out, ONE int32 array of `count` entries: n_local of scale s at [s]
+ * Nothing else is written.  Every array is int32 and 4-byte aligned.  The rest of the pooled tail's data path is the
+ * entry points above with these index arrays: the raw gathers (rewritten slot map / cpix with &n_local_dev[s]), the
+ * normalisation + peer-store gather of the projected rows (mscs_gather_rows_p2p with pix = crow), the pull of their
+ * gradient rows (mscs_scatter_rows_pull with pix = crow) and the raw dense writers (rewritten slot map / cpix). */
+int mscs_local_rows_batch(const int32_t* const* pix, const int32_t* const* n_rows_dev, const int32_t* rows,
+                          int32_t* const* crow, int32_t* const* cpix, int32_t* const* slot, int32_t* n_local_dev,
+                          int count, void* stream);
 
 #ifdef __cplusplus
 }

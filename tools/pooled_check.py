@@ -2,9 +2,13 @@
 with the single-process loss of the concatenated batch computed locally.
 
   torchrun --nproc-per-node N tools/pooled_check.py [cfg5] [--dtype bf16] [--layout channels_last] [--sampler philox]
+                                                   [--tail]
 
 --dtype / --layout / --sampler: element type and memory format of the feature maps (both runs get the same maps) and
-the sampler.  cfg5: also BASELINE config 5 (fp32 NCHW maps, reference sampler) against the fp64-oracle fixture."""
+the sampler.  cfg5: also BASELINE config 5 (fp32 NCHW maps, reference sampler) against the fp64-oracle fixture.
+--tail: the projector tail (ProjectorTailContrastive_ms, c_prev 64 -> d 64, the same weights on every rank) instead of
+the drop-in class on the maps; the sum over the ranks of the weight and bias gradients is compared with the
+single-process ones (within 1e-3 of their maximum)."""
 import argparse, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -18,6 +22,7 @@ ap.add_argument("mode", nargs="?", choices=["cfg5"])
 ap.add_argument("--dtype", choices=["fp32", "bf16", "fp16"], default="fp32")
 ap.add_argument("--layout", choices=["nchw", "channels_last"], default="nchw")
 ap.add_argument("--sampler", choices=["reference", "philox"], default="reference")
+ap.add_argument("--tail", action="store_true")
 args = ap.parse_args()
 dtype = {"fp32": torch.float32, "bf16": torch.bfloat16, "fp16": torch.float16}[args.dtype]
 fmt = torch.channels_last if args.layout == "channels_last" else torch.contiguous_format
@@ -32,13 +37,22 @@ cfg = dict(dataset="CITYSCAPES", experiment=1, temperature=0.1, scales=3, weight
 n = 2 * world
 labels = synth.synth_labels(n, 128, 256, 19, 7, 16, 0.05, 21)
 feats = synth.synth_features(n, 64, 128, 256, [4, 8, 16], 22)
-full = mscs_b200.DenseContrastiveLossV2_ms(dict(cfg))
+
+
+def make(comm=None):
+    if not args.tail:
+        return mscs_b200.DenseContrastiveLossV2_ms(dict(cfg), comm=comm)
+    torch.manual_seed(3)            # the same tails on every rank and in the single process
+    return mscs_b200.ProjectorTailContrastive_ms(dict(cfg), 64, 64, comm=comm).to(dev)
+
+
+full = make()
 fg = [f.to(dev).to(dtype).contiguous(memory_format=fmt).requires_grad_(True) for f in feats]
 torch.manual_seed(5)
 loss_full = full(labels.to(dev), fg)
 loss_full.backward()
 nl = n // world
-mod = mscs_b200.DenseContrastiveLossV2_ms(dict(cfg), comm=mscs_b200.TorchDistComm())
+mod = make(mscs_b200.TorchDistComm())
 fl = [f[rank * nl:(rank + 1) * nl].to(dev).to(dtype).contiguous(memory_format=fmt).requires_grad_(True) for f in feats]
 torch.manual_seed(5)
 loss = mod(labels[rank * nl:(rank + 1) * nl].to(dev), fl)
@@ -51,7 +65,14 @@ for s in range(len(fl)):
     cos = float(g @ w / np.sqrt((g @ g) * (w @ w)))
     ok = ok and cos > 0.99999 and np.array_equal(g != 0, w != 0)
     print(f"rank {rank} scale {s}: cosine {cos:.8f} max-abs {np.abs(g - w).max():.3e}", flush=True)
-print(f"rank {rank} ({args.dtype}, {args.layout}, sampler {args.sampler}): pooled loss {float(loss):.6f} single-process "
+if args.tail:
+    for name, mine, ref in [(f"{k}{s}", getattr(t, k).grad.clone(), getattr(u, k).grad)
+                            for k in ("weight", "bias") for s, (t, u) in enumerate(zip(mod.tails, full.tails))]:
+        dist.all_reduce(mine)           # the ranks' contributions
+        err = float((mine - ref).abs().max()) / float(ref.abs().max())
+        ok = ok and err <= 1e-3
+        print(f"rank {rank} tail {name}: sum over ranks vs single process, max-abs / max {err:.3e}", flush=True)
+print(f"rank {rank} ({'tail, ' if args.tail else ''}{args.dtype}, {args.layout}, sampler {args.sampler}): pooled loss {float(loss):.6f} single-process "
       f"{float(loss_full):.6f} -> {'OK' if ok else 'MISMATCH'}", flush=True)
 
 if args.mode == "cfg5":
